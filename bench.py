@@ -1,7 +1,7 @@
 """Benchmark of the HiT-SIR-pro forward pass (BASELINE.json metric: output megapixels/s).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload cfg2|cfg3|cfg4|cfg5|cfg1]
-                    [--no-extras] [--no-cpu-baseline] [--gather u8|f32|nccl]
+                    [--no-extras] [--no-cpu-baseline] [--gather u8|f32|nccl] [--dump-outputs DIR]
 
 One step = one forward of one batch of synthetic LR images through the public nn.Module (-> C ABI -> CUDA).
 N=1 workload: BASELINE.json configs[1] (32 x 3 x 256 x 256 LR, x4 'nearest+conv', pro config).  For N>1 the launcher is torchrun
@@ -12,7 +12,8 @@ Timed region of `value`: K forwards with per-launch profiling OFF, CUDA events o
 sides, max over ranks.  The per-category breakdown / roofline numbers come from a SECOND, profiled pass of a few steps.
 Extra keys on the same line (unless --no-extras): "cfg4" = BASELINE configs[3] (16 x 512 x 512, x4) strong-scaled over the N ranks,
 "cfg3" = BASELINE configs[2] (the eight 576 x 576 halo tiles of a 1920 x 1080 frame, x2 'pixelshuffle') dealt to the N ranks, gathered
-and stitched on rank 0; "gpu_baseline" = the unmodified reference module run eagerly on the same B200 (when its sources are staged).
+and stitched on rank 0; "gpu_baseline" = the unmodified reference module run eagerly on the same B200 (when HITSIR_REFERENCE_DIR names
+a checkout of the original project).
 """
 import argparse
 import contextlib
@@ -29,6 +30,8 @@ ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
 
 import torch  # noqa: E402
+
+from oracle.reference import reference_dir  # noqa: E402
 
 WORKLOADS = {
     # name: (flags, upsampler, upscale, batch, H, W, description)
@@ -145,18 +148,9 @@ def measured_traffic(cat):
     return None
 
 
-def reference_root():
-    """Where the UNMODIFIED reference sources are: the live tree in the build container, the staged copy (tools/stage_reference.py,
-    git-ignored baseline/_ref) on the GPU box; None when neither exists."""
-    for root in ("/root/reference", os.path.join(ROOT, "baseline", "_ref")):
-        if os.path.exists(os.path.join(root, "models", "hit_sir_pro.py")):
-            return root
-    return None
-
-
 def load_reference_class():
     """The reference's own `HiT_SIR` class (models/hit_sir_pro.py:1065), imported unchanged through the 3-symbol timm shim."""
-    root = reference_root()
+    root = reference_dir()
     if root is None:
         return None
     shim = os.path.join(ROOT, "oracle", "ref_shim")
@@ -362,6 +356,27 @@ def run_cfg3_exact(hitsir_b200, dev, world, rank):
             "note": "ms_per_frame: each band's launches and exchanges replayed as one CUDA graph per rank; ms_per_frame_eager: enqueued per frame (Python exchange callbacks)"}
 
 
+DUMP_MAX_ELEMENTS = 1 << 23                                     # 32 MiB of float32
+
+
+def dump_outputs(out_dir, y):
+    """Write the SR output `y` of the last timed step as float32 .npy for output-by-output comparison of two builds: `sr.npy` (the
+    whole NCHW tensor) when it has at most DUMP_MAX_ELEMENTS values, else `sr_sample.npy`, the values at DUMP_MAX_ELEMENTS flat
+    positions drawn (with replacement, sorted) by a generator seeded with 0 -- the same positions for the same output shape."""
+    os.makedirs(out_dir, exist_ok=True)
+    import numpy as np
+    flat = y.detach().reshape(-1)
+    if flat.numel() <= DUMP_MAX_ELEMENTS:
+        name, arr = "sr", y.detach().float().cpu().numpy()
+    else:
+        g = torch.Generator().manual_seed(0)
+        idx = torch.randint(flat.numel(), (DUMP_MAX_ELEMENTS,), generator=g).sort().values
+        name, arr = "sr_sample", flat[idx.to(flat.device)].float().cpu().numpy()
+    path = os.path.join(out_dir, name + ".npy")
+    np.save(path, arr)
+    print(f"[bench] last timed step's output {tuple(y.shape)} -> {path} {arr.shape}", file=sys.stderr)
+
+
 def run_ours(args):
     import torch.distributed as dist
     import hitsir_b200
@@ -409,6 +424,8 @@ def run_ours(args):
 
     def step():
         y = model(x)
+        if args.dump_outputs:
+            state["y"] = y
         if world > 1:
             if peer is not None:
                 payload = hitsir_b200.to_uint8_hwc(y) if u8 else y
@@ -440,6 +457,8 @@ def run_ours(args):
         launches_per_step = model.last_launch_count
         # ---- the headline: profiling off
         ms_step, clocks = timed_steps(step, drain, args.steps, world, dev, sample_clocks=True)
+        if args.dump_outputs and rank == 0:
+            dump_outputs(args.dump_outputs, state["y"])
         # ---- second pass, per-launch CUDA events on: per-category breakdown and the dominant kernel's launch time
         psteps = max(1, min(args.steps, 3))
         model.profile_enable(dev, True)
@@ -576,7 +595,7 @@ def cpu_forward_fn(workload):
     if RefHiT is not None:
         torch.manual_seed(0)
         m = build_reference(RefHiT, flags, up, scale)
-        return (lambda x: m(x)), "reference", f"unmodified reference module ({reference_root()}/models/hit_sir_pro.py), fp32, eval, no_grad"
+        return (lambda x: m(x)), "reference", f"unmodified reference module ({reference_dir()}/models/hit_sir_pro.py), fp32, eval, no_grad"
     from oracle.hitsir_oracle import HiTSIROracle, OracleConfig
     o = HiTSIROracle(reference_state_dict(workload), OracleConfig(*[bool(f) for f in flags], upscale=scale, upsampler=up))
 
@@ -613,7 +632,7 @@ def cpu_baseline(workload, budget_s=20.0):
 def run_reference(args):
     """Reference arm: the reference's own CPU implementation of the path on the box's host cores.  Each step = the forward of ONE
     full-size image of the workload (cfg2: 1 x 3 x 256 x 256), whatever --steps is; the process never imports the product package.
-    With the reference sources present (/root/reference or the staged baseline/_ref) the UNMODIFIED module is timed (kind
+    With the reference sources present (HITSIR_REFERENCE_DIR) the UNMODIFIED module is timed (kind
     "reference"), else the oracle port (kind "port").  Bounded: one warm-up forward, then K timed steps or ~4 minutes, whichever
     comes first (the count actually timed is reported)."""
     rank = int(os.environ.get("RANK", "0"))
@@ -663,7 +682,14 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="skip the cfg3 / cfg4 / gpu_baseline keys")
     ap.add_argument("--gather", default=os.environ.get("HITSIR_GATHER", "u8"), choices=["u8", "f32", "nccl"])
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write rank 0's SR output of the last timed step to DIR as float32 .npy "
+                    "(the whole output up to 32 MiB, else a fixed seeded sample); inputs and weights are seeded, so two builds "
+                    "run with the same arguments can be compared output for output")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     if args.impl == "reference":
         run_reference(args)

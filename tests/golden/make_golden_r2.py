@@ -169,7 +169,7 @@ def make_scc():
     for scc, meth in restore:
         delattr(scc, meth)                                # back to the class's unmodified bound method
     arrays = {}
-    S_STRIDE, B_STRIDE = 13, 17
+    S_STRIDE, B_STRIDE = 26, 34                           # keeps the fixture under 1 MB
     for j, blk in enumerate(blocks):
         scc = blk.correlation
         wh, ww = scc.window_size

@@ -239,7 +239,7 @@ def _nccl_worker(rank, world, port, out_dir):
 @pytest.mark.gpu
 def test_banded_two_gpus_nvlink(tmp_path):
     if torch.cuda.device_count() < 2:
-        pytest.skip("needs 2 GPUs (run with gpurun --gpus 2)")
+        pytest.skip("needs 2 GPUs")
     world = 2
     mp.spawn(_nccl_worker, args=(world, _free_port(), str(tmp_path)), nprocs=world, join=True)
     assert all(os.path.exists(tmp_path / f"ok_{r}") for r in range(world))

@@ -8,6 +8,7 @@ import torch
 
 import hitsir_b200
 from oracle.weights import synthetic_image
+from oracle.reference import reference_dir
 from tests.helpers import GOLDEN_CASES, build_pair, load_golden
 
 
@@ -160,13 +161,14 @@ def test_known_answer_param_count():
     assert len(m.state_dict()) == 1650
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/models"), reason="reference tree not present on this box")
+@pytest.mark.skipif(reference_dir() is None, reason="HITSIR_REFERENCE_DIR does not name a checkout of the original project")
 def test_oracle_matches_live_reference():
     import contextlib, io, sys, warnings
     warnings.filterwarnings("ignore")
     root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    ref_root = reference_dir()
     sys.path.insert(0, os.path.join(root, "oracle", "ref_shim"))
-    sys.path.insert(0, "/root/reference")
+    sys.path.insert(0, ref_root)
     try:
         with contextlib.redirect_stdout(io.StringIO()):
             from models.hit_sir_pro import HiT_SIR as RefHiT
@@ -177,7 +179,7 @@ def test_oracle_matches_live_reference():
         with torch.no_grad():
             assert (ref(x) - oracle(x)).abs().max().item() < 2e-5
     finally:
-        sys.path.remove("/root/reference")
+        sys.path.remove(ref_root)
         sys.modules.pop("models.hit_sir_pro", None)
         sys.modules.pop("models", None)
 

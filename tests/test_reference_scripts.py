@@ -1,14 +1,14 @@
 """The reference's own inference script, UNCHANGED, on the drop-in module (-m gpu).
 
 north_star: "... the same forward(x) contract, so test.py and experiments/*_experiment.py run unchanged".  `test_experiment.py`
-(/root/reference/test_experiment.py) is the reference's single-image demo: `from models.hit_sir_pro import HiT_SIR` (:8),
+(of the original project) is the reference's single-image demo: `from models.hit_sir_pro import HiT_SIR` (:8),
 `create_model()` (:25-32), `load_model_weights()` of a harness-format checkpoint {'start_epoch','model',...} (:35-50), PIL -> [0,1]
 tensor -> `model(lr.unsqueeze(0)).clip(0, 1)` (:75) -> PIL -> `.show()`; it calls `main(...)` at import time (:96).  The test
 executes that file byte for byte (runpy) from a scratch directory that holds the image and the checkpoint at the relative paths the
 script hard-codes, with exactly the two-line integration of INTEGRATION.md section 1 applied (the `models.hit_sir_pro` import
 resolves to hitsir_b200) and `PIL.Image.Image.show` stubbed to capture the result, and compares the shown image with the CPU oracle.
 
-The script comes from /root/reference when present, else from the staged copy baseline/_ref (tools/stage_reference.py; git-ignored).
+The script comes from a checkout of the original project named by HITSIR_REFERENCE_DIR; without one the test skips.
 `experiments/hitsir_pro_experiment.py` cannot be imported in this image at all (lpips and skimage are not installed), with or
 without the drop-in, so only its constructor call (:15-26) is replayed.
 """
@@ -24,20 +24,17 @@ import torch
 import hitsir_b200
 from oracle.weights import fill_state_dict, synthetic_image
 from oracle.hitsir_oracle import HiTSIROracle, OracleConfig
-
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-sys.path.insert(0, os.path.join(ROOT, "tools"))
-from stage_reference import reference_root  # noqa: E402
+from oracle.reference import reference_dir
 
 CKPT = "weights/hitsir_pro_loss(l1)_mulsizeconvextract(True)_casa(True)_fusion_embed_dim(180)_len(depths)(6)_augment/best_psnr_ssim_lpips_model.pth"
 IMG = "data/test/RealSRSet+5images/0014.jpg"
 
 
 @pytest.mark.gpu
-@pytest.mark.skipif(reference_root() is None, reason="neither /root/reference nor baseline/_ref holds the reference scripts")
+@pytest.mark.skipif(reference_dir() is None, reason="HITSIR_REFERENCE_DIR does not name a checkout of the original project")
 def test_reference_test_experiment_runs_unchanged(tmp_path, monkeypatch):
     from PIL import Image
-    ref_root = reference_root()
+    ref_root = reference_dir()
     # the files the script hard-codes, relative to its working directory
     proto = hitsir_b200.HiT_SIR(True, True, True, **hitsir_b200.PRO_KWARGS)
     sd = fill_state_dict(proto.state_dict(), 77, "init")
