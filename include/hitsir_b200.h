@@ -165,7 +165,7 @@ HITSIR_API int hitsir_psnr_y(const float* sr, const float* hr, int B, int H, int
 /* Test hook standing in for PyTorch forward hooks on reference sub-modules: the next
  * hitsir_forward copies the named intermediate activation (fp32, NHWC, real channels only) into
  * `dst` (device) and, when `stop` != 0, returns right after producing it.  Names: "shallow",
- * "embed", "block<i>.<j>.qkv", "block<i>.<j>.scc", "block<i>.<j>.attn", "block<i>.<j>",
+ * "embed", "block<i>.<j>.qkv", "block<i>.<j>.scc", "block<i>.<j>.attn", "block<i>.<j>.fc1" (GELU(fc1), 360 channels), "block<i>.<j>",
  * "layer<i>", "norm", "conv_after_body", "fused", "conv_before_upsample", "up1", "up2", "hr".
  * Pass name = NULL to clear. */
 HITSIR_API int hitsir_set_tap(HitsirHandle* h, const char* name, float* dst, int64_t dst_floats, int stop);
@@ -193,8 +193,8 @@ HITSIR_API int hitsir_profile_enable(HitsirHandle* h, int on);
 HITSIR_API int hitsir_profile_num_categories(const HitsirHandle* h);
 HITSIR_API int hitsir_profile_get(HitsirHandle* h, int index, const char** name, double* total_ms, int64_t* launches);
 
-/* "umma" (tcgen05 path with TMA-staged epilogues, default) or "umma_direct" (same mainloop, per-row global stores).  A test build with
- * -DHITSIR_AB_PATHS additionally accepts "simt" (fp32 cross-check kernels); the product library has no other backend. */
+/* "umma" (tcgen05 path with TMA-staged epilogues), the only backend of the product library.  A test build with -DHITSIR_AB_PATHS
+ * additionally accepts "umma_direct" (same mainloop, per-row global stores, unfused FFN tail) and "simt" (fp32 cross-check kernels). */
 HITSIR_API int hitsir_set_gemm_backend(HitsirHandle* h, const char* backend);
 
 HITSIR_API const char* hitsir_last_error(void);

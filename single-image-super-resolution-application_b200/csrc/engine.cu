@@ -891,6 +891,7 @@ int forward_block(Fwd& f, int i, int j, float* xin, float* xout) {
   p.epi = EPI_STORE; p.act = ACT_GELU; p.n_real = kHid; p.out_bf16 = ws.H1; p.ldb = kHidp;
   RUN(linear(f, "gemm_fc1_gelu", bw.fc1, ws.xb0, f.N, p));
   }
+  TAP((tn + ".fc1").c_str(), ws.H1, 1, kHidp, f.N, kHid);
   const bool need_shadow = (j == c.depths[i] - 1);      // the RHTB conv after the last block reads a bf16 shadow of the stream (:934)
   if (!h->simt && !h->direct_epilogue && !h->ffn_unfused) {
     // dwconv5 + GELU + input, fc2, norm2 and the residual add in one kernel: the hidden map h2 never reaches HBM
@@ -1369,11 +1370,12 @@ HITSIR_API int hitsir_profile_get(HitsirHandle* h, int i, const char** name, dou
 HITSIR_API int hitsir_set_gemm_backend(HitsirHandle* h, const char* backend) {
   if (!h || !backend) { set_error("null argument"); return HITSIR_ERR_INVALID; }
   if (strcmp(backend, "umma") == 0) { h->simt = false; h->direct_epilogue = false; }
-  else if (strcmp(backend, "umma_direct") == 0) { h->simt = false; h->direct_epilogue = true; }
 #ifdef HITSIR_AB_PATHS
+  // the direct-store epilogues need the unfused FFN tail, which only this build compiles
+  else if (strcmp(backend, "umma_direct") == 0) { h->simt = false; h->direct_epilogue = true; }
   else if (strcmp(backend, "simt") == 0) h->simt = true;
 #endif
-  else { set_error("unknown gemm backend '%s' (umma | umma_direct; 'simt' only in the -DHITSIR_AB_PATHS test build)", backend); return HITSIR_ERR_INVALID; }
+  else { set_error("unknown gemm backend '%s' (umma; 'umma_direct' and 'simt' only in the -DHITSIR_AB_PATHS test build)", backend); return HITSIR_ERR_INVALID; }
   return 0;
 }
 

@@ -8,7 +8,12 @@ import torch.nn.functional as F
 TAPS = {(0, 0): (0,), (0, 1): (1, 2), (1, 0): (0, 1), (1, 1): (2,)}
 
 
-def subpixel_conv(x, w, b):
+def phase_filter(w, a, bb, dyi, dxi):
+    """The (Co, Ci) filter of output phase (a, bb) at LR offset index (dyi, dxi): its taps summed in pack_subpixel_kernel's order."""
+    return sum(w[:, :, ky, kx] for ky in TAPS[(a, dyi)] for kx in TAPS[(bb, dxi)])
+
+
+def subpixel_conv(x, w, b, filt=phase_filter):
     n, _, h, wd = x.shape
     out = torch.empty(n, w.shape[0], 2 * h, 2 * wd, dtype=x.dtype)
     xp = F.pad(x, (1, 1, 1, 1))
@@ -17,7 +22,7 @@ def subpixel_conv(x, w, b):
             acc = b.view(1, -1, 1, 1).expand(n, -1, h, wd).clone()
             for dyi in range(2):
                 for dxi in range(2):
-                    wp = sum(w[:, :, ky, kx] for ky in TAPS[(a, dyi)] for kx in TAPS[(bb, dxi)])
+                    wp = filt(w, a, bb, dyi, dxi)
                     dy, dx = a - 1 + dyi, bb - 1 + dxi
                     acc = acc + torch.einsum("oc,nchw->nohw", wp, xp[:, :, 1 + dy:1 + dy + h, 1 + dx:1 + dx + wd])
             out[:, :, a::2, bb::2] = acc
