@@ -179,6 +179,23 @@ HITSIR_API int64_t hitsir_psnr_y_scratch_doubles(int B, int H, int W);
 HITSIR_API int hitsir_psnr_y(const float* sr, const float* hr, int B, int H, int W, int clip_sr, double* scratch, double* mse_out,
                   void* stream);
 
+/* The evaluation's second metric on the device (experiments/experiment.py:575-640): per-image mean SSIM of the Y channels,
+ * skimage.metrics.structural_similarity(hr_y, sr_y, data_range=1) of scikit-image 0.24.  Y and the clip of `sr` as hitsir_psnr_y.
+ * With x = Y(hr), y = Y(sr) and window means (weighted by the window) ux, uy, uxx, uyy, uxy of x, y, x*x, y*y, x*y:
+ *   vx = cn (uxx - ux^2),  vy = cn (uyy - uy^2),  vxy = cn (uxy - ux uy)
+ *   S  = ((2 ux uy + C1)(2 vxy + C2)) / ((ux^2 + uy^2 + C1)(vx + vy + C2)),  C1 = 0.01^2, C2 = 0.03^2,
+ * and ssim_out[b] (device, double) is the mean of S over the interior [p, H-p) x [p, W-p), p = (win-1)/2, where every window lies
+ * inside the image.  Windows: gaussian == 0 -> uniform 7 x 7 (skimage's default); gaussian != 0 -> Gaussian sigma = 1.5 truncated at
+ * 3.5 sigma, 11 x 11, taps exp(-x^2 / (2 sigma^2)) normalised, x = -5..5 (gaussian_weights=True).  sample_cov != 0 -> cn = win^2 /
+ * (win^2 - 1), for the Gaussian window too, as skimage does (use_sample_covariance=True, its default); 0 -> cn = 1 (Wang et al.).
+ * Products are formed in fp32, window sums in double rounded to fp32, S in fp32 as skimage writes it (ssim(x, x) is exactly 1).
+ * H or W smaller than the window is HITSIR_ERR_INVALID (skimage raises ValueError).  `scratch`: device buffer of
+ * hitsir_ssim_y_scratch_doubles(B,H,W,gaussian) doubles.  Fixed-order reduction (bitwise reproducible, independent of the other images of
+ * the batch); asynchronous on `stream`; needs no handle. */
+HITSIR_API int64_t hitsir_ssim_y_scratch_doubles(int B, int H, int W, int gaussian);
+HITSIR_API int hitsir_ssim_y(const float* sr, const float* hr, int B, int H, int W, int clip_sr, int gaussian, int sample_cov,
+                  double* scratch, double* ssim_out, void* stream);
+
 /* Test hook standing in for PyTorch forward hooks on reference sub-modules: the next
  * hitsir_forward copies the named intermediate activation (fp32, NHWC, real channels only) into
  * `dst` (device) and, when `stop` != 0, returns right after producing it.  Names: "shallow",

@@ -74,6 +74,9 @@ SYMBOLS = {
     "hitsir_f32nchw_to_u8hwc": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p]),
     "hitsir_psnr_y_scratch_doubles": (C.c_int64, [C.c_int, C.c_int, C.c_int]),
     "hitsir_psnr_y": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "hitsir_ssim_y_scratch_doubles": (C.c_int64, [C.c_int, C.c_int, C.c_int, C.c_int]),
+    "hitsir_ssim_y": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p,
+                                C.c_void_p]),
     "hitsir_set_tap": (C.c_int, [C.c_void_p, C.c_char_p, C.c_void_p, C.c_int64, C.c_int]),
     "hitsir_set_inject": (C.c_int, [C.c_void_p, C.c_char_p, C.c_void_p, C.c_int64]),
     "hitsir_get_bias_table": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_int64, C.c_void_p]),

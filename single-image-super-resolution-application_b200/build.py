@@ -19,11 +19,11 @@ CSRC = os.path.join(HERE, "csrc")
 BUILD = os.path.join(HERE, "build")
 LIB = os.path.join(HERE, "libhitsir_b200.so")
 SOURCES = ["engine.cu", "umma_gemm.cu", "umma_gemm_tma.cu", "conv3_c64.cu", "ffn_tail.cu", "scc_umma.cu", "scc_dense.cu", "glue.cu", "pack.cu",
-           "ensemble.cu"]
+           "ensemble.cu", "ssim.cu"]
 # A/B cross-check kernels (SIMT GEMM, stand-alone depthwise conv, SIMT casa gate, the slower proj+fc1 chain): compiled only into a test
 # build (`build.py --ab` -> libhitsir_b200_ab.so, -DHITSIR_AB_PATHS); the product library has one path and no switches
 AB_SOURCES = ["proj_fc1.cu", "simt_ref.cu"]
-HEADERS = ["common.cuh", "gemm.cuh", "kernels.cuh", os.path.join("..", "..", "include", "hitsir_b200.h")]
+HEADERS = ["common.cuh", "gemm.cuh", "kernels.cuh", "ycbcr.cuh", os.path.join("..", "..", "include", "hitsir_b200.h")]
 NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
 FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
          "-Xcompiler", "-fPIC", "-Xcompiler", "-fvisibility=hidden", "-DNDEBUG"]

@@ -1389,6 +1389,23 @@ HITSIR_API int hitsir_psnr_y(const float* sr, const float* hr, int B, int H, int
   return 0;
 }
 
+HITSIR_API int64_t hitsir_ssim_y_scratch_doubles(int B, int H, int W, int gaussian) {
+  if (B <= 0) return 0;
+  return (int64_t)B * ssim_y_tiles(H, W, gaussian);
+}
+
+HITSIR_API int hitsir_ssim_y(const float* sr, const float* hr, int B, int H, int W, int clip_sr, int gaussian, int sample_cov, double* scratch,
+                             double* ssim_out, void* stream) {
+  if (!sr || !hr || !scratch || !ssim_out) { set_error("hitsir_ssim_y: null argument"); return HITSIR_ERR_INVALID; }
+  const int win = 2 * ssim_y_radius(gaussian) + 1;
+  if (B <= 0 || H < win || W < win) {
+    set_error("hitsir_ssim_y: bad shape %d x %d x %d (H and W must be at least the %d x %d window)", B, H, W, win, win);
+    return HITSIR_ERR_INVALID;
+  }
+  if (launch_ssim_y(sr, hr, B, H, W, clip_sr, gaussian, sample_cov, scratch, ssim_out, (cudaStream_t)stream)) return HITSIR_ERR_CUDA;
+  return 0;
+}
+
 HITSIR_API int hitsir_set_tap(HitsirHandle* h, const char* name, float* dst, int64_t dst_floats, int stop) {
   if (!h) { set_error("null handle"); return HITSIR_ERR_INVALID; }
   if (!name) { h->tap = Tap(); return 0; }

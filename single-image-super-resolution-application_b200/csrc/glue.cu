@@ -7,6 +7,7 @@
 
 #include "gemm.cuh"
 #include "kernels.cuh"
+#include "ycbcr.cuh"
 
 namespace hitsir {
 
@@ -210,14 +211,10 @@ __global__ void f32nchw_to_u8hwc_kernel(const float* __restrict__ in, uint8_t* _
 }
 
 // Evaluation metric on the device (experiments/experiment.py:436-463): Y channel of both [0,1] RGB batches exactly as
-// utils/utils.py:170-186 writes it -- 16/255 + (65.738 R + 129.057 G + 25.064 B) / 256, every operation rounded to fp32 in that order
-// (no FMA contraction) -- then the squared fp32 difference accumulated in double (skimage mean_squared_error: float32 squares, float64
-// mean).  Two fixed-order levels (thread -> warp tree -> CTA partial -> per-image sum): bitwise reproducible, no atomics.
+// utils/utils.py:170-186 writes it (y_channel, ycbcr.cuh), then the squared fp32 difference accumulated in double (skimage
+// mean_squared_error: float32 squares, float64 mean).  Two fixed-order levels (thread -> warp tree -> CTA partial -> per-image sum):
+// bitwise reproducible, no atomics.
 constexpr int kPsnrChunk = 4096;                           // pixels per CTA
-__device__ __forceinline__ float y_channel(float r, float g, float b) {
-  const float t = __fadd_rn(__fadd_rn(__fmul_rn(65.738f, r), __fmul_rn(129.057f, g)), __fmul_rn(25.064f, b));
-  return __fadd_rn((float)(16.0 / 255.0), __fdiv_rn(t, 256.0f));
-}
 __global__ void __launch_bounds__(256) psnr_y_partial_kernel(const float* __restrict__ sr, const float* __restrict__ hr, long long HW, int clip,
                                                              double* __restrict__ partial) {
   __shared__ double s_w[8];

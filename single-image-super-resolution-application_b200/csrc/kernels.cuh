@@ -66,6 +66,14 @@ int launch_x8_entry(const float* x, const uint8_t* x_u8hwc, float* xt, int B, in
 // first term; last: * 0.125f, and y_u8hwc != nullptr writes uint8 [B,Hd,Wd,C] as launch_f32nchw_to_u8hwc instead of acc
 int launch_x8_combine(const float* z, float* acc, uint8_t* y_u8hwc, int B, int C, int Hd, int Wd, int k0, int g, int first, int last, cudaStream_t st);
 
+// ---- ssim.cu (Y-channel SSIM of two [0,1] fp32 NCHW RGB batches, skimage structural_similarity(hr_y, sr_y, data_range=1)) ----
+// window radius 3 (uniform 7x7) or 5 (Gaussian sigma 1.5, 11 taps); tiles per image of the interior, 0 when H or W < the window
+int ssim_y_radius(int gaussian);
+long long ssim_y_tiles(int H, int W, int gaussian);
+// partial: B * ssim_y_tiles doubles; ssim[b] = mean of the SSIM map over the interior of image b
+int launch_ssim_y(const float* sr, const float* hr, int B, int H, int W, int clip, int gaussian, int sample_cov, double* partial, double* ssim,
+                  cudaStream_t st);
+
 // ---- casa (SpatialChannelAttention, hit_sir_pro.py:338-359) ------------------------------
 struct CasaW {
   const float* w1; const float* b1;      // linear1: Conv2d(1,C,3) as [9][C], [C]
