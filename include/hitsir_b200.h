@@ -227,8 +227,8 @@ HITSIR_API int hitsir_profile_enable(HitsirHandle* h, int on);
 HITSIR_API int hitsir_profile_num_categories(const HitsirHandle* h);
 HITSIR_API int hitsir_profile_get(HitsirHandle* h, int index, const char** name, double* total_ms, int64_t* launches);
 
-/* "umma" (tcgen05 path with TMA-staged epilogues), the only backend of the product library.  A test build with -DHITSIR_AB_PATHS
- * additionally accepts "umma_direct" (same mainloop, per-row global stores, unfused FFN tail) and "simt" (fp32 cross-check kernels). */
+/* "umma" (tcgen05 path with TMA-staged epilogues) is the only backend.  Any other name returns HITSIR_ERR_INVALID, and
+ * hitsir_last_error() names the rejected backend. */
 HITSIR_API int hitsir_set_gemm_backend(HitsirHandle* h, const char* backend);
 
 HITSIR_API const char* hitsir_last_error(void);

@@ -99,8 +99,8 @@ class HitsirError(RuntimeError):
 
 
 def library_path() -> str:
-    """The in-tree product library.  HITSIR_B200_LIB names another build of the SAME sources (build.py variants for kernel
-    experiments and the -DHITSIR_AB_PATHS cross-check build used by tests); it is never a different backend."""
+    """The in-tree product library.  HITSIR_B200_LIB names another build of this library (a build.py variant for a kernel
+    experiment, or an earlier commit's build for an A/B comparison); it is never a different backend."""
     return os.environ.get("HITSIR_B200_LIB") or _build.LIB
 
 

@@ -20,9 +20,6 @@ BUILD = os.path.join(HERE, "build")
 LIB = os.path.join(HERE, "libhitsir_b200.so")
 SOURCES = ["engine.cu", "umma_gemm.cu", "umma_gemm_tma.cu", "conv3_c64.cu", "ffn_tail.cu", "scc_umma.cu", "scc_dense.cu", "glue.cu", "pack.cu",
            "ensemble.cu", "ssim.cu"]
-# A/B cross-check kernels (SIMT GEMM, stand-alone depthwise conv, SIMT casa gate, the slower proj+fc1 chain): compiled only into a test
-# build (`build.py --ab` -> libhitsir_b200_ab.so, -DHITSIR_AB_PATHS); the product library has one path and no switches
-AB_SOURCES = ["proj_fc1.cu", "simt_ref.cu"]
 HEADERS = ["common.cuh", "gemm.cuh", "kernels.cuh", "ycbcr.cuh", os.path.join("..", "..", "include", "hitsir_b200.h")]
 NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
 FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
@@ -31,7 +28,7 @@ FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std
 
 def _digest() -> str:
     h = hashlib.sha256()
-    for name in SOURCES + AB_SOURCES + HEADERS:
+    for name in SOURCES + HEADERS:
         with open(os.path.join(CSRC, name), "rb") as f:
             h.update(name.encode())
             h.update(f.read())
@@ -46,22 +43,21 @@ def _run(cmd):
     return r.stdout
 
 
-def build(force: bool = False, verbose: bool = False, ab: bool = False, defines=(), lib: str = None) -> str:
+def build(force: bool = False, verbose: bool = False, defines=(), lib: str = None) -> str:
     """Compile every CUDA source for sm_100a and link the shared library.  Returns its path.
-    ab=True builds the A/B test library (libhitsir_b200_ab.so) with the cross-check kernels; `defines` adds -D flags to a variant
-    build written to `lib` (kernel experiments: several variants travel to the GPU box in one snapshot)."""
-    variant = bool(ab or defines or lib)
-    tag = "ab" if ab and not defines and lib is None else (os.path.splitext(os.path.basename(lib))[0] if lib else "var")
+    `defines` adds -D flags to a variant build written to `lib` (kernel experiments: several variants travel to the GPU box in one
+    snapshot)."""
+    variant = bool(defines or lib)
+    tag = os.path.splitext(os.path.basename(lib))[0] if lib else "var"
     bdir = os.path.join(BUILD, tag) if variant else BUILD
-    out_lib = lib or (os.path.join(HERE, "libhitsir_b200_ab.so") if ab else LIB)
+    out_lib = lib or LIB
     os.makedirs(bdir, exist_ok=True)
     stamp = os.path.join(bdir, "stamp.txt")
-    extra = (["-DHITSIR_AB_PATHS"] if ab else []) + ["-D" + d for d in defines]
+    extra = ["-D" + d for d in defines]
     digest = _digest() + " " + " ".join(extra)
     if not force and os.path.exists(out_lib) and os.path.exists(stamp) and open(stamp).read().strip() == digest:
         return out_lib
-    sources = SOURCES + (AB_SOURCES if ab else [])
-    objs = [os.path.join(bdir, s.replace(".cu", ".o")) for s in sources]
+    objs = [os.path.join(bdir, s.replace(".cu", ".o")) for s in SOURCES]
 
     def compile_one(pair):
         src, obj = pair
@@ -69,8 +65,8 @@ def build(force: bool = False, verbose: bool = False, ab: bool = False, defines=
         if verbose and out.strip():
             print(out)
 
-    with ThreadPoolExecutor(max_workers=min(len(sources), os.cpu_count() or 4)) as ex:
-        list(ex.map(compile_one, zip(sources, objs)))
+    with ThreadPoolExecutor(max_workers=min(len(SOURCES), os.cpu_count() or 4)) as ex:
+        list(ex.map(compile_one, zip(SOURCES, objs)))
     _run([NVCC, "-shared", "-gencode", "arch=compute_100a,code=sm_100a", "-Xcompiler", "-fPIC", "-o", out_lib] + objs)
     with open(stamp, "w") as f:
         f.write(digest)
@@ -78,4 +74,4 @@ def build(force: bool = False, verbose: bool = False, ab: bool = False, defines=
 
 
 if __name__ == "__main__":
-    print(build(force="--force" in sys.argv, verbose=True, ab="--ab" in sys.argv))
+    print(build(force="--force" in sys.argv, verbose=True))

@@ -6,7 +6,6 @@
 #include <stdint.h>
 #include <stdio.h>
 
-#ifndef HITSIR_CHECK
 #define HITSIR_CHECK(expr)                                                              \
   do {                                                                                  \
     cudaError_t _e = (expr);                                                            \
@@ -15,7 +14,6 @@
       return 1;                                                                         \
     }                                                                                   \
   } while (0)
-#endif
 
 namespace hitsir {
 
@@ -47,43 +45,19 @@ static inline int round_up(int a, int b) { return cdiv(a, b) * b; }
 __device__ __forceinline__ float gelu_erf(float x) {          // nn.GELU() default (erf form)
   return 0.5f * x * (1.0f + erff(x * 0.70710678118654752440f));
 }
-// erf by Abramowitz-Stegun 7.1.26 (|error| <= 1.5e-7, far below the bf16 rounding of the stored value):
-// branch-free, one MUFU.RCP + one MUFU.EX2 -- the epilogue is instruction-bound, erff() costs 3x more.
-__device__ __forceinline__ float gelu_fast(float x) {
-  const float ax = fabsf(x) * 0.70710678118654752440f;
-  const float t = __frcp_rn(fmaf(0.3275911f, ax, 1.0f));
-  float poly = fmaf(1.061405429f, t, -1.453152027f);
-  poly = fmaf(poly, t, 1.421413741f);
-  poly = fmaf(poly, t, -0.284496736f);
-  poly = fmaf(poly, t, 0.254829592f);
-  const float e = poly * t * __expf(-ax * ax);        // 1 - erf(|x|/sqrt2)
-  const float erf_abs = 1.0f - e;
-  return 0.5f * x * (1.0f + copysignf(erf_abs, x));
-}
-
-// Packed-fp32 GELU (erf form, /root/reference/models/hit_sir_pro.py:32 nn.GELU) for two values: x * Phi(x) with
-// Phi(x) ~= 1 / (1 + 2^(-x (a + b s + c s^2))), s = min(x^2, 81): a minimax fit of the normal CDF by a logistic of an odd quintic.
-// |error| <= 1.6e-5 * max(|x|, 1) (fp32 evaluation and ex2.approx / rcp.approx included), two orders of magnitude below the bf16 rounding of
-// the stored value.  6 packed FMA-pipe instructions + 2 FMNMX + 4 MUFU per pair (the polynomial-only form needed 12 + 4 FMNMX: the FMA pipe
-// is the binding resource of the FFN kernels, the MUFU pipe is otherwise idle).  Saturates exactly: 2^z -> inf gives 0, 2^z -> 0 gives x.
 __device__ __forceinline__ float ex2_approx(float x) { float y; asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(x)); return y; }
 __device__ __forceinline__ float rcp_approx(float x) { float y; asm("rcp.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(x)); return y; }
-__device__ __forceinline__ float2 gelu2_exact(float2 x) {
-  float2 s = __fmul2_rn(x, x);
-  s.x = fminf(s.x, 81.f); s.y = fminf(s.y, 81.f);          // the quintic turns over at |x| ~ 11.4; beyond 9 the logistic is saturated anyway
-  float2 p = __ffma2_rn(s, make_float2(9.481962249e-04f, 9.481962249e-04f), make_float2(-1.064097551e-01f, -1.064097551e-01f));
-  p = __ffma2_rn(p, s, make_float2(-2.301458255f, -2.301458255f));
-  const float2 z = __fmul2_rn(p, x);
-  const float2 e = __fadd2_rn(make_float2(ex2_approx(z.x), ex2_approx(z.y)), make_float2(1.f, 1.f));
-  return __fmul2_rn(x, make_float2(rcp_approx(e.x), rcp_approx(e.y)));
-}
-// The same logistic written with ONE MUFU op per value: 1 / (1 + 2^z) = (1 + tanh(-z ln2 / 2)) / 2, so x Phi(x) = hx + hx tanh(w) with hx = x / 2,
-// w = x (a' + b' s + c' s^2) (the quintic scaled by ln2 / 2).  5 packed FMA-pipe instructions + 2 FMNMX + 2 MUFU per pair instead of 6 + 2 + 4: the fc1
-// epilogue was MUFU-bound (67 % of the pipe, profiles/r1i).  tanh.approx.f32 has a relative error of 2^-11, i.e. an ABSOLUTE error of up to
-// 2.4e-4 |x| on the result (where x < 0 the result itself is smaller than that) -- an eighth of the bf16 rounding step of a stored value of
-// magnitude |x|, which is what the consumers of h1 / h2 see anyway.
 __device__ __forceinline__ float tanh_approx(float x) { float y; asm("tanh.approx.f32 %0, %1;" : "=f"(y) : "f"(x)); return y; }
-__device__ __forceinline__ float2 gelu2_tanh(float2 x) {
+// Packed-fp32 GELU (erf form, hit_sir_pro.py:32 nn.GELU) for two values: x * Phi(x) with
+// Phi(x) ~= 1 / (1 + 2^(-x (a + b s + c s^2))), s = min(x^2, 81): a minimax fit of the normal CDF by a logistic of an odd quintic
+// (|error| <= 1.6e-5 * max(|x|, 1) evaluated in fp32 with ex2.approx / rcp.approx; the quintic turns over at |x| ~ 11.4, beyond 9 the logistic
+// is saturated anyway).  The logistic is written with ONE MUFU op per value: 1 / (1 + 2^z) = (1 + tanh(-z ln2 / 2)) / 2, so
+// x Phi(x) = hx + hx tanh(w) with hx = x / 2, w = x (a' + b' s + c' s^2) (the quintic scaled by ln2 / 2).  5 packed FMA-pipe instructions + 2 FMNMX + 2 MUFU per pair, against 6 + 2 + 4 for
+// the ex2 + rcp form and 12 + 4 FMNMX for a polynomial-only form: the FMA pipe is the binding resource of the FFN kernels, and the fc1
+// epilogue was MUFU-bound with the ex2 + rcp form (67 % of the pipe, profiles/r1i).  tanh.approx.f32 has a relative error of 2^-11, i.e. an
+// ABSOLUTE error of up to 2.4e-4 |x| on the result (where x < 0 the result itself is smaller than that) -- an eighth of the bf16 rounding step
+// of a stored value of magnitude |x|, which is what the consumers of h1 / h2 see anyway.
+__device__ __forceinline__ float2 gelu2(float2 x) {
   float2 s = __fmul2_rn(x, x);
   s.x = fminf(s.x, 81.f); s.y = fminf(s.y, 81.f);
   float2 p = __ffma2_rn(s, make_float2(-3.286197700e-04f, -3.286197700e-04f), make_float2(3.687881087e-02f, 3.687881087e-02f));
@@ -92,11 +66,6 @@ __device__ __forceinline__ float2 gelu2_tanh(float2 x) {
   const float2 hx = __fmul2_rn(x, make_float2(0.5f, 0.5f));
   return __ffma2_rn(hx, make_float2(tanh_approx(w.x), tanh_approx(w.y)), hx);
 }
-#ifdef HITSIR_GELU_EXACT
-__device__ __forceinline__ float2 gelu2(float2 x) { return gelu2_exact(x); }
-#else
-__device__ __forceinline__ float2 gelu2(float2 x) { return gelu2_tanh(x); }
-#endif
 
 __device__ __forceinline__ float lrelu(float x, float slope) { return x > 0.f ? x : x * slope; }
 __device__ __forceinline__ float sigmoidf_(float x) { return 1.0f / (1.0f + __expf(-x)); }
@@ -126,11 +95,6 @@ __device__ __forceinline__ float warp_max(float v) {
 #pragma unroll
   for (int o = 16; o > 0; o >>= 1) v = fmaxf(v, __shfl_xor_sync(0xffffffffu, v, o));
   return v;
-}
-// float atomic max via ordered-int trick (works for any sign, buffer initialised to -inf)
-__device__ __forceinline__ void atomic_max_float(float* addr, float v) {
-  if (v >= 0.f) atomicMax(reinterpret_cast<int*>(addr), __float_as_int(v));
-  else atomicMin(reinterpret_cast<unsigned int*>(addr), __float_as_uint(v));
 }
 
 // ---------------------------------------------------------------------------
@@ -184,14 +148,9 @@ __device__ __forceinline__ void mbar_wait_park(uint32_t bar, uint32_t parity, ui
 // become resident while its predecessor in the stream is still draining; pdl_entry() holds it until that grid has completed and its
 // writes are visible, then lets the NEXT launch in the stream do the same.  Everything before pdl_entry() may only touch memory that no
 // kernel of the forward writes (weights, shared memory, TMEM, barriers).  Kernels launched without the attribute see a no-op.
-#ifndef HITSIR_PDL
-#define HITSIR_PDL 1
-#endif
 __device__ __forceinline__ void pdl_entry() {
-#if HITSIR_PDL
   asm volatile("griddepcontrol.wait;" ::: "memory");
   asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
-#endif
 }
 template <class... KArgs, class... Args>
 static inline cudaError_t launch_pdl(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t st, Args&&... args) {
@@ -200,7 +159,7 @@ static inline cudaError_t launch_pdl(void (*kernel)(KArgs...), dim3 grid, dim3 b
   cudaLaunchAttribute at[1];
   at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
   at[0].val.programmaticStreamSerializationAllowed = 1;
-  cfg.attrs = at; cfg.numAttrs = HITSIR_PDL ? 1 : 0;
+  cfg.attrs = at; cfg.numAttrs = 1;
   return cudaLaunchKernelEx(&cfg, kernel, static_cast<KArgs>(args)...);
 }
 __device__ __forceinline__ void fence_barrier_init() {

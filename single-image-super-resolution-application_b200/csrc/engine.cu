@@ -100,14 +100,6 @@ struct HitsirHandle {
   HitsirConfig cfg;
   int device = 0;
   int num_sms = 148;
-  // A/B switches: only a test build (-DHITSIR_AB_PATHS, build.py --ab) can turn them on; the product has ONE path and they stay false
-  bool simt = false;
-  bool projfc1_fused = false;     // HITSIR_PROJFC1=fused: proj + fc1 chained in one kernel (proj_fc1.cu; slower than the two GEMM launches so far, DESIGN.md 3.7)
-  bool b_streamed = false;        // HITSIR_GEMMW=streamed: linears re-load their weight tile per 128-token tile (A/B switch)
-  bool no_epilogue_stats = false; // HITSIR_STATS=kernel: always compute the casa statistics with the stand-alone sca_stats pass
-  bool ffn_unfused = false;       // HITSIR_FFN=unfused: separate dwconv5 and fc2 kernels for every block
-  bool scc_gram_only = false;     // HITSIR_SCC=gram: use the Gram-matrix kernel (scc_umma.cu) for every window size
-  bool direct_epilogue = false;   // HITSIR_EPILOGUE=direct: per-row global stores instead of the TMA-staged epilogue
   std::vector<ParamSpec> params;
   std::map<std::string, int> index;
   float* arena = nullptr;      // device fp32 master copy of every parameter
@@ -724,8 +716,7 @@ void base_params(GemmParams& p, const GemmW& w) {
 
 // The staged-epilogue kernel covers the plain-store and LayerNorm epilogues; the gate / pixel-shuffle
 // epilogues (once per forward) keep the direct-store kernel.
-bool tma_epilogue(const HitsirHandle* h, const GemmW& w, const GemmParams& p) {
-  if (h->simt || h->direct_epilogue) return false;
+bool tma_epilogue(const GemmW& w, const GemmParams& p) {
   if (p.epi == EPI_MSGATE) return w.BN == 160;
   return (p.epi == EPI_STORE || p.epi == EPI_LN) && (w.BN == 192 || w.BN == 64) && p.out2_f32 == nullptr && w.Npad <= 384;
 }
@@ -733,9 +724,6 @@ bool tma_epilogue(const HitsirHandle* h, const GemmW& w, const GemmParams& p) {
 int run_gemm(Fwd& f, const char* cat, const GemmW& w, GemmParams& p, const CUtensorMap* maps, bool tma) {
   ProfScope ps(f.h, f.st, cat);
   f.h->launches++;
-#ifdef HITSIR_AB_PATHS
-  if (f.h->simt) return launch_simt_gemm(w.BN, p, f.st);
-#endif
   if (tma) return launch_umma_gemm_tma(w.BN, p, maps, f.h->num_sms, f.st);
   return launch_umma_gemm(w.BN, p, maps[0], w.tm, f.h->num_sms, f.st);
 }
@@ -744,18 +732,16 @@ int run_gemm(Fwd& f, const char* cat, const GemmW& w, GemmParams& p, const CUten
 int linear(Fwd& f, const char* cat, const GemmW& w, const bf16* A, long long M, GemmParams& p) {
   p.conv = 0; p.M = (int)M; p.m_tiles = (int)cdiv64(M, 128);
   p.A = A; p.lda = w.K;
-  p.b_resident = f.h->b_streamed ? 0 : 1;                  // honoured by the TMA kernel when the weight tile fits next to the A ring
+  p.b_resident = 1;                                        // honoured by the TMA kernel when the weight tile fits next to the A ring
 
   CUtensorMap maps[5];
-  const bool tma = tma_epilogue(f.h, w, p);
-  if (!f.h->simt) {
-    if (make_tmap_2d(&maps[0], A, (uint64_t)w.K, (uint64_t)M, (uint64_t)w.K * 2, 64, 128)) return 1;
-    maps[1] = w.tm; maps[2] = maps[0]; maps[3] = maps[0]; maps[4] = maps[0];
-    if (tma) {
-      if (p.out_f32 && make_tmap_2d_t(&maps[2], p.out_f32, 4, (uint64_t)p.n_real, (uint64_t)M, (uint64_t)p.ldf * 4, 32, 128)) return 1;
-      if (p.out_bf16 && make_tmap_2d_t(&maps[3], p.out_bf16, 2, (uint64_t)p.ldb, (uint64_t)M, (uint64_t)p.ldb * 2, 64, 128)) return 1;
-      if (p.res && make_tmap_2d_t(&maps[4], p.res, 4, (uint64_t)p.n_real, (uint64_t)M, (uint64_t)p.ldr * 4, 32, 128)) return 1;
-    }
+  const bool tma = tma_epilogue(w, p);
+  if (make_tmap_2d(&maps[0], A, (uint64_t)w.K, (uint64_t)M, (uint64_t)w.K * 2, 64, 128)) return 1;
+  maps[1] = w.tm; maps[2] = maps[0]; maps[3] = maps[0]; maps[4] = maps[0];
+  if (tma) {
+    if (p.out_f32 && make_tmap_2d_t(&maps[2], p.out_f32, 4, (uint64_t)p.n_real, (uint64_t)M, (uint64_t)p.ldf * 4, 32, 128)) return 1;
+    if (p.out_bf16 && make_tmap_2d_t(&maps[3], p.out_bf16, 2, (uint64_t)p.ldb, (uint64_t)M, (uint64_t)p.ldb * 2, 64, 128)) return 1;
+    if (p.res && make_tmap_2d_t(&maps[4], p.res, 4, (uint64_t)p.n_real, (uint64_t)M, (uint64_t)p.ldr * 4, 32, 128)) return 1;
   }
   return run_gemm(f, cat, w, p, maps, tma);
 }
@@ -774,7 +760,7 @@ int conv3(Fwd& f, const char* cat, const GemmW& w, const bf16* A, int B, int H, 
   p.A = A; p.lda = Cpad;
   if (w.K != 9 * Cpad) { set_error("conv3: packed K %d != 9*%d", w.K, Cpad); return 1; }
   // 64-channel inputs (HR stage): resident filter bank + kx-shared halo boxes (conv3_c64.cu)
-  if (!f.h->simt && !f.h->direct_epilogue && Cpad == 64 && p.res == nullptr && p.out2_f32 == nullptr &&
+  if (Cpad == 64 && p.res == nullptr && p.out2_f32 == nullptr &&
       ((w.BN == 64 && p.epi == EPI_STORE && p.out_bf16 != nullptr && p.out_f32 == nullptr && p.ldb == 64) ||
        (w.BN == 16 && w.wf != nullptr && p.res_img == nullptr && p.epi == EPI_SHUFFLE_NCHW && p.ps == 1 && p.n_real <= 4))) {
     ProfScope ps(f.h, f.st, cat);
@@ -783,15 +769,13 @@ int conv3(Fwd& f, const char* cat, const GemmW& w, const bf16* A, int B, int H, 
     return launch_conv3_c64(w.BN, p, A, w.tm, f.h->num_sms, f.st);
   }
   CUtensorMap maps[5];
-  const bool tma = tma_epilogue(f.h, w, p);
-  if (!f.h->simt) {
-    if (make_tmap_nhwc(&maps[0], A - (size_t)p.a_y_off * W * Cpad, B, H + 2 * p.a_y_off, W, Cpad, 64, 16, 8)) return 1;
-    maps[1] = w.tm; maps[2] = maps[0]; maps[3] = maps[0]; maps[4] = maps[0];
-    if (tma) {
-      if (p.out_f32 && make_tmap_nhwc_t(&maps[2], p.out_f32, 4, B, H, W, p.n_real, p.ldf, 32, 16, 8)) return 1;
-      if (p.out_bf16 && make_tmap_nhwc_t(&maps[3], p.out_bf16, 2, B, H, W, p.ldb, p.ldb, 64, 16, 8)) return 1;
-      if (p.res && make_tmap_nhwc_t(&maps[4], p.res, 4, B, H, W, p.n_real, p.ldr, 32, 16, 8)) return 1;
-    }
+  const bool tma = tma_epilogue(w, p);
+  if (make_tmap_nhwc(&maps[0], A - (size_t)p.a_y_off * W * Cpad, B, H + 2 * p.a_y_off, W, Cpad, 64, 16, 8)) return 1;
+  maps[1] = w.tm; maps[2] = maps[0]; maps[3] = maps[0]; maps[4] = maps[0];
+  if (tma) {
+    if (p.out_f32 && make_tmap_nhwc_t(&maps[2], p.out_f32, 4, B, H, W, p.n_real, p.ldf, 32, 16, 8)) return 1;
+    if (p.out_bf16 && make_tmap_nhwc_t(&maps[3], p.out_bf16, 2, B, H, W, p.ldb, p.ldb, 64, 16, 8)) return 1;
+    if (p.res && make_tmap_nhwc_t(&maps[4], p.res, 4, B, H, W, p.n_real, p.ldr, 32, 16, 8)) return 1;
   }
   return run_gemm(f, cat, w, p, maps, tma);
 }
@@ -843,7 +827,7 @@ int forward_block(Fwd& f, int i, int j, float* xin, float* xout) {
   }
   if (c.is_channel_spatial_attn) {
     int nparts = f.stats_nparts;
-    if (nparts == 0) {       // no producer epilogue delivered them (first block of a layer, unfused fallback): one pass over the stream
+    if (nparts == 0) {       // no producer epilogue delivered them (first block of a layer): one pass over the stream
       nparts = ws.nparts;
       LAUNCH("sca_stats", 1, launch_sca_stats(xin, g.pg, ws.cavg, ws.cmax, ws.part_sum, ws.part_max, nparts, f.st));
     }
@@ -864,23 +848,15 @@ int forward_block(Fwd& f, int i, int j, float* xin, float* xout) {
   {
     const bool want_dbg = h->tap.dst != nullptr && h->tap.name == tn + ".sccdbg";
     char cat[16]; snprintf(cat, sizeof(cat), "scc_w%d", w);
-    if (g.r == 1 && !want_dbg && !h->scc_gram_only)
+    if (g.r == 1 && !want_dbg)
       LAUNCH(cat, 1, launch_scc_dense(ws.T, g, bw.scc, ws.outsc, h->num_sms, f.st));
     else
       LAUNCH(cat, 1, launch_scc_umma(ws.T, g, bw.scc, ws.outsc, want_dbg ? ws.scc_dbg : nullptr, h->num_sms, f.st));
   }
   TAP((tn + ".sccdbg").c_str(), ws.scc_dbg, 0, kSccDbgFloats, 1, kSccDbgFloats);
   TAPP((tn + ".scc").c_str(), ws.outsc, 1, kCp, f.N, kC);
-  GemmParams p;
-#ifdef HITSIR_AB_PATHS
-  if (!h->simt && !h->direct_epilogue && h->projfc1_fused && bw.proj.BN == 192 && bw.proj.K == 192 && bw.fc1.K == 192 && bw.fc1.Npad == 384) {
-    // proj + norm1 + residual and fc1 + GELU in one kernel (:597, :700-703, :39-41)
-    LAUNCH("proj_fc1", 1, launch_proj_fc1(ws.outsc, bw.proj.tm, bw.proj.b, bw.g1, bw.b1, xin, xout, bw.fc1.w, bw.fc1.b, ws.H1, f.N, h->num_sms, f.st));
-    TAP((tn + ".attn").c_str(), xout, 0, kC, f.N, kC);
-  } else
-#endif
-  {
   // proj + norm1 + residual (:597, :700-703)
+  GemmParams p;
   base_params(p, bw.proj);
   p.epi = EPI_LN; p.n_real = kC; p.gamma = bw.g1; p.beta = bw.b1; p.res = xin; p.ldr = kC;
   p.out_f32 = xout; p.ldf = kC; p.out_bf16 = ws.xb0; p.ldb = kCp;
@@ -890,39 +866,23 @@ int forward_block(Fwd& f, int i, int j, float* xin, float* xout) {
   base_params(p, bw.fc1);
   p.epi = EPI_STORE; p.act = ACT_GELU; p.n_real = kHid; p.out_bf16 = ws.H1; p.ldb = kHidp;
   RUN(linear(f, "gemm_fc1_gelu", bw.fc1, ws.xb0, f.N, p));
-  }
   TAP((tn + ".fc1").c_str(), ws.H1, 1, kHidp, f.N, kHid);
   const bool need_shadow = (j == c.depths[i] - 1);      // the RHTB conv after the last block reads a bf16 shadow of the stream (:934)
-  if (!h->simt && !h->direct_epilogue && !h->ffn_unfused) {
-    // dwconv5 + GELU + input, fc2, norm2 and the residual add in one kernel: the hidden map h2 never reaches HBM
-    // ... and, when another block of this layer follows, the casa statistics of the new stream for that block's window padding
-    FfnStats fs; const FfnStats* fsp = nullptr;
-    if (c.is_channel_spatial_attn && !need_shadow && !h->no_epilogue_stats) {
-      const int wn = h->blocks[i][j + 1].win;
-      fs = FfnStats{ws.cavg, ws.cmax, ws.part_sum, ws.part_max, round_up(f.band ? f.Hf : f.H, wn), round_up(f.W, wn)};
-      fsp = &fs;
-    }
-    bf16* shadow = (need_shadow && fsp == nullptr) ? ws.xb0 : nullptr;      // emitted by the kernel's statistics warp
-    FfnBand fb{2, f.row0, f.Hf};
-    if (f.band != nullptr) RUN(fill_halo(f, ws.H1, (size_t)f.W * kHidp * sizeof(bf16), f.H, 2));   // the depthwise 5x5 reads two rows across the band edge
-    LAUNCH("ffn_tail", 1, launch_ffn_tail(ws.H1, bw.dw_mma, bw.w2_img, bw.fc2.b, bw.g2, bw.b2, xout, f.B, f.H, f.W, fsp, shadow, h->num_sms, f.st,
-                                          f.band ? &fb : nullptr));
-    if (fsp != nullptr) f.stats_nparts = ffn_tiles_per_image(f.H, f.W);
-    if (need_shadow && shadow == nullptr) LAUNCH("cast_shadow", 1, launch_cast_rows_bf16(xout, ws.xb0, f.N, f.st));
-  } else {
-#ifdef HITSIR_AB_PATHS
-    LAUNCH("dwconv5", 1, launch_dwconv5_gelu_add(ws.H1, bw.dw_w, bw.dw_b, ws.H2, f.B, f.H, f.W, h->num_sms, f.st));
-    // fc2 + norm2 + residual (:704)
-    base_params(p, bw.fc2);
-    p.epi = EPI_LN; p.n_real = kC; p.gamma = bw.g2; p.beta = bw.b2; p.res = xout; p.ldr = kC;
-    p.out_f32 = xout; p.ldf = kC;
-    if (need_shadow) { p.out_bf16 = ws.xb0; p.ldb = kCp; }
-    RUN(linear(f, "gemm_fc2_ln", bw.fc2, ws.H2, f.N, p));
-#else
-    set_error("unfused FFN path is only available in the A/B test build (-DHITSIR_AB_PATHS)");
-    return HITSIR_ERR_UNSUPPORTED;
-#endif
+  // dwconv5 + GELU + input, fc2, norm2 and the residual add in one kernel: the hidden map h2 never reaches HBM
+  // ... and, when another block of this layer follows, the casa statistics of the new stream for that block's window padding
+  FfnStats fs; const FfnStats* fsp = nullptr;
+  if (c.is_channel_spatial_attn && !need_shadow) {
+    const int wn = h->blocks[i][j + 1].win;
+    fs = FfnStats{ws.cavg, ws.cmax, ws.part_sum, ws.part_max, round_up(f.band ? f.Hf : f.H, wn), round_up(f.W, wn)};
+    fsp = &fs;
   }
+  bf16* shadow = (need_shadow && fsp == nullptr) ? ws.xb0 : nullptr;      // emitted by the kernel's statistics warp
+  FfnBand fb{2, f.row0, f.Hf};
+  if (f.band != nullptr) RUN(fill_halo(f, ws.H1, (size_t)f.W * kHidp * sizeof(bf16), f.H, 2));   // the depthwise 5x5 reads two rows across the band edge
+  LAUNCH("ffn_tail", 1, launch_ffn_tail(ws.H1, bw.dw_mma, bw.w2_img, bw.fc2.b, bw.g2, bw.b2, xout, f.B, f.H, f.W, fsp, shadow, h->num_sms, f.st,
+                                        f.band ? &fb : nullptr));
+  if (fsp != nullptr) f.stats_nparts = ffn_tiles_per_image(f.H, f.W);
+  if (need_shadow && shadow == nullptr) LAUNCH("cast_shadow", 1, launch_cast_rows_bf16(xout, ws.xb0, f.N, f.st));
   TAP(tn.c_str(), xout, 0, kC, f.N, kC);
   return 0;
 }
@@ -1202,22 +1162,6 @@ HITSIR_API int hitsir_create(const HitsirConfig* cfg, HitsirHandle** out) {
   h->device = dev;
   h->num_sms = prop.multiProcessorCount;
   if (cfg->in_chans == 3) { h->mean[0] = 0.485f; h->mean[1] = 0.456f; h->mean[2] = 0.4060f; }   // (:1128)
-#ifdef HITSIR_AB_PATHS
-  const char* env = getenv("HITSIR_GEMM");
-  h->simt = env && strcmp(env, "simt") == 0;
-  const char* env5 = getenv("HITSIR_STATS");
-  h->no_epilogue_stats = env5 && strcmp(env5, "kernel") == 0;
-  const char* env7 = getenv("HITSIR_PROJFC1");
-  h->projfc1_fused = env7 && strcmp(env7, "fused") == 0;
-  const char* env8 = getenv("HITSIR_GEMMW");
-  h->b_streamed = env8 && strcmp(env8, "streamed") == 0;
-  const char* env4 = getenv("HITSIR_FFN");
-  h->ffn_unfused = env4 && strcmp(env4, "unfused") == 0;
-  const char* env3 = getenv("HITSIR_SCC");
-  h->scc_gram_only = env3 && strcmp(env3, "gram") == 0;
-  const char* env2 = getenv("HITSIR_EPILOGUE");
-  h->direct_epilogue = env2 && strcmp(env2, "direct") == 0;
-#endif
   build_param_list(h);
   e = cudaMalloc(reinterpret_cast<void**>(&h->arena), h->arena_floats * sizeof(float));
   if (e != cudaSuccess) { set_error("cudaMalloc(param arena): %s", cudaGetErrorString(e)); delete h; return HITSIR_ERR_CUDA; }
@@ -1459,13 +1403,7 @@ HITSIR_API int hitsir_profile_get(HitsirHandle* h, int i, const char** name, dou
 
 HITSIR_API int hitsir_set_gemm_backend(HitsirHandle* h, const char* backend) {
   if (!h || !backend) { set_error("null argument"); return HITSIR_ERR_INVALID; }
-  if (strcmp(backend, "umma") == 0) { h->simt = false; h->direct_epilogue = false; }
-#ifdef HITSIR_AB_PATHS
-  // the direct-store epilogues need the unfused FFN tail, which only this build compiles
-  else if (strcmp(backend, "umma_direct") == 0) { h->simt = false; h->direct_epilogue = true; }
-  else if (strcmp(backend, "simt") == 0) h->simt = true;
-#endif
-  else { set_error("unknown gemm backend '%s' (umma; 'umma_direct' and 'simt' only in the -DHITSIR_AB_PATHS test build)", backend); return HITSIR_ERR_INVALID; }
+  if (strcmp(backend, "umma") != 0) { set_error("unknown gemm backend '%s' (the only backend is 'umma')", backend); return HITSIR_ERR_INVALID; }
   return 0;
 }
 

@@ -24,11 +24,6 @@ namespace {
 
 constexpr int kPH = 12, kPW = 20;                         // halo patch of an 8 x 16 tile
 constexpr int kHalo = kPH * kPW * 128;                    // 30720 B, dense 128-byte pixel rows (no swizzle)
-#if defined(HITSIR_FFN_EXP) && (HITSIR_FFN_EXP & 4)
-constexpr int kHaloTx = 8 * 16 * 128, kBoxW = 16, kBoxH = 8;   // timing experiment (results wrong): no halo overfetch
-#else
-constexpr int kHaloTx = kHalo, kBoxW = kPW, kBoxH = kPH;
-#endif
 constexpr int kDwRow = 28;                                // words per channel of the tap table (kernels.cuh launch_pack_dw_mma)
 constexpr int kDwTbl = 64 * kDwRow * 4;                   // the slice's 64 channel rows
 constexpr int kHaloStage = 37 * 1024;                     // halo box + tap table, padded to keep the next region 1024-byte aligned
@@ -89,11 +84,6 @@ __device__ __forceinline__ void ldmatrix_x2(uint32_t addr, uint32_t& r0, uint32_
 // the four compute warps that share a TMEM lane quarter (= the same 32 pixel rows) exchange their LayerNorm / statistics partials
 __device__ __forceinline__ void epi_bar_sync(int q) { asm volatile("bar.sync %0, 128;" ::"r"(q + 1) : "memory"); }
 
-#ifdef HITSIR_SPIN_WAITS
-#define RWAIT(...) mbar_wait(__VA_ARGS__)
-#else
-#define RWAIT(...) mbar_wait_park(__VA_ARGS__)
-#endif
 __global__ void __launch_bounds__(640, 1)
 ffn_tail_kernel(const __grid_constant__ CUtensorMap tm_h1, const __grid_constant__ CUtensorMap tm_x, const Params p) {
   extern __shared__ uint8_t smem_raw[];
@@ -160,21 +150,11 @@ ffn_tail_kernel(const __grid_constant__ CUtensorMap tm_h1, const __grid_constant
         for (int k = 0; k < 6; ++k) {
           const int h = k & 1;
           const uint32_t u = (uint32_t)(it * 3 + (k >> 1));
-          RWAIT(halo_empty(h), (u & 1u) ^ 1u);
-#if defined(HITSIR_FFN_EXP) && (HITSIR_FFN_EXP & 1)
-          // timing experiment (results wrong): weights / tap rows fetched for the first tile only
-          if (it > 0) {
-            mbar_expect_tx(halo_full(h), kHaloTx);
-            tma_load_4d(sb + kOffHalo + h * kHaloStage, &tm_h1, halo_full(h), k * 64, x0 - 2, y0 - 2 + p.h1_y_off, b);
-            RWAIT(w_empty(h), (u & 1u) ^ 1u);
-            mbar_arrive(w_full(h));
-            continue;
-          }
-#endif
-          mbar_expect_tx(halo_full(h), kHaloTx + kDwTbl);
+          mbar_wait_park(halo_empty(h), (u & 1u) ^ 1u);
+          mbar_expect_tx(halo_full(h), kHalo + kDwTbl);
           tma_load_4d(sb + kOffHalo + h * kHaloStage, &tm_h1, halo_full(h), k * 64, x0 - 2, y0 - 2 + p.h1_y_off, b);
           bulk_load(sb + kOffHalo + h * kHaloStage + kHalo, p.dw_tbl + (size_t)k * (kDwTbl / 4), kDwTbl, halo_full(h));   // 64 contiguous tap rows
-          RWAIT(w_empty(h), (u & 1u) ^ 1u);
+          mbar_wait_park(w_empty(h), (u & 1u) ^ 1u);
           mbar_expect_tx(w_full(h), kWStage);
           bulk_load(sb + kOffWs + h * kWStage, p.w2_img + (size_t)k * kWStage, kWStage, w_full(h));   // pre-swizzled operand image: one request, not 192 rows
         }
@@ -187,14 +167,14 @@ ffn_tail_kernel(const __grid_constant__ CUtensorMap tm_h1, const __grid_constant
       int it = 0;
       for (int t = blockIdx.x; t < p.total; t += gridDim.x, ++it) {
         const int as = it & 1;
-        RWAIT(d_empty(as), (((uint32_t)(it >> 1)) & 1u) ^ 1u);
+        mbar_wait_park(d_empty(as), (((uint32_t)(it >> 1)) & 1u) ^ 1u);
         tc_fence_after();
         const uint32_t d_tmem = tmem_base + (uint32_t)(as * 192);
         for (int k = 0; k < 6; ++k) {
           const int h = k & 1;
           const uint32_t u = (uint32_t)(it * 3 + (k >> 1));
-          RWAIT(a_full(h), u & 1u);
-          RWAIT(w_full(h), u & 1u);
+          mbar_wait_park(a_full(h), u & 1u);
+          mbar_wait_park(w_full(h), u & 1u);
           tc_fence_after();
           const uint64_t adesc = umma_desc_sw128(sb + kOffA + h * kABuf);
           const uint64_t bdesc = umma_desc_sw128(sb + kOffWs + h * kWStage);
@@ -220,7 +200,7 @@ ffn_tail_kernel(const __grid_constant__ CUtensorMap tm_h1, const __grid_constant
         __syncwarp();
         for (int j = 0; j < 6; ++j, ++u) {
           const int s = (int)(u % kNBox);
-          RWAIT(out_bar(s), (u / kNBox) & 1u);
+          mbar_wait_park(out_bar(s), (u / kNBox) & 1u);
           const uint8_t* box = sp + kOffBox + s * kBoxBytes;
           const int ck = lane & 7, rph = lane >> 3;
           float4 sum = make_float4(0.f, 0.f, 0.f, 0.f), mx = make_float4(-INFINITY, -INFINITY, -INFINITY, -INFINITY);
@@ -257,7 +237,7 @@ ffn_tail_kernel(const __grid_constant__ CUtensorMap tm_h1, const __grid_constant
         int x0, y0, b; tile_xyb(t, &x0, &y0, &b);
         for (int j = 0; j < 6; ++j, ++u) {
           const int s = (int)(u % kNBox);
-          RWAIT(out_bar(s), (u / kNBox) & 1u);
+          mbar_wait_park(out_bar(s), (u / kNBox) & 1u);
           const uint8_t* box = sp + kOffBox + s * kBoxBytes;
 #pragma unroll 4
           for (int i = lane; i < 512; i += 32) {            // 128 pixels x 4 chunks of 8 channels
@@ -281,10 +261,8 @@ ffn_tail_kernel(const __grid_constant__ CUtensorMap tm_h1, const __grid_constant
       uint32_t u_prep = 0, u_store = 0;
       auto store_one = [&]() {
         const int s = (int)(u_store % kNBox);
-        RWAIT(out_bar(s), (u_store / kNBox) & 1u);
-#if !(defined(HITSIR_FFN_EXP) && (HITSIR_FFN_EXP & 2))
+        mbar_wait_park(out_bar(s), (u_store / kNBox) & 1u);
         tma_store_4d(&tm_x, sb + kOffBox + s * kBoxBytes, c0s[s], r0s[s], r1s[s], r2s[s]);
-#endif
         tma_commit();
         ++u_store;
       };
@@ -296,12 +274,9 @@ ffn_tail_kernel(const __grid_constant__ CUtensorMap tm_h1, const __grid_constant
             const uint32_t need = u_prep - (uint32_t)kNBox + 2u;
             while (u_store < need && u_store < u_prep) store_one();
             tma_wait_read1();                              // bulk groups retire in order: store #(u_prep - kNBox) has left the box
-            if (want_stats || want_shadow) RWAIT(red_done(s), ((u_prep / kNBox) - 1u) & 1u);   // ... and the statistics warp has read it
+            if (want_stats || want_shadow) mbar_wait_park(red_done(s), ((u_prep / kNBox) - 1u) & 1u);   // ... and the statistics warp has read it
           }
           c0s[s] = 32 * j; r0s[s] = x0; r1s[s] = y0; r2s[s] = b;
-#if defined(HITSIR_FFN_EXP) && (HITSIR_FFN_EXP & 2)
-          if (u_prep >= (uint32_t)kNBox) { mbar_arrive(in_bar(s)); ++u_prep; continue; }      // timing experiment: no residual loads after the first boxes
-#endif
           mbar_expect_tx(in_bar(s), kBoxBytes);
           tma_load_4d(sb + kOffBox + s * kBoxBytes, &tm_x, in_bar(s), 32 * j, x0, y0, b);
           ++u_prep;
@@ -542,7 +517,7 @@ int launch_ffn_tail(const bf16* h1, const uint32_t* dw_tbl_mma, const uint8_t* w
   if (band && B != 1) { set_error("launch_ffn_tail: band mode needs B == 1"); return 1; }
   CUtensorMap tm_h1, tm_x;
   // SWIZZLE_128B halo boxes, zero fill outside the image; band mode: the map starts h1_y_off rows above image row 0 (rows filled by the neighbour)
-  if (make_tmap_nhwc(&tm_h1, h1 - (size_t)p.h1_y_off * W * kHidp, B, H + 2 * p.h1_y_off, W, kHidp, 64, kBoxW, kBoxH)) return 1;
+  if (make_tmap_nhwc(&tm_h1, h1 - (size_t)p.h1_y_off * W * kHidp, B, H + 2 * p.h1_y_off, W, kHidp, 64, kPW, kPH)) return 1;
   if (make_tmap_nhwc_t(&tm_x, x, 4, B, H, W, kC, kC, 32, 16, 8)) return 1;
   const int grid = p.total < num_sms ? p.total : num_sms;
   HITSIR_CHECK(launch_pdl(ffn_tail_kernel, dim3(grid), dim3(640), kSmemBytes, st, tm_h1, tm_x, p));

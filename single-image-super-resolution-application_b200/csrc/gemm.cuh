@@ -1,5 +1,5 @@
-// Dense-contraction front end shared by the tcgen05 kernel (umma_gemm.cu) and the
-// SIMT cross-check kernel (simt_ref.cu): problem description + the fused epilogue.
+// Dense-contraction front end of the tcgen05 kernels (umma_gemm.cu, umma_gemm_tma.cu, conv3_c64.cu): problem description + the
+// fused epilogue of the direct-store kernel.
 //
 // One "problem" is  D[M, N] = A[M, K] * Wp[N, K]^T  with bf16 operands and fp32 accumulation:
 //   * linear:  A is a token-major activation [M, K] (K padded to a multiple of 64);
@@ -47,12 +47,12 @@ struct GemmParams {
   float out_scale;   // 1 / img_range
   float mean[4];     // per-channel mean added after scaling (NCHW)
   const float* res_img;   // EPI_SHUFFLE_NCHW, ps == 1: NCHW fp32 image added INSTEAD of the mean (upsampler=None: x + conv_last(res), :1340-1342)
-  // debug / SIMT cross-check operand views
+  // operand views for debugging (no kernel reads them: the kernels take tensor maps)
   const bf16* A; int lda;         // linear: [M, lda]; conv: NHWC base with lda = Cin_pad
   const bf16* Wp; int ldw;        // [n_tiles*BN, ldw]
 };
 
-// Row bookkeeping shared by both kernels
+// Row bookkeeping of the direct-store kernel
 struct RowInfo {
   bool valid;
   long long grow;   // linear row / NHWC pixel index
@@ -256,7 +256,7 @@ __device__ __forceinline__ void epilogue_row(const GemmParams& p, Acc& acc, cons
   }
 }
 
-// host-side launchers (umma_gemm.cu / simt_ref.cu)
+// host-side launchers (umma_gemm.cu)
 struct TensorMaps {
   CUtensorMap a, b;
 };
@@ -266,7 +266,6 @@ int make_tmap_2d_t(CUtensorMap* m, const void* base, int elem_bytes, uint64_t in
 int make_tmap_nhwc_t(CUtensorMap* m, const void* base, int elem_bytes, int B, int H, int W, int C, int ldc, uint32_t box_c, uint32_t box_w, uint32_t box_h);
 int make_tmap_2d_plain(CUtensorMap* m, const void* base, int elem_bytes, uint64_t inner, uint64_t outer, uint64_t pitch_bytes,
                        uint32_t box_inner, uint32_t box_outer);
-int make_tmap_nhwc_plain(CUtensorMap* m, const void* base, int B, int H, int W, int C, uint32_t box_c, uint32_t box_w, uint32_t box_h);
 // bf16 NHWC view with explicit pixel / row / image strides (bytes): the four phase sub-lattices of a x2 upsampled map
 int make_tmap_nhwc_strided(CUtensorMap* m, const void* base, int B, int H, int W, int C, uint64_t pix_bytes, uint64_t row_bytes, uint64_t img_bytes,
                            uint32_t box_c, uint32_t box_w, uint32_t box_h);
@@ -277,6 +276,5 @@ int launch_conv_last_fold(const GemmParams& p, const bf16* A, const CUtensorMap&
 int launch_conv3_c64(int BN, const GemmParams& p, const bf16* A, const CUtensorMap& tb, int num_sms, cudaStream_t st);
 int launch_umma_gemm_tma(int BN, const GemmParams& p, const CUtensorMap* maps, int num_sms, cudaStream_t st);
 int launch_umma_gemm(int BN, const GemmParams& p, const CUtensorMap& ta, const CUtensorMap& tb, int num_sms, cudaStream_t st);
-int launch_simt_gemm(int BN, const GemmParams& p, cudaStream_t st);
 
 }  // namespace hitsir

@@ -1,10 +1,7 @@
 // Bandwidth-bound glue kernels of the HiT-SIR-pro forward (everything that is not a dense
-// contraction or the window self-correlation): entry im2col, LayerNorm, depthwise 5x5 + GELU,
-// casa (SpatialChannelAttention) statistics and gating, UnionAttention/Fusion statistics and
+// contraction or the window self-correlation): entry im2col, LayerNorm, casa
+// (SpatialChannelAttention) statistics and gating, UnionAttention/Fusion statistics and
 // gating, nearest upsampling.  Token-major (NHWC) throughout; 128-bit accesses where rows allow.
-#include <cstdlib>
-#include <cstring>
-
 #include "gemm.cuh"
 #include "kernels.cuh"
 #include "ycbcr.cuh"
@@ -93,105 +90,6 @@ __global__ void ln_rows_kernel(const float* __restrict__ x, const float* __restr
   }
 }
 
-#ifdef HITSIR_AB_PATHS   // stand-alone depthwise path: A/B test build only (the product runs ffn_tail.cu)
-// h2 = h1 + gelu(dw5x5(h1) + b)   (ConvFFN middle, hit_sir_pro.py:42 with :15-17).
-// Persistent CTAs (one per SM, 16 warps) walk (16 x 32 pixel tile, 64-channel slice) work items.  One TMA box load stages the
-// (16+4) x (32+4) x 64 bf16 input patch (the conv's zero padding = TMA out-of-bounds fill) into one of two buffers while the
-// other is being consumed.  A warp owns 4 x 4 output blocks across the 64 channels (lane = channel pair, so every shared-memory
-// access is one conflict-free 128-byte pixel row); the 25 taps of the lane's channel pair live in registers, each input word is
-// loaded once per block and feeds up to 20 packed FMAs.
-constexpr int kDwTH = 16, kDwTW = 32, kDwPH = kDwTH + 4, kDwPW = kDwTW + 4;
-constexpr int kDwTileBytes = kDwPH * kDwPW * 128;
-constexpr int kDwThreads = 512;
-
-__global__ void __launch_bounds__(kDwThreads, 1) dwconv5_kernel(const __grid_constant__ CUtensorMap tm_in, const float* __restrict__ wt,
-                                                                const float* __restrict__ bias, bf16* __restrict__ h2, int B, int H, int W,
-                                                                int tiles_x, int tiles_y, int total) {
-  extern __shared__ __align__(128) uint8_t dw_smem[];
-  const uint32_t tile_s = smem_u32(dw_smem);
-  const uint32_t bar0 = tile_s + 2 * kDwTileBytes;
-  constexpr int kSlices = kHidp / 64;
-  auto issue = [&](int item, int buf) {
-    const int cchunk = item % kSlices; const int t1 = item / kSlices;
-    const int tx = t1 % tiles_x; const int t2 = t1 / tiles_x;
-    const int ty = t2 % tiles_y; const int b = t2 / tiles_y;
-    mbar_expect_tx(bar0 + 8u * buf, kDwTileBytes);
-    tma_load_4d(tile_s + buf * kDwTileBytes, &tm_in, bar0 + 8u * buf, cchunk * 64, tx * kDwTW - 2, ty * kDwTH - 2, b);
-  };
-  if (threadIdx.x == 0) { mbar_init(bar0, 1); mbar_init(bar0 + 8, 1); fence_barrier_init(); }
-  __syncthreads();
-  if (threadIdx.x == 0 && (int)blockIdx.x < total) issue(blockIdx.x, 0);
-  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-  int it = 0;
-  for (int item = blockIdx.x; item < total; item += gridDim.x, ++it) {
-    const int buf = it & 1;
-    if (threadIdx.x == 0 && item + (int)gridDim.x < total) issue(item + gridDim.x, buf ^ 1);   // freed by the barrier ending iteration it-1
-    const int cchunk = item % kSlices; const int t1 = item / kSlices;
-    const int tx = t1 % tiles_x; const int t2 = t1 / tiles_x;
-    const int ty = t2 % tiles_y; const int b = t2 / tiles_y;
-    const int y0 = ty * kDwTH, x0 = tx * kDwTW;
-    const int c = cchunk * 64 + 2 * lane;
-    float2 w[25];
-#pragma unroll
-    for (int t = 0; t < 25; ++t) w[t] = *reinterpret_cast<const float2*>(wt + t * kHidp + c);
-    const float2 bs = *reinterpret_cast<const float2*>(bias + c);
-    const bool live = c < kHid;                     // kHid is even: a channel pair is entirely real or entirely padding
-    const bool full = (y0 + kDwTH <= H) && (x0 + kDwTW <= W);
-    mbar_wait(bar0 + 8u * buf, (uint32_t)((it >> 1) & 1));
-    const uint32_t* tile = reinterpret_cast<const uint32_t*>(dw_smem + buf * kDwTileBytes) + lane;      // + pixel * 32 words
-    bf16* out_tile = h2 + (((long long)b * H + y0) * W + x0) * kHidp + c;
-    const int rowstride = W * kHidp;
-#pragma unroll 1
-    for (int pass = 0; pass < 2; ++pass) {
-      const int blk = warp * 2 + pass;              // 4 x 8 blocks of 4 x 4 pixels
-      const int by = (blk >> 3) * 4, bx = (blk & 7) * 4;
-      float2 acc[4][4];
-#pragma unroll
-      for (int oy = 0; oy < 4; ++oy)
-#pragma unroll
-        for (int ox = 0; ox < 4; ++ox) acc[oy][ox] = bs;
-      uint32_t center[4][4];
-      const uint32_t* tp = tile + (by * kDwPW + bx) * 32;
-#pragma unroll
-      for (int iy = 0; iy < 8; ++iy) {
-        float2 in[8];
-#pragma unroll
-        for (int ix = 0; ix < 8; ++ix) {
-          const uint32_t u = tp[(iy * kDwPW + ix) * 32];
-          in[ix] = unpack_bf16x2(u);
-          if (iy >= 2 && iy < 6 && ix >= 2 && ix < 6) center[iy - 2][ix - 2] = u;
-        }
-#pragma unroll
-        for (int ky = 0; ky < 5; ++ky) {
-          const int oy = iy - ky;                   // compile-time after unrolling
-          if (oy >= 0 && oy < 4) {
-#pragma unroll
-            for (int ox = 0; ox < 4; ++ox)
-#pragma unroll
-              for (int kx = 0; kx < 5; ++kx) acc[oy][ox] = __ffma2_rn(in[ox + kx], w[ky * 5 + kx], acc[oy][ox]);
-          }
-        }
-      }
-      bf16* ob = out_tile + by * rowstride + bx * kHidp;
-#pragma unroll
-      for (int oy = 0; oy < 4; ++oy) {
-#pragma unroll
-        for (int ox = 0; ox < 4; ++ox) {
-          if (full || (y0 + by + oy < H && x0 + bx + ox < W)) {
-            const float2 cv = unpack_bf16x2(center[oy][ox]);
-            const float2 g = gelu2(acc[oy][ox]);
-            const uint32_t o = live ? pack_bf16x2(cv.x + g.x, cv.y + g.y) : 0u;
-            *reinterpret_cast<uint32_t*>(ob + oy * rowstride + ox * kHidp) = o;
-          }
-        }
-      }
-    }
-    __syncthreads();                                // every warp is done with `buf` before it is refilled (next iteration's issue)
-  }
-}
-
-#endif  // HITSIR_AB_PATHS
-
 // PIL-style uint8 HWC image -> [0,1] fp32 NCHW (torchvision to_tensor: true division by 255; reference utils/utils.py:143-145)
 __global__ void u8hwc_to_f32nchw_kernel(const uint8_t* __restrict__ in, float* __restrict__ out, int B, int H, int W, int C) {
   const long long total = (long long)B * C * H * W;
@@ -249,10 +147,6 @@ __global__ void psnr_y_final_kernel(const double* __restrict__ partial, int chun
   double t = 0.0;
   for (int c = 0; c < chunks; ++c) t += partial[(long long)blockIdx.x * chunks + c];
   mse[blockIdx.x] = t / (double)HW;
-}
-
-__global__ void fill_kernel(float* p, float v, long long n) {
-  for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (long long)gridDim.x * blockDim.x) p[i] = v;
 }
 
 __global__ void tap_kernel(const void* src, int is_bf16, int ld, float* dst, long long rows, int cols, int perm) {
@@ -403,90 +297,9 @@ __global__ void qkv_build_kernel(const float* __restrict__ x, PadGeom g, bf16* _
   }
 }
 
-#ifdef HITSIR_AB_PATHS   // SIMT gate: A/B test build only
-// casa gate: CTA = (image b, padded row yp, run of 64 padded pixels); thread = pair of head-padded positions (2t, 2t+1);
-// an even position is never a pad, the odd one is a pad when (2t+1) % 16 == 15 (position 15 carries the constant 1).
-// The two 3x3 filters of a channel pair live in registers, the 3 x 66 window of both statistic maps in shared
-// memory; per pixel a thread does 18 packed FMAs, one 8-byte token load and one 4-byte bf16x2 store, so a warp
-// reads/writes whole contiguous token rows.
-constexpr int kQkvRun = 64;
-__global__ void __launch_bounds__(96, 10) qkv_casa_kernel(const float* __restrict__ x, PadGeom g, const float* __restrict__ cavg,
-                                                      const float* __restrict__ cmax, const float* __restrict__ s1, const float* __restrict__ s2,
-                                                      CasaW w, bf16* __restrict__ t, int runs) {
-  __shared__ float sa[3][kQkvRun + 2], sm[3][kQkvRun + 2];
-  const int run = blockIdx.x % runs; const int t2 = blockIdx.x / runs;
-  const int yp = t2 % g.Hp; const int b = t2 / g.Hp;
-  const int xs = run * kQkvRun;
-  const float* ca = cavg + (long long)b * g.H * g.W;      // statistics of the unpadded pixels, gathered through the reflect map
-  const float* cm = cmax + (long long)b * g.H * g.W;
-  for (int i = threadIdx.x; i < 3 * (kQkvRun + 2); i += 96) {
-    const int rr = i / (kQkvRun + 2), cc = i - rr * (kQkvRun + 2);
-    const int yy = yp + rr - 1, xx = xs + cc - 1;
-    const bool ok = yy >= 0 && yy < g.Hp && xx >= 0 && xx < g.Wp;     // zero padding of the PADDED map
-    const int src = ok ? reflect_src(yy, g.H) * g.W + reflect_src(xx, g.W) : 0;
-    sa[rr][cc] = ok ? ca[src] : 0.f;
-    sm[rr][cc] = ok ? cm[src] : 0.f;
-  }
-  const int pos = 2 * threadIdx.x;
-  const int cA = scc_chan(pos), cb = scc_chan(pos + 1);
-  const int cbs = cb >= 0 ? cb : cA;                    // pad slot: compute a harmless duplicate, overwrite below
-  const float padv = (pos + 1 < 96) ? 1.0f : 0.f;     // q pads carry the constant 1 (k-gen bias rider), v pads 0
-  float2 w1[9], w2[9];
-#pragma unroll
-  for (int tap = 0; tap < 9; ++tap) {
-    w1[tap] = make_float2(w.w1[tap * kC + cA], w.w1[tap * kC + cbs]);
-    w2[tap] = make_float2(w.w2[tap * kC + cA], w.w2[tap * kC + cbs]);
-  }
-  const float2 b1 = make_float2(w.b1[cA], w.b1[cbs]), b2 = make_float2(w.b2[cA], w.b2[cbs]);
-  const float2 g1 = make_float2(s1[(long long)b * kC + cA], s1[(long long)b * kC + cbs]);
-  const float2 g2 = make_float2(s2[(long long)b * kC + cA], s2[(long long)b * kC + cbs]);
-  __syncthreads();
-  const int ysrc = reflect_src(yp, g.H);
-  const int n = min(kQkvRun, g.Wp - xs);
-  const float* xrow = x + ((long long)b * g.H + ysrc) * g.W * kC;
-  bf16* trow = t + (((long long)b * g.Hp + yp) * g.Wp + xs) * kCp + pos;
-  // sliding 3x3 window of both statistic maps in registers: columns i, i+1 carried, column i+2 loaded per pixel
-  float a0[3], a1c[3], m0[3], m1c[3];
-#pragma unroll
-  for (int ky = 0; ky < 3; ++ky) { a0[ky] = sa[ky][0]; a1c[ky] = sa[ky][1]; m0[ky] = sm[ky][0]; m1c[ky] = sm[ky][1]; }
-  constexpr int kBatch = 4;
-  for (int i0 = 0; i0 < n; i0 += kBatch) {
-    float2 xv[kBatch];
-#pragma unroll
-    for (int u = 0; u < kBatch; ++u) {
-      const int xp = min(xs + i0 + u, g.Wp - 1);
-      const float* xr = xrow + (long long)reflect_src(xp, g.W) * kC;
-      xv[u] = make_float2(xr[cA], xr[cbs]);
-    }
-#pragma unroll
-    for (int u = 0; u < kBatch; ++u) {
-      const int i = i0 + u;
-      float a2c[3], m2c[3];
-#pragma unroll
-      for (int ky = 0; ky < 3; ++ky) { a2c[ky] = sa[ky][min(i + 2, kQkvRun + 1)]; m2c[ky] = sm[ky][min(i + 2, kQkvRun + 1)]; }
-      float2 acc1 = b1, acc2 = b2;
-#pragma unroll
-      for (int ky = 0; ky < 3; ++ky) {
-        acc1 = __ffma2_rn(w1[ky * 3 + 0], make_float2(a0[ky], a0[ky]), acc1);
-        acc1 = __ffma2_rn(w1[ky * 3 + 1], make_float2(a1c[ky], a1c[ky]), acc1);
-        acc1 = __ffma2_rn(w1[ky * 3 + 2], make_float2(a2c[ky], a2c[ky]), acc1);
-        acc2 = __ffma2_rn(w2[ky * 3 + 0], make_float2(m0[ky], m0[ky]), acc2);
-        acc2 = __ffma2_rn(w2[ky * 3 + 1], make_float2(m1c[ky], m1c[ky]), acc2);
-        acc2 = __ffma2_rn(w2[ky * 3 + 2], make_float2(m2c[ky], m2c[ky]), acc2);
-        a0[ky] = a1c[ky]; a1c[ky] = a2c[ky]; m0[ky] = m1c[ky]; m1c[ky] = m2c[ky];
-      }
-      const float o0 = xv[u].x + 0.5f * (lrelu(acc1.x, 0.2f) * g1.x + lrelu(acc2.x, 0.2f) * g2.x);     // (:345-359)
-      const float o1 = xv[u].y + 0.5f * (lrelu(acc1.y, 0.2f) * g1.y + lrelu(acc2.y, 0.2f) * g2.y);
-      if (i < n) *reinterpret_cast<uint32_t*>(trow + (long long)i * kCp) = pack_bf16x2(o0, cb >= 0 ? o1 : padv);
-    }
-  }
-}
-
-#endif  // HITSIR_AB_PATHS
-
 // ---------------------------------------------------------------------------------------------
 // casa gate on the tensor core.  The two Conv2d(1, C, 3) of SpatialChannelAttention (:345-347) are a K = 9 contraction per pixel
-// and channel: 18 FP32 FMAs per output on the SIMT path above, which made the kernel FMA/issue-bound at 2.8 TB/s.  Here they are
+// and channel: 18 FP32 FMAs per output, which made a SIMT version of this kernel FMA/issue-bound at 2.8 TB/s.  Here they are
 // warp-level bf16 MMAs (m16n8k16, fp32 accumulate) with a three-term split so that nothing is lost to bf16:
 //     k  0.. 8: a_hi[tap] * W_hi[tap]      k  9..17: a_lo[tap] * W_hi[tap]      k 18..26: a_hi[tap] * W_lo[tap]
 //     k 27, 28: 1 * b_hi, 1 * b_lo         k 29..31: 0                          (x = x_hi + x_lo, both bf16: ~16 mantissa bits)
@@ -496,9 +309,7 @@ __global__ void __launch_bounds__(96, 10) qkv_casa_kernel(const float* __restric
 // (48 head-padded positions) whose B fragments stay in registers for the whole row, the A
 // rows [32 px][32 k] of both statistic maps are built once per run in shared memory, and the gated bf16 tokens leave through a
 // padded shared tile as one 384-byte bulk store per pixel (per-thread 16-byte stores: 18.8 -> 17.9 ms/step).  What is left per output: 2 LeakyReLU, 2 FMA, the token read and the bf16 pack.
-#ifndef QKV_MIN_CTAS
-#define QKV_MIN_CTAS 5                           // 96 registers, no spills: shared memory (43 KB per CTA) then allows 5 CTAs per SM instead of 3 at 140 registers
-#endif
+constexpr int kQkvMinCtas = 5;                   // 96 registers, no spills: shared memory (43 KB per CTA) then allows 5 CTAs per SM instead of 3 at 140 registers
 constexpr int kMmaRun = 32;
 constexpr int kMmaXS = 180;                      // staged token rows keep their global pitch (720 B): a run of pixels is ONE bulk copy
 constexpr int kMmaOS = 100;                      // output row: 96 words + 4 (rows of a quad-store land on distinct banks)
@@ -537,7 +348,7 @@ __global__ void casa_bfrag_kernel(CasaW w, uint32_t* __restrict__ img) {
   img[idx] = (uint32_t)out[0] | ((uint32_t)out[1] << 16);
 }
 
-__global__ void __launch_bounds__(128, QKV_MIN_CTAS) qkv_casa_mma_kernel(const float* __restrict__ x, PadGeom g, const float* __restrict__ cavg,
+__global__ void __launch_bounds__(128, kQkvMinCtas) qkv_casa_mma_kernel(const float* __restrict__ x, PadGeom g, const float* __restrict__ cavg,
                                                            const float* __restrict__ cmax, const float* __restrict__ s1, const float* __restrict__ s2,
                                                            const uint32_t* __restrict__ bfrag, bf16* __restrict__ t) {
   pdl_entry();
@@ -861,22 +672,6 @@ int launch_ln_rows(const float* x, const float* gamma, const float* beta, bf16* 
   HITSIR_CHECK(cudaGetLastError());
   return 0;
 }
-#ifdef HITSIR_AB_PATHS
-int launch_dwconv5_gelu_add(const bf16* h1, const float* w, const float* bias, bf16* h2, int B, int H, int W, int num_sms, cudaStream_t st) {
-  const int smem = 2 * kDwTileBytes + 32;
-  static unsigned long long configured = 0;
-  if (ensure_dynamic_smem(dwconv5_kernel, smem, &configured)) return 1;
-  CUtensorMap tm;
-  if (make_tmap_nhwc_plain(&tm, h1, B, H, W, kHidp, 64, kDwPW, kDwPH)) return 1;
-  const int tiles_x = (W + kDwTW - 1) / kDwTW, tiles_y = (H + kDwTH - 1) / kDwTH;
-  const long long total = (long long)tiles_x * tiles_y * B * (kHidp / 64);
-  if (total > 2147483647LL) { set_error("launch_dwconv5: too many tiles"); return 1; }
-  const int grid = total < num_sms ? (int)total : num_sms;
-  dwconv5_kernel<<<grid, kDwThreads, smem, st>>>(tm, w, bias, h2, B, H, W, tiles_x, tiles_y, (int)total);
-  HITSIR_CHECK(cudaGetLastError());
-  return 0;
-}
-#endif
 int launch_u8hwc_to_f32nchw(const uint8_t* in, float* out, int B, int H, int W, int C, cudaStream_t st) {
   u8hwc_to_f32nchw_kernel<<<grid_for((long long)B * C * H * W, 256), 256, 0, st>>>(in, out, B, H, W, C);
   HITSIR_CHECK(cudaGetLastError());
@@ -894,11 +689,6 @@ int launch_psnr_y(const float* sr, const float* hr, int B, int H, int W, int cli
   psnr_y_partial_kernel<<<dim3((unsigned)chunks, (unsigned)B), 256, 0, st>>>(sr, hr, HW, clip, partial);
   HITSIR_CHECK(cudaGetLastError());
   psnr_y_final_kernel<<<B, 32, 0, st>>>(partial, (int)chunks, HW, mse);
-  HITSIR_CHECK(cudaGetLastError());
-  return 0;
-}
-int launch_fill_f32(float* p, float v, long long n, cudaStream_t st) {
-  fill_kernel<<<grid_for(n, 256), 256, 0, st>>>(p, v, n);
   HITSIR_CHECK(cudaGetLastError());
   return 0;
 }
@@ -946,15 +736,6 @@ int launch_sca_mlp(const float* part_sum, const float* part_max, int nparts, Pad
 int launch_qkv_build(const float* x, PadGeom g, int casa, const float* cavg, const float* cmax, const float* s1, const float* s2, CasaW w, bf16* t,
                      cudaStream_t st) {
   if (casa) {
-#ifdef HITSIR_AB_PATHS
-    static const bool simt = getenv("HITSIR_CASA") != nullptr && strcmp(getenv("HITSIR_CASA"), "simt") == 0;   // A/B switch: the SIMT gate
-    if (simt || w.bfrag == nullptr) {
-      const int runs = (g.Wp + kQkvRun - 1) / kQkvRun;
-      qkv_casa_kernel<<<g.B * g.Hp * runs, 96, 0, st>>>(x, g, cavg, cmax, s1, s2, w, t, runs);
-      HITSIR_CHECK(cudaGetLastError());
-      return 0;
-    }
-#endif
     if (w.bfrag == nullptr) { set_error("launch_qkv_build: casa B fragments were not packed"); return 1; }
     static unsigned long long configured = 0;
     if (ensure_dynamic_smem(qkv_casa_mma_kernel, kMmaSmem, &configured)) return 1;

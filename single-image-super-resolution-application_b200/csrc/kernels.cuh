@@ -21,8 +21,6 @@ int launch_entry_im2col(const float* x, bf16* a0, int B, int H, int W, int in_ch
 // add (optional): fp32 [add_rows, 180] added after the normalisation, row index modulo add_rows (absolute position embedding)
 int launch_ln_rows(const float* x, const float* gamma, const float* beta, bf16* out_bf16, float* out_f32, long long N, cudaStream_t st,
                    const float* add = nullptr, long long add_rows = 0);
-// depthwise 5x5 (zero pad 2) + bias -> GELU -> + input  (ConvFFN middle, hit_sir_pro.py:42)
-int launch_dwconv5_gelu_add(const bf16* h1, const float* w_tap_major, const float* bias, bf16* h2, int B, int H, int W, int num_sms, cudaStream_t st);
 // ffn_tail.cu: dwconv5 + GELU + input fused with fc2 + LayerNorm + residual (x updated in place); tm_w2 = packed fc2 weights, box {64, 192}
 // Optional by-product of ffn_tail: the casa statistics of the block output for the NEXT block (padded to Hp x Wp there):
 // cavg/cmax [B*H*W], part_sum/part_max [B * tiles][180] with tiles = ceil(H/8) * ceil(W/16) 8x16-pixel tiles per image
@@ -40,11 +38,6 @@ struct FfnBand { int halo, yg0, Hf; };
 int launch_ffn_tail(const bf16* h1, const uint32_t* dw_tbl_mma, const uint8_t* w2_img, const float* b2, const float* gamma,
                     const float* beta, float* x, int B, int H, int W, const FfnStats* stats, bf16* shadow, int num_sms, cudaStream_t st,
                     const FfnBand* band = nullptr);
-// proj_fc1.cu: proj + norm1 + residual chained with fc1 + GELU (the bf16 copy of the stream stays in shared memory); tm_wp = packed proj
-// weights (box {64, 192}), w1 = packed fc1 weights bf16 [384][192], res / xout fp32 [N][180], h1 bf16 [N][384]
-int launch_proj_fc1(const bf16* outsc, const CUtensorMap& tm_wp, const float* bp, const float* gamma, const float* beta, const float* res,
-                    float* xout, const bf16* w1, const float* b1, bf16* h1, long long N, int num_sms, cudaStream_t st);
-int launch_fill_f32(float* p, float v, long long n, cudaStream_t st);
 // per-image mean squared difference of the YCbCr Y channels of two [0,1] fp32 NCHW RGB batches (utils/utils.py:170-186, experiment.py:436-463)
 long long psnr_y_chunks(int H, int W);
 int launch_psnr_y(const float* sr, const float* hr, int B, int H, int W, int clip, double* partial, double* mse, cudaStream_t st);
@@ -82,7 +75,7 @@ struct CasaW {
   const float* l1s_w; const float* l1s_b;   // [180][18], [180]
   const float* l2f_w; const float* l2f_b;
   const float* l2s_w; const float* l2s_b;
-  const uint32_t* bfrag;                 // linear1/linear2 as split-bf16 MMA B fragments (launch_pack_casa_bfrag); nullptr = SIMT gate
+  const uint32_t* bfrag;                 // linear1/linear2 as split-bf16 MMA B fragments (launch_pack_casa_bfrag); required when casa is on
 };
 int casa_bfrag_words();
 int launch_pack_casa_bfrag(CasaW w, uint32_t* img, cudaStream_t st);

@@ -260,20 +260,6 @@ int make_tmap_2d_plain(CUtensorMap* m, const void* base, int elem_bytes, uint64_
   return 0;
 }
 
-// bf16 NHWC map without shared-memory swizzle (dense 2*box_c-byte pixel rows), OOB = zero fill
-int make_tmap_nhwc_plain(CUtensorMap* m, const void* base, int B, int H, int W, int C, uint32_t box_c, uint32_t box_w, uint32_t box_h) {
-  PFN_encodeTiled enc = get_encode();
-  if (!enc) return 1;
-  cuuint64_t dims[4] = {(cuuint64_t)C, (cuuint64_t)W, (cuuint64_t)H, (cuuint64_t)B};
-  cuuint64_t strides[3] = {(cuuint64_t)C * 2, (cuuint64_t)W * C * 2, (cuuint64_t)H * W * C * 2};
-  cuuint32_t box[4] = {box_c, box_w, box_h, 1};
-  cuuint32_t es[4] = {1, 1, 1, 1};
-  CUresult r = enc(m, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, const_cast<void*>(base), dims, strides, box, es, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                   CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  if (r != CUDA_SUCCESS) { set_error("cuTensorMapEncodeTiled(nhwc plain B=%d H=%d W=%d C=%d) failed with CUresult %d", B, H, W, C, (int)r); return 1; }
-  return 0;
-}
-
 template <int BN>
 static int launch_bn(const GemmParams& p, const CUtensorMap& ta, const CUtensorMap& tb, int num_sms, cudaStream_t st) {
   using Cfg = UmmaCfg<BN>;

@@ -44,7 +44,6 @@ __device__ __forceinline__ void tma_store_4d(const void* tmap, uint32_t src, int
                "r"(c2), "r"(c3) : "memory");
 }
 __device__ __forceinline__ void tma_commit() { asm volatile("cp.async.bulk.commit_group;" ::: "memory"); }
-__device__ __forceinline__ void tma_wait_read0() { asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory"); }
 __device__ __forceinline__ void tma_wait_read1() { asm volatile("cp.async.bulk.wait_group.read 1;" ::: "memory"); }   // all but the newest group
 __device__ __forceinline__ void tma_wait_all0() { asm volatile("cp.async.bulk.wait_group 0;" ::: "memory"); }
 template <int N>

@@ -266,8 +266,8 @@ def test_resi_3conv():
 
 
 def test_umma_direct_backend_is_rejected_by_the_product_library(trunk):
-    """The direct-store epilogue needs the unfused FFN tail, which only the -DHITSIR_AB_PATHS test build has: the product library
-    refuses the backend instead of failing every forward afterwards."""
+    """The library has one GEMM backend, "umma": any other name is refused with an error that names it, and the handle keeps
+    working."""
     model, _, x = trunk
     with pytest.raises(Exception, match="umma_direct"):
         model.set_gemm_backend(DEV, "umma_direct")

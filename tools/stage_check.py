@@ -1,6 +1,6 @@
 """Per-stage parity table: CUDA path (tap by tap) vs the CPU oracle.  GPU box only.
 
-    python tools/stage_check.py [--backend umma|simt] [--case pro|ablation|ps2|direct3] [--hw 64 64] [--batch 1]
+    python tools/stage_check.py [--case pro|ablation|ps2|direct3] [--hw 64 64] [--batch 1]
                                 [--mode stress|init] [--taps all|coarse]
 
 Prints one line per tap: rel-L2 and max-abs error against the oracle tensor of the same name.
@@ -30,7 +30,6 @@ CASES = {
 
 def main():
     ap = argparse.ArgumentParser()
-    ap.add_argument("--backend", default="umma")
     ap.add_argument("--case", default="pro")
     ap.add_argument("--hw", type=int, nargs=2, default=[64, 64])
     ap.add_argument("--batch", type=int, default=1)
@@ -45,10 +44,9 @@ def main():
     t0 = time.time()
     with torch.no_grad():
         y_ref = oracle.forward(x, taps)
-    print(f"oracle forward {time.time() - t0:.1f}s; case={args.case} hw={args.hw} batch={args.batch} mode={args.mode} backend={args.backend}", flush=True)
+    print(f"oracle forward {time.time() - t0:.1f}s; case={args.case} hw={args.hw} batch={args.batch} mode={args.mode}", flush=True)
     dev = torch.device("cuda:0")
     model = model.to(dev)
-    model.set_gemm_backend(dev, args.backend)
     xd = x.to(dev)
     names = list(taps.keys())
     if args.taps == "coarse":
