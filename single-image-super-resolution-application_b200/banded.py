@@ -28,6 +28,7 @@ from typing import List, Optional, Tuple
 import torch
 
 from . import _capi
+from .hit_sir_pro import _ws_alloc_bytes, _ws_offset
 
 BAND_UNIT = 192        # lcm of the window sizes 4, 8, 16, 32, 48, 64 (hier_win_ratios x base window 8)
 MIN_LAST_BAND = 64     # a band must be longer than its own reflect padding for every window (hit_sir_pro.py:672)
@@ -58,20 +59,16 @@ def _band_struct(frame_h, row0, layout_h, has_top, has_bottom, halo_cb, allreduc
 
 
 def _forward_band(model, x_frame, y_band, rows, W, band, ws, stream):
-    lib = _capi.load()
-    device = x_frame.device
-    with torch.cuda.device(device):
-        h = model._handle(device)
-        base = (ws.data_ptr() + 255) // 256 * 256
+    with model._native_call(x_frame.device, ws=ws, stream=stream) as (lib, h, ws_ptr, ws_bytes, st):
         _capi.check(lib.hitsir_forward_band(h, ctypes.c_void_p(x_frame.data_ptr()), ctypes.c_void_p(y_band.data_ptr()), rows, W, ctypes.byref(band),
-                                            ctypes.c_void_p(base), ws.numel() - (base - ws.data_ptr()), ctypes.c_void_p(stream)))
+                                            ws_ptr, ws_bytes, st))
 
 
 def _workspace_bytes(model, device, layout_h, W) -> int:
     n = ctypes.c_size_t()
     with torch.cuda.device(device):
         _capi.check(_capi.load().hitsir_workspace_bytes_band(model._handle(device), layout_h, W, ctypes.byref(n)))
-    return n.value + 512
+    return _ws_alloc_bytes(n.value)
 
 
 class LocalBandedSR:
@@ -103,7 +100,7 @@ class LocalBandedSR:
             model._sync_weights(h, device, cur.cuda_stream)
         nbytes = _workspace_bytes(model, device, layout_h, W)
         wss = [torch.empty(nbytes, dtype=torch.uint8, device=device) for _ in range(R)]
-        bases = [(w.data_ptr() + 255) // 256 * 256 - w.data_ptr() for w in wss]
+        bases = [_ws_offset(w) for w in wss]
         ys = [torch.empty((1, C, s * r, s * W), dtype=torch.float32, device=device) for _, r in plan]
         streams = [torch.cuda.Stream(device) for _ in range(R)]
         for st in streams:
@@ -271,7 +268,7 @@ class BandedSR:
         _, C, Hf, W = x.shape
         R = len(plan)
         ws = self._ws
-        base = (ws.data_ptr() + 255) // 256 * 256 - ws.data_ptr()           # identical on every rank (symmetric allocations are equally aligned)
+        base = _ws_offset(ws)                                                # identical on every rank (symmetric allocations are equally aligned)
         me = self.rank
         hdl, peers = self._hdl, self._peers
         cur = torch.cuda.current_stream(device)

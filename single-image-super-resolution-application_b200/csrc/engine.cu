@@ -646,6 +646,31 @@ struct Fwd {
   bool top = false, bot = false;     // a neighbour band exists above / below
 };
 
+#define RUN(expr) do { int _r = (expr); if (_r) return _r; } while (0)
+
+// The refusals every forward entry starts with.  `no_taps`: nullptr where taps and injections are supported, else how the refusal ends.
+int check_entry(const HitsirHandle* h, const char* entry, const char* no_taps) {
+  if (!h->finalized) { set_error("%s: weights not finalized (call hitsir_set_param for every key, then hitsir_finalize_weights)", entry); return HITSIR_ERR_WEIGHTS; }
+  if (no_taps && (h->tap.dst != nullptr || h->inject.src != nullptr)) { set_error("%s: taps / injections are not supported %s", entry, no_taps); return HITSIR_ERR_UNSUPPORTED; }
+  return 0;
+}
+
+int check_workspace(const void* workspace, size_t need, size_t have) {
+  if (((uintptr_t)workspace & 255) != 0) { set_error("workspace must be 256-byte aligned"); return HITSIR_ERR_WORKSPACE; }
+  if (need > have) { set_error("workspace too small: need %zu bytes, got %zu", need, have); return HITSIR_ERR_WORKSPACE; }
+  return 0;
+}
+
+// One forward of B images of H x W over `workspace`; band mode (`band` given, B = 1): the band's H rows of the frame, laid out for
+// band->layout_h rows so that every band of the frame finds its buffers at the same offsets
+int init_fwd(Fwd& f, HitsirHandle* h, int B, int H, int W, const HitsirBand* band, void* workspace, size_t workspace_bytes, cudaStream_t st) {
+  const int layout_h = band != nullptr ? band->layout_h : H;
+  f.h = h; f.st = st; f.B = B; f.H = H; f.W = W; f.N = (long long)B * H * W; f.Nl = (long long)B * layout_h * W; f.ws_base = workspace;
+  if (band != nullptr) { f.band = band; f.row0 = band->row0; f.Hf = band->frame_h; f.top = band->has_top != 0; f.bot = band->has_bottom != 0; }
+  RUN(layout_workspace(h, B, layout_h, W, workspace, &f.ws, band != nullptr ? 1 : 0));
+  return check_workspace(workspace, f.ws.bytes, workspace_bytes);
+}
+
 // Make the `halo` rows above and below the `rows` core rows of a row-major buffer valid before a vertical stencil reads them: rows
 // outside the frame are zero (the stencil's zero padding), rows of a neighbour band are fetched through the caller's exchange callback
 // (which runs on the host while the forward is being enqueued and must order its copies on `stream`).  No-op outside band mode.
@@ -689,7 +714,6 @@ int do_inject(Fwd& f, const char* name, float* dst_f32, bf16* dst_bf16, long lon
   return 0;
 }
 
-#define RUN(expr) do { int _r = (expr); if (_r) return _r; } while (0)
 struct ProfScope {
   HitsirHandle* h; cudaStream_t st; int idx = -1;
   ProfScope(HitsirHandle* h_, cudaStream_t st_, const char* cat) : h(h_), st(st_) {
@@ -722,10 +746,8 @@ bool tma_epilogue(const GemmW& w, const GemmParams& p) {
 }
 
 int run_gemm(Fwd& f, const char* cat, const GemmW& w, GemmParams& p, const CUtensorMap* maps, bool tma) {
-  ProfScope ps(f.h, f.st, cat);
-  f.h->launches++;
-  if (tma) return launch_umma_gemm_tma(w.BN, p, maps, f.h->num_sms, f.st);
-  return launch_umma_gemm(w.BN, p, maps[0], w.tm, f.h->num_sms, f.st);
+  LAUNCH(cat, 1, tma ? launch_umma_gemm_tma(w.BN, p, maps, f.h->num_sms, f.st) : launch_umma_gemm(w.BN, p, maps[0], w.tm, f.h->num_sms, f.st));
+  return 0;
 }
 
 // token-major linear: A [M, lda] bf16 (lda == w.K)
@@ -746,9 +768,9 @@ int linear(Fwd& f, const char* cat, const GemmW& w, const bf16* A, long long M, 
   return run_gemm(f, cat, w, p, maps, tma);
 }
 
-// 3x3 conv over NHWC bf16 [B,H,W,Cpad].  Band mode: the rows above / below A are made valid first (fill_halo: zeros at the frame
-// border, the neighbour band's rows otherwise) and the A tensor map starts one row above image row 0.
-int conv3(Fwd& f, const char* cat, const GemmW& w, const bf16* A, int B, int H, int W, int Cpad, GemmParams& p) {
+// Geometry of a 3x3 conv over NHWC bf16 A [B,H,W,Cpad] in 8 x 16-pixel tiles.  Band mode: the rows above / below A are made valid
+// first (fill_halo: zeros at the frame border, the neighbour band's rows otherwise) and the A tensor map starts one row above image row 0.
+int conv_geometry(Fwd& f, const bf16* A, int B, int H, int W, int Cpad, GemmParams& p) {
   p.conv = 1; p.B = B; p.H = H; p.W = W;
   if (f.band != nullptr) {
     RUN(fill_halo(f, const_cast<bf16*>(A), (size_t)W * Cpad * sizeof(bf16), H, 1));
@@ -758,15 +780,18 @@ int conv3(Fwd& f, const char* cat, const GemmW& w, const bf16* A, int B, int H, 
   p.m_tiles = B * p.tiles_x * p.tiles_y;
   p.cblocks = Cpad / 64;
   p.A = A; p.lda = Cpad;
+  return 0;
+}
+
+int conv3(Fwd& f, const char* cat, const GemmW& w, const bf16* A, int B, int H, int W, int Cpad, GemmParams& p) {
+  RUN(conv_geometry(f, A, B, H, W, Cpad, p));
   if (w.K != 9 * Cpad) { set_error("conv3: packed K %d != 9*%d", w.K, Cpad); return 1; }
   // 64-channel inputs (HR stage): resident filter bank + kx-shared halo boxes (conv3_c64.cu)
   if (Cpad == 64 && p.res == nullptr && p.out2_f32 == nullptr &&
       ((w.BN == 64 && p.epi == EPI_STORE && p.out_bf16 != nullptr && p.out_f32 == nullptr && p.ldb == 64) ||
        (w.BN == 16 && w.wf != nullptr && p.res_img == nullptr && p.epi == EPI_SHUFFLE_NCHW && p.ps == 1 && p.n_real <= 4))) {
-    ProfScope ps(f.h, f.st, cat);
-    f.h->launches++;
-    if (w.BN == 16) return launch_conv_last_fold(p, A, w.tmf, f.h->num_sms, f.st);
-    return launch_conv3_c64(w.BN, p, A, w.tm, f.h->num_sms, f.st);
+    LAUNCH(cat, 1, w.BN == 16 ? launch_conv_last_fold(p, A, w.tmf, f.h->num_sms, f.st) : launch_conv3_c64(w.BN, p, A, w.tm, f.h->num_sms, f.st));
+    return 0;
   }
   CUtensorMap maps[5];
   const bool tma = tma_epilogue(w, p);
@@ -783,19 +808,10 @@ int conv3(Fwd& f, const char* cat, const GemmW& w, const bf16* A, int B, int H, 
 // x2 nearest upsampling + 3x3 conv 64 -> 64 (+ LeakyReLU) on the LR map A [B,H,W,64] -> out [B,2H,2W,64] (:1331-1332).  Band mode: the
 // LR rows above / below the band are exchanged (one LR row is what the replicated map's halo row was made of)
 int conv3_up(Fwd& f, const char* cat, const GemmW& w, const bf16* A, int B, int H, int W, GemmParams& p) {
-  p.conv = 1; p.B = B; p.H = H; p.W = W;
-  if (f.band != nullptr) {
-    RUN(fill_halo(f, const_cast<bf16*>(A), (size_t)W * kNumFeat * sizeof(bf16), H, 1));
-    p.a_y_off = 1;
-  }
-  p.tiles_x = cdiv(W, 16); p.tiles_y = cdiv(H, 8);
-  p.m_tiles = B * p.tiles_x * p.tiles_y;
-  p.cblocks = 1;
-  p.A = A; p.lda = kNumFeat;
+  RUN(conv_geometry(f, A, B, H, W, kNumFeat, p));
   if (w.K != 16 * kNumFeat) { set_error("conv3_up: packed K %d is not the sub-pixel layout", w.K); return 1; }
-  ProfScope ps(f.h, f.st, cat);
-  f.h->launches++;
-  return launch_conv3_c64_up(p, A, w.tm, f.h->num_sms, f.st);
+  LAUNCH(cat, 1, launch_conv3_c64_up(p, A, w.tm, f.h->num_sms, f.st));
+  return 0;
 }
 
 #define TAP(name, src, is_bf16, ld, rows, cols) do { RUN(do_tap(f, name, src, is_bf16, ld, rows, cols)); if (f.stopped) return 0; } while (0)
@@ -1110,12 +1126,10 @@ int layout_x8(const HitsirHandle* h, int B, int H, int W, int group, X8Layout* L
 // exactly one of x / x_u8 and of y / y_u8 is given; y doubles as the accumulator
 int forward_x8(HitsirHandle* h, const float* x, const uint8_t* x_u8, float* y, uint8_t* y_u8, int B, int H, int W, int group, void* workspace,
                size_t workspace_bytes, cudaStream_t st) {
-  if (!h->finalized) { set_error("hitsir_forward_x8: weights not finalized (call hitsir_set_param for every key, then hitsir_finalize_weights)"); return HITSIR_ERR_WEIGHTS; }
-  if (h->tap.dst != nullptr || h->inject.src != nullptr) { set_error("hitsir_forward_x8: taps / injections are not supported by the self-ensemble"); return HITSIR_ERR_UNSUPPORTED; }
+  RUN(check_entry(h, "hitsir_forward_x8", "by the self-ensemble"));
   X8Layout L;
   RUN(layout_x8(h, B, H, W, group, &L));
-  if (((uintptr_t)workspace & 255) != 0) { set_error("workspace must be 256-byte aligned"); return HITSIR_ERR_WORKSPACE; }
-  if (L.bytes > workspace_bytes) { set_error("workspace too small: need %zu bytes, got %zu", L.bytes, workspace_bytes); return HITSIR_ERR_WORKSPACE; }
+  RUN(check_workspace(workspace, L.bytes, workspace_bytes));
   uint8_t* base = reinterpret_cast<uint8_t*>(workspace);
   float* xt = reinterpret_cast<float*>(base + L.xt);
   float* z = reinterpret_cast<float*>(base + L.z);
@@ -1125,8 +1139,7 @@ int forward_x8(HitsirHandle* h, const float* x, const uint8_t* x_u8, float* y, u
   for (int k0 = 0; k0 < 8; k0 += group) {
     const bool t = (k0 & 4) != 0;
     Fwd f;
-    f.h = h; f.st = st; f.B = group * B; f.H = t ? W : H; f.W = t ? H : W; f.N = (long long)f.B * H * W; f.Nl = f.N;
-    RUN(layout_workspace(h, f.B, f.H, f.W, workspace, &f.ws));
+    RUN(init_fwd(f, h, group * B, t ? W : H, t ? H : W, nullptr, workspace, L.xt, st));
     LAUNCH("x8_in", 1, launch_x8_entry(x, x_u8, xt, B, C, H, W, k0, group, st));
     RUN(forward_impl(f, xt, z));
     const bool last = k0 + group == 8;
@@ -1208,35 +1221,26 @@ HITSIR_API int hitsir_finalize_weights(HitsirHandle* h, void* stream) {
 HITSIR_API int hitsir_workspace_bytes(const HitsirHandle* h, int B, int H, int W, size_t* bytes) {
   if (!h || !bytes || B < 1 || H < 1 || W < 1) { set_error("hitsir_workspace_bytes: bad argument"); return HITSIR_ERR_INVALID; }
   Workspace ws;
-  int rc = layout_workspace(h, B, H, W, nullptr, &ws);
-  if (rc) return rc;
+  RUN(layout_workspace(h, B, H, W, nullptr, &ws));
   *bytes = ws.bytes;
   return 0;
 }
 
 HITSIR_API int hitsir_forward(HitsirHandle* h, const float* x, float* y, int B, int H, int W, void* workspace, size_t workspace_bytes, void* stream) {
   if (!h || !x || !y || !workspace) { set_error("hitsir_forward: null argument"); return HITSIR_ERR_INVALID; }
-  if (!h->finalized) { set_error("hitsir_forward: weights not finalized (call hitsir_set_param for every key, then hitsir_finalize_weights)"); return HITSIR_ERR_WEIGHTS; }
-  if ((long long)B * H * W * 16 >= 2147483647LL / 4) {
-    // row indices are kept in 32 bit inside the GEMM tile maps; 16x upsampled pixel counts must fit too
-    if ((long long)B * H * W * 16 >= 2147483647LL) { set_error("input too large: B*H*W*16 must be < 2^31"); return HITSIR_ERR_UNSUPPORTED; }
-  }
+  RUN(check_entry(h, "hitsir_forward", nullptr));
+  // row indices are kept in 32 bit inside the GEMM tile maps; 16x upsampled pixel counts must fit too
+  if ((long long)B * H * W * 16 >= 2147483647LL) { set_error("input too large: B*H*W*16 must be < 2^31"); return HITSIR_ERR_UNSUPPORTED; }
   Fwd f;
-  f.h = h; f.st = (cudaStream_t)stream; f.B = B; f.H = H; f.W = W; f.N = (long long)B * H * W; f.Nl = f.N;
-  int rc = layout_workspace(h, B, H, W, workspace, &f.ws);
-  if (rc) return rc;
-  if (((uintptr_t)workspace & 255) != 0) { set_error("workspace must be 256-byte aligned"); return HITSIR_ERR_WORKSPACE; }
-  if (f.ws.bytes > workspace_bytes) { set_error("workspace too small: need %zu bytes, got %zu", f.ws.bytes, workspace_bytes); return HITSIR_ERR_WORKSPACE; }
+  RUN(init_fwd(f, h, B, H, W, nullptr, workspace, workspace_bytes, (cudaStream_t)stream));
   h->launches = 0;
-  rc = forward_impl(f, x, y);
-  return rc;
+  return forward_impl(f, x, y);
 }
 
 HITSIR_API int hitsir_workspace_bytes_band(const HitsirHandle* h, int layout_h, int W, size_t* bytes) {
   if (!h || !bytes || layout_h < 1 || W < 1) { set_error("hitsir_workspace_bytes_band: bad argument"); return HITSIR_ERR_INVALID; }
   Workspace ws;
-  int rc = layout_workspace(h, 1, layout_h, W, nullptr, &ws, 1);
-  if (rc) return rc;
+  RUN(layout_workspace(h, 1, layout_h, W, nullptr, &ws, 1));
   *bytes = ws.bytes;
   return 0;
 }
@@ -1244,7 +1248,7 @@ HITSIR_API int hitsir_workspace_bytes_band(const HitsirHandle* h, int layout_h, 
 HITSIR_API int hitsir_forward_band(HitsirHandle* h, const float* x_frame, float* y_band, int H, int W, const HitsirBand* band, void* workspace,
                                    size_t workspace_bytes, void* stream) {
   if (!h || !x_frame || !y_band || !workspace || !band) { set_error("hitsir_forward_band: null argument"); return HITSIR_ERR_INVALID; }
-  if (!h->finalized) { set_error("hitsir_forward_band: weights not finalized"); return HITSIR_ERR_WEIGHTS; }
+  RUN(check_entry(h, "hitsir_forward_band", "in band mode"));
   if ((band->has_top || band->has_bottom) && (!band->halo || !band->allreduce)) { set_error("hitsir_forward_band: exchange callbacks missing"); return HITSIR_ERR_INVALID; }
   if (H < 1 || H > band->layout_h || band->row0 < 0 || band->row0 + H > band->frame_h) { set_error("hitsir_forward_band: band rows [%d, %d) do not fit frame_h %d / layout_h %d", band->row0, band->row0 + H, band->frame_h, band->layout_h); return HITSIR_ERR_INVALID; }
   if (band->row0 % 192 != 0 || (band->has_bottom && H % 192 != 0)) {
@@ -1253,14 +1257,8 @@ HITSIR_API int hitsir_forward_band(HitsirHandle* h, const float* x_frame, float*
   }
   if (h->cfg.ape_tokens > 0) { set_error("hitsir_forward_band: ape=True is not supported in band mode"); return HITSIR_ERR_UNSUPPORTED; }
   if (h->cfg.upsampler == HITSIR_UP_NONE) { set_error("hitsir_forward_band: upsampler=None (same-size output added to the input) is not supported in band mode"); return HITSIR_ERR_UNSUPPORTED; }
-  if (h->tap.dst != nullptr || h->inject.src != nullptr) { set_error("hitsir_forward_band: taps / injections are not supported in band mode"); return HITSIR_ERR_UNSUPPORTED; }
   Fwd f;
-  f.h = h; f.st = (cudaStream_t)stream; f.B = 1; f.H = H; f.W = W; f.N = (long long)H * W; f.Nl = (long long)band->layout_h * W;
-  f.band = band; f.ws_base = workspace; f.row0 = band->row0; f.Hf = band->frame_h; f.top = band->has_top != 0; f.bot = band->has_bottom != 0;
-  int rc = layout_workspace(h, 1, band->layout_h, W, workspace, &f.ws, 1);
-  if (rc) return rc;
-  if (((uintptr_t)workspace & 255) != 0) { set_error("workspace must be 256-byte aligned"); return HITSIR_ERR_WORKSPACE; }
-  if (f.ws.bytes > workspace_bytes) { set_error("workspace too small: need %zu bytes, got %zu", f.ws.bytes, workspace_bytes); return HITSIR_ERR_WORKSPACE; }
+  RUN(init_fwd(f, h, 1, H, W, band, workspace, workspace_bytes, (cudaStream_t)stream));
   // the reference pads the FRAME: a band of the last rows may be shorter than its own reflect padding only if the frame is
   for (int j = 0; j < h->cfg.depths[0]; ++j) {
     const int w = win_of(h->cfg, j), pad = round_up(H, w) - H;

@@ -264,8 +264,6 @@ int make_tmap_2d(CUtensorMap* m, const void* base, uint64_t inner, uint64_t oute
 int make_tmap_nhwc(CUtensorMap* m, const void* base, int B, int H, int W, int Cpad, uint32_t box_c, uint32_t box_w, uint32_t box_h);
 int make_tmap_2d_t(CUtensorMap* m, const void* base, int elem_bytes, uint64_t inner, uint64_t outer, uint64_t pitch_bytes, uint32_t box_inner, uint32_t box_outer);
 int make_tmap_nhwc_t(CUtensorMap* m, const void* base, int elem_bytes, int B, int H, int W, int C, int ldc, uint32_t box_c, uint32_t box_w, uint32_t box_h);
-int make_tmap_2d_plain(CUtensorMap* m, const void* base, int elem_bytes, uint64_t inner, uint64_t outer, uint64_t pitch_bytes,
-                       uint32_t box_inner, uint32_t box_outer);
 // bf16 NHWC view with explicit pixel / row / image strides (bytes): the four phase sub-lattices of a x2 upsampled map
 int make_tmap_nhwc_strided(CUtensorMap* m, const void* base, int B, int H, int W, int C, uint64_t pix_bytes, uint64_t row_bytes, uint64_t img_bytes,
                            uint32_t box_c, uint32_t box_w, uint32_t box_h);

@@ -160,19 +160,37 @@ typedef CUresult (*PFN_encodeTiled)(CUtensorMap*, CUtensorMapDataType, cuuint32_
                                     const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
                                     CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
 
-static PFN_encodeTiled get_encode() {
-  static PFN_encodeTiled fn = nullptr;
-  if (fn == nullptr) {
+// Every tensor map of the library: a `rank`-D (2 or 4) tensor of fp32 (elem_bytes 4) or bf16 elements, dims and box innermost first,
+// `strides` the rank - 1 outer strides in bytes; boxes land in 128B-swizzled shared memory, out-of-bounds elements read as zero.
+static int encode_tmap(CUtensorMap* m, const void* base, int elem_bytes, int rank, const cuuint64_t* dims, const cuuint64_t* strides,
+                       const cuuint32_t* box) {
+  static PFN_encodeTiled enc = nullptr;
+  if (enc == nullptr) {
     void* ptr = nullptr;
     cudaDriverEntryPointQueryResult qres;
     cudaError_t e = cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &ptr, cudaEnableDefault, &qres);
     if (e != cudaSuccess || qres != cudaDriverEntryPointSuccess || ptr == nullptr) {
       set_error("cudaGetDriverEntryPoint(cuTensorMapEncodeTiled) failed: %s", cudaGetErrorString(e));
-      return nullptr;
+      return 1;
     }
-    fn = reinterpret_cast<PFN_encodeTiled>(ptr);
+    enc = reinterpret_cast<PFN_encodeTiled>(ptr);
   }
-  return fn;
+  const cuuint32_t es[4] = {1, 1, 1, 1};
+  const CUresult r = enc(m, elem_bytes == 4 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT32 : CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, (cuuint32_t)rank,
+                         const_cast<void*>(base), dims, strides, box, es, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B,
+                         CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+  if (r != CUDA_SUCCESS) {
+    char shape[320];
+    int n = snprintf(shape, sizeof(shape), "%d-byte elements, dims", elem_bytes);
+    for (int i = 0; i < rank; ++i) n += snprintf(shape + n, sizeof(shape) - n, " %llu", (unsigned long long)dims[i]);
+    n += snprintf(shape + n, sizeof(shape) - n, ", byte strides");
+    for (int i = 0; i < rank - 1; ++i) n += snprintf(shape + n, sizeof(shape) - n, " %llu", (unsigned long long)strides[i]);
+    n += snprintf(shape + n, sizeof(shape) - n, ", box");
+    for (int i = 0; i < rank; ++i) n += snprintf(shape + n, sizeof(shape) - n, " %u", box[i]);
+    set_error("cuTensorMapEncodeTiled(%s) failed with CUresult %d", shape, (int)r);
+    return 1;
+  }
+  return 0;
 }
 
 int make_tmap_2d(CUtensorMap* m, const void* base, uint64_t inner, uint64_t outer, uint64_t pitch_bytes,
@@ -182,22 +200,9 @@ int make_tmap_2d(CUtensorMap* m, const void* base, uint64_t inner, uint64_t oute
 
 int make_tmap_2d_t(CUtensorMap* m, const void* base, int elem_bytes, uint64_t inner, uint64_t outer, uint64_t pitch_bytes,
                    uint32_t box_inner, uint32_t box_outer) {
-  PFN_encodeTiled enc = get_encode();
-  if (!enc) return 1;
-  const CUtensorMapDataType dt = elem_bytes == 4 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT32 : CU_TENSOR_MAP_DATA_TYPE_BFLOAT16;
-  cuuint64_t dims[2] = {inner, outer};
-  cuuint64_t strides[1] = {pitch_bytes};
-  cuuint32_t box[2] = {box_inner, box_outer};
-  cuuint32_t es[2] = {1, 1};
-  CUresult r = enc(m, dt, 2, const_cast<void*>(base), dims, strides, box, es,
-                   CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                   CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  if (r != CUDA_SUCCESS) {
-    set_error("cuTensorMapEncodeTiled(2d inner=%llu outer=%llu pitch=%llu box=%ux%u) failed with CUresult %d",
-              (unsigned long long)inner, (unsigned long long)outer, (unsigned long long)pitch_bytes, box_inner, box_outer, (int)r);
-    return 1;
-  }
-  return 0;
+  const cuuint64_t dims[2] = {inner, outer}, strides[1] = {pitch_bytes};
+  const cuuint32_t box[2] = {box_inner, box_outer};
+  return encode_tmap(m, base, elem_bytes, 2, dims, strides, box);
 }
 
 int make_tmap_nhwc(CUtensorMap* m, const void* base, int B, int H, int W, int Cpad, uint32_t box_c, uint32_t box_w, uint32_t box_h) {
@@ -207,57 +212,17 @@ int make_tmap_nhwc(CUtensorMap* m, const void* base, int B, int H, int W, int Cp
 // NHWC tensor with `C` visible channels out of a pixel pitch of `ldc` elements
 int make_tmap_nhwc_t(CUtensorMap* m, const void* base, int elem_bytes, int B, int H, int W, int C, int ldc, uint32_t box_c, uint32_t box_w,
                      uint32_t box_h) {
-  PFN_encodeTiled enc = get_encode();
-  if (!enc) return 1;
-  const CUtensorMapDataType dt = elem_bytes == 4 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT32 : CU_TENSOR_MAP_DATA_TYPE_BFLOAT16;
-  const int Cpad = C;
-  const cuuint64_t eb = (cuuint64_t)elem_bytes;
-  cuuint64_t dims[4] = {(cuuint64_t)C, (cuuint64_t)W, (cuuint64_t)H, (cuuint64_t)B};
-  cuuint64_t strides[3] = {(cuuint64_t)ldc * eb, (cuuint64_t)W * ldc * eb, (cuuint64_t)H * W * ldc * eb};
-  cuuint32_t box[4] = {box_c, box_w, box_h, 1};
-  cuuint32_t es[4] = {1, 1, 1, 1};
-  CUresult r = enc(m, dt, 4, const_cast<void*>(base), dims, strides, box, es,
-                   CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                   CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  if (r != CUDA_SUCCESS) {
-    set_error("cuTensorMapEncodeTiled(nhwc B=%d H=%d W=%d C=%d) failed with CUresult %d", B, H, W, Cpad, (int)r);
-    return 1;
-  }
-  return 0;
+  const cuuint64_t pix = (cuuint64_t)ldc * elem_bytes;
+  const cuuint64_t dims[4] = {(cuuint64_t)C, (cuuint64_t)W, (cuuint64_t)H, (cuuint64_t)B}, strides[3] = {pix, W * pix, (cuuint64_t)H * W * pix};
+  const cuuint32_t box[4] = {box_c, box_w, box_h, 1};
+  return encode_tmap(m, base, elem_bytes, 4, dims, strides, box);
 }
 
 int make_tmap_nhwc_strided(CUtensorMap* m, const void* base, int B, int H, int W, int C, uint64_t pix_bytes, uint64_t row_bytes, uint64_t img_bytes,
                            uint32_t box_c, uint32_t box_w, uint32_t box_h) {
-  PFN_encodeTiled enc = get_encode();
-  if (!enc) return 1;
-  cuuint64_t dims[4] = {(cuuint64_t)C, (cuuint64_t)W, (cuuint64_t)H, (cuuint64_t)B};
-  cuuint64_t strides[3] = {pix_bytes, row_bytes, img_bytes};
-  cuuint32_t box[4] = {box_c, box_w, box_h, 1};
-  cuuint32_t es[4] = {1, 1, 1, 1};
-  CUresult r = enc(m, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, const_cast<void*>(base), dims, strides, box, es,
-                   CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                   CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  if (r != CUDA_SUCCESS) {
-    set_error("cuTensorMapEncodeTiled(strided nhwc B=%d H=%d W=%d C=%d) failed with CUresult %d", B, H, W, C, (int)r);
-    return 1;
-  }
-  return 0;
-}
-
-// 2-D map without shared-memory swizzle (dense box rows)
-int make_tmap_2d_plain(CUtensorMap* m, const void* base, int elem_bytes, uint64_t inner, uint64_t outer, uint64_t pitch_bytes,
-                       uint32_t box_inner, uint32_t box_outer) {
-  PFN_encodeTiled enc = get_encode();
-  if (!enc) return 1;
-  const CUtensorMapDataType dt = elem_bytes == 4 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT32 : CU_TENSOR_MAP_DATA_TYPE_BFLOAT16;
-  cuuint64_t dims[2] = {inner, outer};
-  cuuint64_t strides[1] = {pitch_bytes};
-  cuuint32_t box[2] = {box_inner, box_outer};
-  cuuint32_t es[2] = {1, 1};
-  CUresult r = enc(m, dt, 2, const_cast<void*>(base), dims, strides, box, es, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE,
-                   CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  if (r != CUDA_SUCCESS) { set_error("cuTensorMapEncodeTiled(2d plain) failed with CUresult %d", (int)r); return 1; }
-  return 0;
+  const cuuint64_t dims[4] = {(cuuint64_t)C, (cuuint64_t)W, (cuuint64_t)H, (cuuint64_t)B}, strides[3] = {pix_bytes, row_bytes, img_bytes};
+  const cuuint32_t box[4] = {box_c, box_w, box_h, 1};
+  return encode_tmap(m, base, 2, 4, dims, strides, box);
 }
 
 template <int BN>

@@ -13,6 +13,7 @@ NotImplementedError where they would change the result.
 """
 from __future__ import annotations
 
+import contextlib
 import ctypes
 import math
 import warnings
@@ -49,6 +50,16 @@ def x8_group(B: int, H: int, W: int) -> int:
         if n <= X8_GROUP_TOKENS and n * 16 < 2 ** 31:
             return g
     return 1
+
+
+def _ws_alloc_bytes(nbytes: int) -> int:
+    """Size of a tensor that holds a library workspace of `nbytes` from its first 256-byte boundary on (_ws_offset)."""
+    return nbytes + 256
+
+
+def _ws_offset(ws: torch.Tensor) -> int:
+    """Bytes from the start of `ws` to its first 256-byte boundary: the library takes 256-byte aligned workspaces."""
+    return -ws.data_ptr() % 256
 
 
 def _trunc_normal_(t: torch.Tensor, std: float = .02):
@@ -451,7 +462,21 @@ class HiT_SIR(nn.Module, PyTorchModelHubMixin):
                 _capi.check(lib.hitsir_workspace_bytes_x8(h, B, H, W, group, ctypes.byref(n)))
             else:
                 _capi.check(lib.hitsir_workspace_bytes(h, B, H, W, ctypes.byref(n)))
-        return torch.empty(n.value + 256, dtype=torch.uint8, device=device)
+        return torch.empty(_ws_alloc_bytes(n.value), dtype=torch.uint8, device=device)
+
+    @contextlib.contextmanager
+    def _native_call(self, device, shape=None, ws: Optional[torch.Tensor] = None, stream: Optional[int] = None):
+        """Enters `device` for one call of a forward entry of the C ABI: creates the handle and syncs the weights on `stream` (default:
+        the device's current stream), then yields (library, handle, workspace pointer, workspace bytes, stream) for `ws`, or for the
+        cached workspace of `shape` = (B, H, W[, group]) when `ws` is None."""
+        with torch.cuda.device(device):
+            stream = torch.cuda.current_stream(device).cuda_stream if stream is None else stream
+            h = self._handle(device)
+            self._sync_weights(h, device, stream)
+            if ws is None:
+                ws = self._workspace(h, device, *shape)
+            off = _ws_offset(ws)
+            yield _capi.load(), h, ctypes.c_void_p(ws.data_ptr() + off), ws.numel() - off, ctypes.c_void_p(stream)
 
     def set_inject(self, device, name: Optional[str], src: Optional[torch.Tensor] = None):
         """Test hook (stands in for a forward pre-hook that replaces a sub-module's input), see hitsir_set_inject.  `src` is kept
@@ -525,17 +550,9 @@ class HiT_SIR(nn.Module, PyTorchModelHubMixin):
         B, _, H, W = x.shape
         in_dtype = x.dtype
         xin = x.detach().to(torch.float32).contiguous()
-        device = xin.device
-        stream = torch.cuda.current_stream(device).cuda_stream
-        lib = _capi.load()
-        with torch.cuda.device(device):
-            h = self._handle(device)
-            self._sync_weights(h, device, stream)
-            ws = self._forced_workspace if self._forced_workspace is not None else self._workspace(h, device, B, H, W)
-            base = (ws.data_ptr() + 255) // 256 * 256
-            y = torch.empty((B, self.in_chans, H * self.out_scale, W * self.out_scale), dtype=torch.float32, device=device)
-            _capi.check(lib.hitsir_forward(h, ctypes.c_void_p(xin.data_ptr()), ctypes.c_void_p(y.data_ptr()), B, H, W,
-                                           ctypes.c_void_p(base), ws.numel() - (base - ws.data_ptr()), ctypes.c_void_p(stream)))
+        y = torch.empty((B, self.in_chans, H * self.out_scale, W * self.out_scale), dtype=torch.float32, device=xin.device)
+        with self._native_call(xin.device, (B, H, W), self._forced_workspace) as (lib, h, ws, ws_bytes, st):
+            _capi.check(lib.hitsir_forward(h, ctypes.c_void_p(xin.data_ptr()), ctypes.c_void_p(y.data_ptr()), B, H, W, ws, ws_bytes, st))
             self.last_launch_count = int(lib.hitsir_last_launch_count(h))
         return y if in_dtype == torch.float32 else y.to(in_dtype)
 
@@ -551,17 +568,10 @@ class HiT_SIR(nn.Module, PyTorchModelHubMixin):
         group = x8_group(B, H, W) if group is None else group
         in_dtype = x.dtype
         xin = x.detach().to(torch.float32).contiguous()
-        device = xin.device
-        stream = torch.cuda.current_stream(device).cuda_stream
-        lib = _capi.load()
-        with torch.cuda.device(device):
-            h = self._handle(device)
-            self._sync_weights(h, device, stream)
-            ws = self._workspace(h, device, B, H, W, group)
-            base = (ws.data_ptr() + 255) // 256 * 256
-            y = torch.empty((B, self.in_chans, H * self.out_scale, W * self.out_scale), dtype=torch.float32, device=device)
+        y = torch.empty((B, self.in_chans, H * self.out_scale, W * self.out_scale), dtype=torch.float32, device=xin.device)
+        with self._native_call(xin.device, (B, H, W, group)) as (lib, h, ws, ws_bytes, st):
             _capi.check(lib.hitsir_forward_x8(h, ctypes.c_void_p(xin.data_ptr()), ctypes.c_void_p(y.data_ptr()), B, H, W, group,
-                                              ctypes.c_void_p(base), ws.numel() - (base - ws.data_ptr()), ctypes.c_void_p(stream)))
+                                              ws, ws_bytes, st))
             self.last_launch_count = int(lib.hitsir_last_launch_count(h))
         return y if in_dtype == torch.float32 else y.to(in_dtype)
 
@@ -575,18 +585,11 @@ class HiT_SIR(nn.Module, PyTorchModelHubMixin):
         x_host = x_host.contiguous().float()
         if y_host is None:
             y_host = torch.empty((B, self.in_chans, H * self.out_scale, W * self.out_scale), dtype=torch.float32, pin_memory=True)
-        lib = _capi.load()
-        with torch.cuda.device(device):
-            stream = torch.cuda.current_stream(device).cuda_stream
-            h = self._handle(device)
-            self._sync_weights(h, device, stream)
-            ws = self._workspace(h, device, B, H, W)
-            base = (ws.data_ptr() + 255) // 256 * 256
-            dx = torch.empty(x_host.shape, dtype=torch.float32, device=device)
-            dy = torch.empty(y_host.shape, dtype=torch.float32, device=device)
+        dx = torch.empty(x_host.shape, dtype=torch.float32, device=device)
+        dy = torch.empty(y_host.shape, dtype=torch.float32, device=device)
+        with self._native_call(device, (B, H, W)) as (lib, h, ws, ws_bytes, st):
             _capi.check(lib.hitsir_forward_host(h, ctypes.c_void_p(x_host.data_ptr()), ctypes.c_void_p(y_host.data_ptr()), B, H, W,
-                                                ctypes.c_void_p(dx.data_ptr()), ctypes.c_void_p(dy.data_ptr()),
-                                                ctypes.c_void_p(base), ws.numel() - (base - ws.data_ptr()), ctypes.c_void_p(stream)))
+                                                ctypes.c_void_p(dx.data_ptr()), ctypes.c_void_p(dy.data_ptr()), ws, ws_bytes, st))
             torch.cuda.current_stream(device).synchronize()
             self.last_launch_count = int(lib.hitsir_last_launch_count(h))
         return y_host
@@ -605,26 +608,18 @@ class HiT_SIR(nn.Module, PyTorchModelHubMixin):
         device = x_u8.device
         x_u8 = x_u8.contiguous()
         y = torch.empty((B, H * self.out_scale, W * self.out_scale, C), dtype=torch.uint8, device=device)
-        lib = _capi.load()
-        with torch.cuda.device(device):
-            stream = torch.cuda.current_stream(device).cuda_stream
-            h = self._handle(device)
-            self._sync_weights(h, device, stream)
-            if self_ensemble:
-                group = x8_group(B, H, W)
-                ws = self._workspace(h, device, B, H, W, group)
-                base = (ws.data_ptr() + 255) // 256 * 256
+        if self_ensemble:
+            group = x8_group(B, H, W)
+            with self._native_call(device, (B, H, W, group)) as (lib, h, ws, ws_bytes, st):
                 _capi.check(lib.hitsir_forward_x8_u8(h, ctypes.c_void_p(x_u8.data_ptr()), ctypes.c_void_p(y.data_ptr()), B, H, W, group,
-                                                     ctypes.c_void_p(base), ws.numel() - (base - ws.data_ptr()), ctypes.c_void_p(stream)))
+                                                     ws, ws_bytes, st))
                 self.last_launch_count = int(lib.hitsir_last_launch_count(h))
-                return y
-            ws = self._workspace(h, device, B, H, W)
-            base = (ws.data_ptr() + 255) // 256 * 256
-            dx = torch.empty((B, C, H, W), dtype=torch.float32, device=device)
-            dy = torch.empty((B, C, H * self.out_scale, W * self.out_scale), dtype=torch.float32, device=device)
+            return y
+        dx = torch.empty((B, C, H, W), dtype=torch.float32, device=device)
+        dy = torch.empty((B, C, H * self.out_scale, W * self.out_scale), dtype=torch.float32, device=device)
+        with self._native_call(device, (B, H, W)) as (lib, h, ws, ws_bytes, st):
             _capi.check(lib.hitsir_forward_u8(h, ctypes.c_void_p(x_u8.data_ptr()), ctypes.c_void_p(y.data_ptr()), B, H, W,
-                                              ctypes.c_void_p(dx.data_ptr()), ctypes.c_void_p(dy.data_ptr()),
-                                              ctypes.c_void_p(base), ws.numel() - (base - ws.data_ptr()), ctypes.c_void_p(stream)))
+                                              ctypes.c_void_p(dx.data_ptr()), ctypes.c_void_p(dy.data_ptr()), ws, ws_bytes, st))
             self.last_launch_count = int(lib.hitsir_last_launch_count(h))
         return y
 
