@@ -450,6 +450,10 @@ int finalize(HitsirHandle* h, cudaStream_t st) {
       if (make_gemm_w(h, &bw.proj, s + ".proj", C, C, 1, st, 1)) return 1;
       if (make_gemm_w(h, &bw.fc1, p + ".mlp.fc1", kHid, C, 1, st)) return 1;
       if (make_gemm_w(h, &bw.fc2, p + ".mlp.fc2", C, kHid, 1, st)) return 1;
+      if (bw.proj.Npad != kCp || bw.proj.K != kCp || bw.fc1.Npad != kHidp || bw.fc1.K != kCp) {
+        set_error("proj / fc1 packing %d x %d / %d x %d is not the 192 x 192 / 384 x 192 proj_fc1 expects", bw.proj.Npad, bw.proj.K, bw.fc1.Npad, bw.fc1.K);
+        return 1;
+      }
       // [26][384] fp32: 25 tap rows + the bias as row 25 (one TMA box per 64-channel slice in ffn_tail.cu)
       if (dev_alloc(h, &bw.dw_w, 26 * kHidp)) return 1;
       bw.dw_b = bw.dw_w + 25 * kHidp;
@@ -738,11 +742,11 @@ void base_params(GemmParams& p, const GemmW& w) {
   p.slope = 1.f;
 }
 
-// The staged-epilogue kernel covers the plain-store and LayerNorm epilogues; the gate / pixel-shuffle
-// epilogues (once per forward) keep the direct-store kernel.
+// The staged-epilogue kernel covers the plain-store and gate epilogues; the pixel-shuffle epilogues (once per forward) keep the
+// direct-store kernel.
 bool tma_epilogue(const GemmW& w, const GemmParams& p) {
   if (p.epi == EPI_MSGATE) return w.BN == 160;
-  return (p.epi == EPI_STORE || p.epi == EPI_LN) && (w.BN == 192 || w.BN == 64) && p.out2_f32 == nullptr && w.Npad <= 384;
+  return p.epi == EPI_STORE && (w.BN == 192 || w.BN == 64) && w.Npad <= 384;
 }
 
 int run_gemm(Fwd& f, const char* cat, const GemmW& w, GemmParams& p, const CUtensorMap* maps, bool tma) {
@@ -787,7 +791,7 @@ int conv3(Fwd& f, const char* cat, const GemmW& w, const bf16* A, int B, int H, 
   RUN(conv_geometry(f, A, B, H, W, Cpad, p));
   if (w.K != 9 * Cpad) { set_error("conv3: packed K %d != 9*%d", w.K, Cpad); return 1; }
   // 64-channel inputs (HR stage): resident filter bank + kx-shared halo boxes (conv3_c64.cu)
-  if (Cpad == 64 && p.res == nullptr && p.out2_f32 == nullptr &&
+  if (Cpad == 64 && p.res == nullptr &&
       ((w.BN == 64 && p.epi == EPI_STORE && p.out_bf16 != nullptr && p.out_f32 == nullptr && p.ldb == 64) ||
        (w.BN == 16 && w.wf != nullptr && p.res_img == nullptr && p.epi == EPI_SHUFFLE_NCHW && p.ps == 1 && p.n_real <= 4))) {
     LAUNCH(cat, 1, w.BN == 16 ? launch_conv_last_fold(p, A, w.tmf, f.h->num_sms, f.st) : launch_conv3_c64(w.BN, p, A, w.tm, f.h->num_sms, f.st));
@@ -871,17 +875,19 @@ int forward_block(Fwd& f, int i, int j, float* xin, float* xout) {
   }
   TAP((tn + ".sccdbg").c_str(), ws.scc_dbg, 0, kSccDbgFloats, 1, kSccDbgFloats);
   TAPP((tn + ".scc").c_str(), ws.outsc, 1, kCp, f.N, kC);
-  // proj + norm1 + residual (:597, :700-703)
-  GemmParams p;
-  base_params(p, bw.proj);
-  p.epi = EPI_LN; p.n_real = kC; p.gamma = bw.g1; p.beta = bw.b1; p.res = xin; p.ldr = kC;
-  p.out_f32 = xout; p.ldf = kC; p.out_bf16 = ws.xb0; p.ldb = kCp;
-  RUN(linear(f, "gemm_proj_ln", bw.proj, ws.outsc, f.N, p));
+  // proj + norm1 + residual (:597, :700-703) and ConvFFN fc1 + GELU (:39-41) in one kernel
+  {
+    const long long M = f.N;
+    CUtensorMap maps[6];
+    maps[1] = bw.proj.tm; maps[2] = bw.fc1.tm;
+    if (make_tmap_2d(&maps[0], ws.outsc, (uint64_t)kCp, (uint64_t)M, (uint64_t)kCp * 2, 64, 128)) return 1;
+    if (make_tmap_2d_t(&maps[3], xin, 4, (uint64_t)kC, (uint64_t)M, (uint64_t)kC * 4, 32, 128)) return 1;
+    if (make_tmap_2d_t(&maps[4], xout, 4, (uint64_t)kC, (uint64_t)M, (uint64_t)kC * 4, 32, 128)) return 1;
+    if (make_tmap_2d_t(&maps[5], ws.H1, 2, (uint64_t)kHidp, (uint64_t)M, (uint64_t)kHidp * 2, 64, 128)) return 1;
+    const ProjFc1Params pp{(int)cdiv64(M, 128), bw.proj.b, bw.g1, bw.b1, bw.fc1.b};
+    LAUNCH("proj_fc1", 1, launch_proj_fc1(pp, maps, h->num_sms, f.st));
+  }
   TAP((tn + ".attn").c_str(), xout, 0, kC, f.N, kC);
-  // ConvFFN (:39-46): fc1 + GELU
-  base_params(p, bw.fc1);
-  p.epi = EPI_STORE; p.act = ACT_GELU; p.n_real = kHid; p.out_bf16 = ws.H1; p.ldb = kHidp;
-  RUN(linear(f, "gemm_fc1_gelu", bw.fc1, ws.xb0, f.N, p));
   TAP((tn + ".fc1").c_str(), ws.H1, 1, kHidp, f.N, kHid);
   const bool need_shadow = (j == c.depths[i] - 1);      // the RHTB conv after the last block reads a bf16 shadow of the stream (:934)
   // dwconv5 + GELU + input, fc2, norm2 and the residual add in one kernel: the hidden map h2 never reaches HBM

@@ -13,7 +13,6 @@ namespace hitsir {
 
 enum EpiMode : int {
   EPI_STORE = 0,    // v = act(acc + bias) (+ res)            -> out_f32 / out_bf16
-  EPI_LN = 1,       // v = acc + bias; (out2 = v); y = LN(v)*g + b (+ res) -> out_f32 / out_bf16   (BN == 192, one N tile)
   EPI_MSGATE = 2,   // MultipleSizeConvExtract gate (hit_sir_pro.py:83-92), see epilogue
   EPI_SHUFFLE_NCHW = 3,  // pixel-shuffle(ps) + de-normalise -> NCHW fp32 image
   EPI_SHUFFLE_BF16 = 4,  // pixel-shuffle(ps) -> NHWC bf16 feature map with `shuf_c` channels
@@ -37,10 +36,8 @@ struct GemmParams {
   float slope;       // leaky-relu slope
   const float* bias; // [n_tiles*BN], zero padded
   const float* res; int ldr;      // fp32 residual rows
-  const float* gamma; const float* beta;
   float* out_f32; int ldf;
   bf16* out_bf16; int ldb;        // columns [0, ldb) are written (zeros beyond n_real)
-  float* out2_f32; int ldf2;
   // shuffle epilogues
   int ps;            // pixel-shuffle factor (1 = none)
   int shuf_c;        // channels after shuffle (NCHW: image channels; BF16: feature channels = ldb)
@@ -132,70 +129,6 @@ __device__ __forceinline__ void epilogue_row(const GemmParams& p, Acc& acc, cons
         o[1] = make_uint4(w[4], w[5], w[6], w[7]);
       }
     }
-  } else if (p.epi == EPI_LN) {
-    // LayerNorm over the n_real columns of this row (eps 1e-5, hit_sir_pro.py:651,659,1219), then optional residual.
-    float s = 0.f;
-#pragma unroll 1
-    for (int c0 = 0; c0 < BN; c0 += 16) {
-      float v[16];
-      acc.load16(c0, v);
-#pragma unroll
-      for (int i = 0; i < 16; ++i)
-        if (c0 + i < p.n_real) s += v[i] + __ldg(p.bias + c0 + i);
-    }
-    const float mean = s / (float)p.n_real;
-    float q = 0.f;
-#pragma unroll 1
-    for (int c0 = 0; c0 < BN; c0 += 16) {
-      float v[16];
-      acc.load16(c0, v);
-#pragma unroll
-      for (int i = 0; i < 16; ++i)
-        if (c0 + i < p.n_real) { float d = v[i] + __ldg(p.bias + c0 + i) - mean; q += d * d; }
-    }
-    const float rstd = rsqrtf(q / (float)p.n_real + 1e-5f);
-#pragma unroll 1
-    for (int c0 = 0; c0 < BN; c0 += 16) {
-      float v[16];
-      acc.load16(c0, v);
-      if (!ri.valid) continue;
-      float pre[16];
-#pragma unroll
-      for (int i = 0; i < 16; ++i) {
-        const int c = c0 + i;
-        const bool ok = c < p.n_real;
-        float t = ok ? v[i] + __ldg(p.bias + c) : 0.f;
-        pre[i] = t;
-        float y = ok ? (t - mean) * rstd * __ldg(p.gamma + c) + __ldg(p.beta + c) : 0.f;
-        if (ok && p.res != nullptr) y += __ldg(p.res + ri.grow * p.ldr + c);
-        v[i] = y;
-      }
-      if (p.out2_f32 != nullptr) {
-        float* o = p.out2_f32 + ri.grow * p.ldf2 + c0;
-#pragma unroll
-        for (int i = 0; i < 16; ++i)
-          if (c0 + i < p.n_real) o[i] = pre[i];
-      }
-      if (p.out_f32 != nullptr) {
-        float* o = p.out_f32 + ri.grow * p.ldf + c0;
-        if (c0 + 16 <= p.n_real && (p.ldf & 3) == 0) {
-#pragma unroll
-          for (int i = 0; i < 16; i += 4) *reinterpret_cast<float4*>(o + i) = make_float4(v[i], v[i + 1], v[i + 2], v[i + 3]);
-        } else {
-#pragma unroll
-          for (int i = 0; i < 16; ++i)
-            if (c0 + i < p.n_real) o[i] = v[i];
-        }
-      }
-      if (p.out_bf16 != nullptr && c0 < p.ldb) {
-        uint32_t w[8];
-#pragma unroll
-        for (int i = 0; i < 8; ++i) w[i] = pack_bf16x2(v[2 * i], v[2 * i + 1]);
-        uint4* o = reinterpret_cast<uint4*>(p.out_bf16 + ri.grow * p.ldb + c0);
-        o[0] = make_uint4(w[0], w[1], w[2], w[3]);
-        o[1] = make_uint4(w[4], w[5], w[6], w[7]);
-      }
-    }
   } else if (p.epi == EPI_MSGATE) {
     // N tile `n_tile` (BN == 160) holds, for the 32 embedding channels c = 32*n_tile + i:
     //   cols [32k, 32k+32), k=0..3 : conv3/5/7/9 outputs, cols [128,160): conv_x (1x1) output.
@@ -273,6 +206,15 @@ int launch_conv3_c64_up(const GemmParams& p, const bf16* A, const CUtensorMap& t
 int launch_conv_last_fold(const GemmParams& p, const bf16* A, const CUtensorMap& tb, int num_sms, cudaStream_t st);
 int launch_conv3_c64(int BN, const GemmParams& p, const bf16* A, const CUtensorMap& tb, int num_sms, cudaStream_t st);
 int launch_umma_gemm_tma(int BN, const GemmParams& p, const CUtensorMap* maps, int num_sms, cudaStream_t st);
+// proj + norm1 + residual and fc1 + GELU of one transformer block (proj_fc1.cu); maps: {outsc [M,192] bf16 box {64,128}, Wp and W1 packed
+// (box {64,192}), residual x and stream x' fp32 [M,180] box {32,128}, h1 bf16 [M,384] box {64,128}}
+struct ProjFc1Params {
+  int m_tiles;
+  const float* bias_p;               // [192], zero padded
+  const float* gamma; const float* beta;   // norm1, [180]
+  const float* bias1;                // [384], zero padded
+};
+int launch_proj_fc1(const ProjFc1Params& p, const CUtensorMap* maps, int num_sms, cudaStream_t st);
 int launch_umma_gemm(int BN, const GemmParams& p, const CUtensorMap& ta, const CUtensorMap& tb, int num_sms, cudaStream_t st);
 
 }  // namespace hitsir
