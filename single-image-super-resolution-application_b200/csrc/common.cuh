@@ -42,9 +42,6 @@ static inline int round_up(int a, int b) { return cdiv(a, b) * b; }
 // ---------------------------------------------------------------------------
 // small math
 // ---------------------------------------------------------------------------
-__device__ __forceinline__ float gelu_erf(float x) {          // nn.GELU() default (erf form)
-  return 0.5f * x * (1.0f + erff(x * 0.70710678118654752440f));
-}
 __device__ __forceinline__ float ex2_approx(float x) { float y; asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(x)); return y; }
 __device__ __forceinline__ float rcp_approx(float x) { float y; asm("rcp.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(x)); return y; }
 __device__ __forceinline__ float tanh_approx(float x) { float y; asm("tanh.approx.f32 %0, %1;" : "=f"(y) : "f"(x)); return y; }
@@ -143,6 +140,25 @@ __device__ __forceinline__ void mbar_wait_park(uint32_t bar, uint32_t parity, ui
       "DONE:\n\t"
       "}" ::"r"(bar), "r"(parity), "r"(hint_ns) : "memory");
 }
+// mbarrier wait with a watchdog: a protocol bug traps (-> launch error) instead of hanging the device
+__device__ __forceinline__ void wait_bar(uint32_t bar, uint32_t parity) {
+  uint32_t done = 0;
+  long long spins = 0;
+  while (true) {
+    asm volatile(
+        "{\n\t.reg .pred p;\n\t"
+        "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"
+        "selp.u32 %0, 1, 0, p;\n\t}"
+        : "=r"(done) : "r"(bar), "r"(parity) : "memory");
+    if (done) break;
+    if (++spins > (1LL << 26)) {
+      printf("mbarrier timeout (block %d thread %d bar %u parity %u)\n", blockIdx.x, threadIdx.x, (bar >> 3) & 31u, parity);
+      __trap();
+    }
+  }
+}
+// barrier `id` (1..15) over the first `nthreads` threads that reach it: a subset of the CTA's warps synchronises without the others
+__device__ __forceinline__ void named_bar_sync(int id, int nthreads) { asm volatile("bar.sync %0, %1;" ::"r"(id), "r"(nthreads) : "memory"); }
 // Programmatic dependent launch (the per-block chain casa gate -> SCC -> proj -> fc1 -> FFN tail -> pool MLP is 6 dependent launches x 36
 // blocks; on small inputs the grid launch latency between them is a sixth of the forward).  A kernel launched with launch_pdl() may
 // become resident while its predecessor in the stream is still draining; pdl_entry() holds it until that grid has completed and its
@@ -186,6 +202,20 @@ __device__ __forceinline__ void tma_load_4d(uint32_t dst, const void* tmap, uint
       "cp.async.bulk.tensor.4d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5, %6}], [%2];"
       ::"r"(dst), "l"(tmap), "r"(bar), "r"(c0), "r"(c1), "r"(c2), "r"(c3) : "memory");
 }
+// shared -> global tensor stores, tracked as bulk groups of the issuing thread
+__device__ __forceinline__ void tma_store_2d(const void* tmap, uint32_t src, int c0, int c1) {
+  asm volatile("cp.async.bulk.tensor.2d.global.shared::cta.bulk_group [%0, {%2, %3}], [%1];" ::"l"(tmap), "r"(src), "r"(c0), "r"(c1) : "memory");
+}
+__device__ __forceinline__ void tma_store_4d(const void* tmap, uint32_t src, int c0, int c1, int c2, int c3) {
+  asm volatile("cp.async.bulk.tensor.4d.global.shared::cta.bulk_group [%0, {%2, %3, %4, %5}], [%1];" ::"l"(tmap), "r"(src), "r"(c0), "r"(c1),
+               "r"(c2), "r"(c3) : "memory");
+}
+__device__ __forceinline__ void tma_commit() { asm volatile("cp.async.bulk.commit_group;" ::: "memory"); }
+// until at most N of this thread's bulk groups are still reading shared memory (N = 1: all but the newest)
+template <int N>
+__device__ __forceinline__ void tma_wait_read() { asm volatile("cp.async.bulk.wait_group.read %0;" ::"n"(N) : "memory"); }
+// until every bulk group of this thread has completed (its global writes done)
+__device__ __forceinline__ void tma_wait_all0() { asm volatile("cp.async.bulk.wait_group 0;" ::: "memory"); }
 
 __device__ __forceinline__ void tc_fence_before() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
 __device__ __forceinline__ void tc_fence_after() { asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory"); }
@@ -239,7 +269,22 @@ __device__ __forceinline__ void reg_fence16(uint32_t* r) {
                     "+r"(r[8]), "+r"(r[9]), "+r"(r[10]), "+r"(r[11]), "+r"(r[12]), "+r"(r[13]), "+r"(r[14]), "+r"(r[15]));
 }
 
-// 32 consecutive fp32 columns with a single wait
+// NG x 16 consecutive accumulator columns of this thread's TMEM lane -> registers with a single wait
+template <int NG>
+__device__ __forceinline__ void tmem_ld_cols(uint32_t taddr, float (&v)[NG][16]) {
+  uint32_t r[NG][16];
+#pragma unroll
+  for (int i = 0; i < NG; ++i) tmem_ld16_nw(taddr + 16 * i, r[i]);
+  tmem_ld_wait();
+#pragma unroll
+  for (int i = 0; i < NG; ++i) {
+    reg_fence16(r[i]);
+#pragma unroll
+    for (int e = 0; e < 16; ++e) v[i][e] = __uint_as_float(r[i][e]);
+  }
+}
+// 32 consecutive fp32 columns with a single wait (the same loads as tmem_ld_cols<2>; written out, it keeps the conv3_c64_up epilogue's
+// instruction schedule)
 __device__ __forceinline__ void tmem_ld32(uint32_t taddr, float* v) {
   uint32_t r0[16], r1[16];
   tmem_ld16_nw(taddr, r0);
@@ -251,20 +296,41 @@ __device__ __forceinline__ void tmem_ld32(uint32_t taddr, float* v) {
   for (int i = 0; i < 16; ++i) { v[i] = __uint_as_float(r0[i]); v[16 + i] = __uint_as_float(r1[i]); }
 }
 
-// UMMA shared-memory matrix descriptor: K-major operand, 128-byte swizzle, rows of 128 B,
-// 8-row swizzle atoms 1024 B apart (SBO), version 1 (sm_100), layout type 2 (SWIZZLE_128B).
-__device__ __forceinline__ uint64_t umma_desc_sw128(uint32_t saddr) {
+// 16-byte chunk address inside a SWIZZLE_128B block with 128-byte rows
+__device__ __forceinline__ uint8_t* swz(uint8_t* block, int row, int chunk) { return block + row * 128 + ((chunk ^ (row & 7)) << 4); }
+// 16 fp32 values -> bf16 chunks chunk0, chunk0 + 1 of `row`
+__device__ __forceinline__ void store16(uint8_t* block, int row, int chunk0, const float* v) {
+  *reinterpret_cast<uint4*>(swz(block, row, chunk0)) =
+      make_uint4(pack_bf16x2(v[0], v[1]), pack_bf16x2(v[2], v[3]), pack_bf16x2(v[4], v[5]), pack_bf16x2(v[6], v[7]));
+  *reinterpret_cast<uint4*>(swz(block, row, chunk0 + 1)) =
+      make_uint4(pack_bf16x2(v[8], v[9]), pack_bf16x2(v[10], v[11]), pack_bf16x2(v[12], v[13]), pack_bf16x2(v[14], v[15]));
+}
+
+// UMMA shared-memory matrix descriptor, SWIZZLE_128B (layout type 2), descriptor version 1 (sm_100).  K-major: lbo ignored, sbo = 1024
+// (8 rows of 128 B).  MN-major: lbo = stride between 64-element blocks along M/N, sbo = stride between 8-row groups along K
+// (cute/atom/mma_traits_sm100.hpp canonical forms).
+__device__ __forceinline__ uint64_t make_desc(uint32_t saddr, uint32_t lbo_bytes, uint32_t sbo_bytes) {
   uint64_t d = 0;
   d |= (uint64_t)((saddr & 0x3FFFFu) >> 4);      // start address, bits [0,14)
-  d |= (uint64_t)1 << 16;                        // LBO (ignored for swizzled K-major), bits [16,30)
-  d |= (uint64_t)(1024 >> 4) << 32;              // SBO = 1024 B, bits [32,46)
-  d |= (uint64_t)1 << 46;                        // descriptor version (Blackwell)
-  d |= (uint64_t)2 << 61;                        // SWIZZLE_128B
+  d |= (uint64_t)(lbo_bytes >> 4) << 16;         // bits [16,30)
+  d |= (uint64_t)(sbo_bytes >> 4) << 32;         // bits [32,46)
+  d |= (uint64_t)1 << 46;
+  d |= (uint64_t)2 << 61;
   return d;
 }
-// instruction descriptor for kind::f16: D=f32, A=B=bf16, both K-major, M=128, N=n
-__host__ __device__ constexpr uint32_t umma_idesc_bf16(int m, int n) {
-  return (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(n >> 3) << 17) | ((uint32_t)(m >> 4) << 24);
+// K-major operand with 128-byte rows
+__device__ __forceinline__ uint64_t umma_desc_sw128(uint32_t saddr) { return make_desc(saddr, 16, 1024); }
+// instruction descriptor for kind::f16: D = f32, A = B = bf16, M = m, N = n; a_mn / b_mn = 1: that operand is MN-major (0: K-major)
+__host__ __device__ constexpr uint32_t make_idesc(int m, int n, int a_mn, int b_mn) {
+  return (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)a_mn << 15) | ((uint32_t)b_mn << 16) | ((uint32_t)(n >> 3) << 17) |
+         ((uint32_t)(m >> 4) << 24);
+}
+__host__ __device__ constexpr uint32_t umma_idesc_bf16(int m, int n) { return make_idesc(m, n, 0, 0); }
+
+// warp-level bf16 MMA m16n8k16, fp32 accumulate in place: A = four fragment registers, B = two
+__device__ __forceinline__ void mma_bf16_16816(float* d, uint32_t a0, uint32_t a1, uint32_t a2, uint32_t a3, uint32_t b0, uint32_t b1) {
+  asm volatile("mma.sync.aligned.m16n8k16.row.col.f32.bf16.bf16.f32 {%0,%1,%2,%3}, {%4,%5,%6,%7}, {%8,%9}, {%0,%1,%2,%3};"
+               : "+f"(d[0]), "+f"(d[1]), "+f"(d[2]), "+f"(d[3]) : "r"(a0), "r"(a1), "r"(a2), "r"(a3), "r"(b0), "r"(b1));
 }
 
 }  // namespace hitsir

@@ -33,14 +33,6 @@ struct Cfg {
   static constexpr int kTmemCols = 128;
 };
 
-__device__ __forceinline__ void tma_store_4d(const void* tmap, uint32_t src, int c0, int c1, int c2, int c3) {
-  asm volatile("cp.async.bulk.tensor.4d.global.shared::cta.bulk_group [%0, {%2, %3, %4, %5}], [%1];" ::"l"(tmap), "r"(src), "r"(c0), "r"(c1),
-               "r"(c2), "r"(c3) : "memory");
-}
-__device__ __forceinline__ void tma_commit() { asm volatile("cp.async.bulk.commit_group;" ::: "memory"); }
-__device__ __forceinline__ void tma_wait_read1() { asm volatile("cp.async.bulk.wait_group.read 1;" ::: "memory"); }
-__device__ __forceinline__ void tma_wait_all0() { asm volatile("cp.async.bulk.wait_group 0;" ::: "memory"); }
-
 template <int BN>
 __global__ void __launch_bounds__(384, 1)
 conv3_c64_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant__ CUtensorMap tmap_b, const __grid_constant__ CUtensorMap tmap_o,
@@ -77,11 +69,6 @@ conv3_c64_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_consta
   tc_fence_after();
   const uint32_t tmem_base = *tmem_ptr_smem;
 
-  auto tile_xyb = [&](int t, int* x0, int* y0, int* b) {
-    const int tx = t % p.tiles_x; const int t2 = t / p.tiles_x;
-    *x0 = tx * 16; *y0 = (t2 % p.tiles_y) * 8; *b = t2 / p.tiles_y;
-  };
-
   if (warp == 0) {
     if (lane == 0) {
       // ===================== producer: filter bank once, then one halo box per (tile, kx) =====================
@@ -89,7 +76,7 @@ conv3_c64_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_consta
       for (int tap = 0; tap < 9; ++tap) tma_load_2d(sb + tap * BN * 128, &tmap_b, b_full, tap * 64, 0);
       uint32_t cnt = 0;
       for (int t = blockIdx.x; t < total; t += gridDim.x) {
-        int x0, y0, b; tile_xyb(t, &x0, &y0, &b);
+        const auto [b, y0, x0] = conv_tile(t, p.tiles_x, p.tiles_y);
         for (int kx = 0; kx < 3; ++kx, ++cnt) {
           const int s = (int)(cnt % kAStages);
           mbar_wait(empty_bar(s), ((cnt / kAStages) & 1u) ^ 1u);
@@ -132,12 +119,12 @@ conv3_c64_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_consta
       // ===================== TMA store of finished boxes =====================
       uint32_t u = 0;
       for (int t = blockIdx.x; t < total; t += gridDim.x, ++u) {
-        int x0, y0, b; tile_xyb(t, &x0, &y0, &b);
+        const auto [b, y0, x0] = conv_tile(t, p.tiles_x, p.tiles_y);
         const int s = (int)(u % kNBox);
         mbar_wait(box_ready(s), (u / kNBox) & 1u);
         tma_store_4d(&tmap_o, sb + C::kOffBox + s * kBoxBytes, 0, x0, y0, b);
         tma_commit();
-        tma_wait_read1();                                  // groups retire in order: the previous box is free again
+        tma_wait_read<1>();                                // groups retire in order: the previous box is free again
         if (u >= 1) mbar_arrive(box_free((int)((u - 1) % kNBox)));
       }
       tma_wait_all0();
@@ -239,11 +226,6 @@ conv3_c64_up_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_con
   tc_fence_after();
   const uint32_t tmem_base = *tmem_ptr_smem;
 
-  auto tile_xyb = [&](int t, int* x0, int* y0, int* b) {
-    const int tx = t % p.tiles_x; const int t2 = t / p.tiles_x;
-    *x0 = tx * 16; *y0 = (t2 % p.tiles_y) * 8; *b = t2 / p.tiles_y;
-  };
-
   if (warp == 0) {
     if (lane == 0) {
       // ===================== producer: phase filters once, then one LR halo box per (tile, kx) =====================
@@ -251,7 +233,7 @@ conv3_c64_up_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_con
       for (int tap = 0; tap < 16; ++tap) tma_load_2d(sb + tap * 64 * 128, &tmap_b, b_full, tap * 64, 0);
       uint32_t cnt = 0;
       for (int t = blockIdx.x; t < total; t += gridDim.x) {
-        int x0, y0, b; tile_xyb(t, &x0, &y0, &b);
+        const auto [b, y0, x0] = conv_tile(t, p.tiles_x, p.tiles_y);
         for (int kx = 0; kx < 3; ++kx, ++cnt) {
           const int s = (int)(cnt % kUpAStages);
           mbar_wait(empty_bar(s), ((cnt / kUpAStages) & 1u) ^ 1u);
@@ -307,14 +289,14 @@ conv3_c64_up_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_con
       // ===================== TMA store: box u = (tile, phase) through the phase's strided view of the HR map =====================
       uint32_t u = 0;
       for (int t = blockIdx.x; t < total; t += gridDim.x) {
-        int x0, y0, b; tile_xyb(t, &x0, &y0, &b);
+        const auto [b, y0, x0] = conv_tile(t, p.tiles_x, p.tiles_y);
         for (int ph = 0; ph < 4; ++ph, ++u) {
           const int s = (int)(u % kUpNBox);
           mbar_wait(box_ready(s), (u / kUpNBox) & 1u);
           const CUtensorMap* tm = ph == 0 ? &tmap_o0 : ph == 1 ? &tmap_o1 : ph == 2 ? &tmap_o2 : &tmap_o3;
           tma_store_4d(tm, sb + C::kOffBox + s * kBoxBytes, 0, x0, y0, b);
           tma_commit();
-          tma_wait_read1();                                  // groups retire in order: the previous box is free again
+          tma_wait_read<1>();                                // groups retire in order: the previous box is free again
           if (u >= 1) mbar_arrive(box_free((int)((u - 1) % kUpNBox)));
         }
       }
@@ -410,11 +392,6 @@ conv_last_fold_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_c
   tc_fence_after();
   const uint32_t tmem_base = *tmem_ptr_smem;
 
-  auto tile_xyb = [&](int t, int* x0, int* y0, int* b) {
-    const int tx = t % p.tiles_x; const int t2 = t / p.tiles_x;
-    *x0 = tx * kFoldTW; *y0 = (t2 % p.tiles_y) * kFoldTH; *b = t2 / p.tiles_y;
-  };
-
   if (warp == 0) {
     if (lane == 0) {
       // ===================== producer: folded filters once, then one halo box per tile =====================
@@ -422,7 +399,7 @@ conv_last_fold_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_c
       tma_load_2d(sb, &tmap_b, b_full, 0, 0);
       uint32_t cnt = 0;
       for (int t = blockIdx.x; t < total; t += gridDim.x, ++cnt) {
-        int x0, y0, b; tile_xyb(t, &x0, &y0, &b);
+        const auto [b, y0, x0] = conv_tile(t, p.tiles_x, p.tiles_y, kFoldTH, kFoldTW);
         const int s = (int)(cnt % kFoldStages);
         mbar_wait(empty_bar(s), ((cnt / kFoldStages) & 1u) ^ 1u);
         mbar_expect_tx(full_bar(s), kFoldA);
@@ -484,9 +461,9 @@ conv_last_fold_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_c
         for (int i = 0; i < 4; ++i) dst[4 + i] = make_uint4(r1[4 * i], r1[4 * i + 1], r1[4 * i + 2], r1[4 * i + 3]);
         dst[8] = make_uint4(r2[0], r2[1], r2[2], r2[3]);      // columns 32..35 = tap 8; 36..47 are padding
       }
-      asm volatile("bar.sync 1, 256;" ::: "memory");          // the eight epilogue warps only; P is double-buffered by tile parity
+      named_bar_sync(1, 256);                        // the eight epilogue warps only; P is double-buffered by tile parity
       if (tid < kFoldTW * kFoldTH) {
-        int x0, y0, b; tile_xyb(t, &x0, &y0, &b);
+        const auto [b, y0, x0] = conv_tile(t, p.tiles_x, p.tiles_y, kFoldTH, kFoldTW);
         const int y = y0 + oy, x = x0 + ox;
         float4 acc = make_float4(bias[0], bias[1], bias[2], bias[3]);
 #pragma unroll

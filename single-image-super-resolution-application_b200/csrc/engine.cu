@@ -313,7 +313,6 @@ int dev_alloc(HitsirHandle* h, T** p, size_t count) {
 int pick_bn(int n) {
   if (n <= 16) return 16;
   if (n <= 32) return 32;
-  if (n <= 48) return 48;
   if (n <= 64) return 64;
   if (n % 256 == 0) return 256;
   return 192;
@@ -737,39 +736,23 @@ void base_params(GemmParams& p, const GemmW& w) {
   p.num_kb = w.K / 64;
   p.cblocks = p.num_kb;
   p.bias = w.b;
-  p.Wp = w.w; p.ldw = w.K;
   p.ps = 1;
   p.slope = 1.f;
 }
 
-// The staged-epilogue kernel covers the plain-store and gate epilogues; the pixel-shuffle epilogues (once per forward) keep the
-// direct-store kernel.
-bool tma_epilogue(const GemmW& w, const GemmParams& p) {
-  if (p.epi == EPI_MSGATE) return w.BN == 160;
-  return p.epi == EPI_STORE && (w.BN == 192 || w.BN == 64) && w.Npad <= 384;
-}
-
-int run_gemm(Fwd& f, const char* cat, const GemmW& w, GemmParams& p, const CUtensorMap* maps, bool tma) {
-  LAUNCH(cat, 1, tma ? launch_umma_gemm_tma(w.BN, p, maps, f.h->num_sms, f.st) : launch_umma_gemm(w.BN, p, maps[0], w.tm, f.h->num_sms, f.st));
-  return 0;
-}
-
-// token-major linear: A [M, lda] bf16 (lda == w.K)
+// token-major linear: A [M, w.K] bf16; plain-store or gate epilogue (TMA-staged kernel)
 int linear(Fwd& f, const char* cat, const GemmW& w, const bf16* A, long long M, GemmParams& p) {
   p.conv = 0; p.M = (int)M; p.m_tiles = (int)cdiv64(M, 128);
-  p.A = A; p.lda = w.K;
   p.b_resident = 1;                                        // honoured by the TMA kernel when the weight tile fits next to the A ring
 
   CUtensorMap maps[5];
-  const bool tma = tma_epilogue(w, p);
   if (make_tmap_2d(&maps[0], A, (uint64_t)w.K, (uint64_t)M, (uint64_t)w.K * 2, 64, 128)) return 1;
   maps[1] = w.tm; maps[2] = maps[0]; maps[3] = maps[0]; maps[4] = maps[0];
-  if (tma) {
-    if (p.out_f32 && make_tmap_2d_t(&maps[2], p.out_f32, 4, (uint64_t)p.n_real, (uint64_t)M, (uint64_t)p.ldf * 4, 32, 128)) return 1;
-    if (p.out_bf16 && make_tmap_2d_t(&maps[3], p.out_bf16, 2, (uint64_t)p.ldb, (uint64_t)M, (uint64_t)p.ldb * 2, 64, 128)) return 1;
-    if (p.res && make_tmap_2d_t(&maps[4], p.res, 4, (uint64_t)p.n_real, (uint64_t)M, (uint64_t)p.ldr * 4, 32, 128)) return 1;
-  }
-  return run_gemm(f, cat, w, p, maps, tma);
+  if (p.out_f32 && make_tmap_2d_t(&maps[2], p.out_f32, 4, (uint64_t)p.n_real, (uint64_t)M, (uint64_t)p.ldf * 4, 32, 128)) return 1;
+  if (p.out_bf16 && make_tmap_2d_t(&maps[3], p.out_bf16, 2, (uint64_t)p.ldb, (uint64_t)M, (uint64_t)p.ldb * 2, 64, 128)) return 1;
+  if (p.res && make_tmap_2d_t(&maps[4], p.res, 4, (uint64_t)p.n_real, (uint64_t)M, (uint64_t)p.ldr * 4, 32, 128)) return 1;
+  LAUNCH(cat, 1, launch_umma_gemm_tma(w.BN, p, maps, f.h->num_sms, f.st));
+  return 0;
 }
 
 // Geometry of a 3x3 conv over NHWC bf16 A [B,H,W,Cpad] in 8 x 16-pixel tiles.  Band mode: the rows above / below A are made valid
@@ -780,10 +763,9 @@ int conv_geometry(Fwd& f, const bf16* A, int B, int H, int W, int Cpad, GemmPara
     RUN(fill_halo(f, const_cast<bf16*>(A), (size_t)W * Cpad * sizeof(bf16), H, 1));
     p.a_y_off = 1;
   }
-  p.tiles_x = cdiv(W, 16); p.tiles_y = cdiv(H, 8);
+  p.tiles_x = cdiv(W, kConvTileW); p.tiles_y = cdiv(H, kConvTileH);
   p.m_tiles = B * p.tiles_x * p.tiles_y;
   p.cblocks = Cpad / 64;
-  p.A = A; p.lda = Cpad;
   return 0;
 }
 
@@ -798,15 +780,18 @@ int conv3(Fwd& f, const char* cat, const GemmW& w, const bf16* A, int B, int H, 
     return 0;
   }
   CUtensorMap maps[5];
-  const bool tma = tma_epilogue(w, p);
-  if (make_tmap_nhwc(&maps[0], A - (size_t)p.a_y_off * W * Cpad, B, H + 2 * p.a_y_off, W, Cpad, 64, 16, 8)) return 1;
-  maps[1] = w.tm; maps[2] = maps[0]; maps[3] = maps[0]; maps[4] = maps[0];
-  if (tma) {
-    if (p.out_f32 && make_tmap_nhwc_t(&maps[2], p.out_f32, 4, B, H, W, p.n_real, p.ldf, 32, 16, 8)) return 1;
-    if (p.out_bf16 && make_tmap_nhwc_t(&maps[3], p.out_bf16, 2, B, H, W, p.ldb, p.ldb, 64, 16, 8)) return 1;
-    if (p.res && make_tmap_nhwc_t(&maps[4], p.res, 4, B, H, W, p.n_real, p.ldr, 32, 16, 8)) return 1;
+  if (make_tmap_nhwc(&maps[0], A - (size_t)p.a_y_off * W * Cpad, B, H + 2 * p.a_y_off, W, Cpad, 64, kConvTileW, kConvTileH)) return 1;
+  // the pixel-shuffle heads scatter their outputs from the direct-store kernel; every other epilogue leaves through TMA-staged boxes
+  if (p.epi == EPI_SHUFFLE_NCHW || p.epi == EPI_SHUFFLE_BF16) {
+    LAUNCH(cat, 1, launch_umma_gemm(w.BN, p, maps[0], w.tm, f.h->num_sms, f.st));
+    return 0;
   }
-  return run_gemm(f, cat, w, p, maps, tma);
+  maps[1] = w.tm; maps[2] = maps[0]; maps[3] = maps[0]; maps[4] = maps[0];
+  if (p.out_f32 && make_tmap_nhwc_t(&maps[2], p.out_f32, 4, B, H, W, p.n_real, p.ldf, 32, kConvTileW, kConvTileH)) return 1;
+  if (p.out_bf16 && make_tmap_nhwc_t(&maps[3], p.out_bf16, 2, B, H, W, p.ldb, p.ldb, 64, kConvTileW, kConvTileH)) return 1;
+  if (p.res && make_tmap_nhwc_t(&maps[4], p.res, 4, B, H, W, p.n_real, p.ldr, 32, kConvTileW, kConvTileH)) return 1;
+  LAUNCH(cat, 1, launch_umma_gemm_tma(w.BN, p, maps, f.h->num_sms, f.st));
+  return 0;
 }
 
 // x2 nearest upsampling + 3x3 conv 64 -> 64 (+ LeakyReLU) on the LR map A [B,H,W,64] -> out [B,2H,2W,64] (:1331-1332).  Band mode: the

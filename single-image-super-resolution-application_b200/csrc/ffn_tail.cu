@@ -62,27 +62,13 @@ struct Params {
   // reflect multiplicities of the casa pools are those of the whole frame (row yg0 + y of a frame with Hf rows)
   int h1_y_off, yg0, Hf;
 };
-__device__ __forceinline__ int reflect_mult(int i, int n, int np) { return 1 + ((i >= 2 * (n - 1) - (np - 1) && i <= n - 2) ? 1 : 0); }
 
-__device__ __forceinline__ void tma_store_4d(const void* tmap, uint32_t src, int c0, int c1, int c2, int c3) {
-  asm volatile("cp.async.bulk.tensor.4d.global.shared::cta.bulk_group [%0, {%2, %3, %4, %5}], [%1];" ::"l"(tmap), "r"(src), "r"(c0), "r"(c1),
-               "r"(c2), "r"(c3) : "memory");
-}
-__device__ __forceinline__ void tma_commit() { asm volatile("cp.async.bulk.commit_group;" ::: "memory"); }
-__device__ __forceinline__ void tma_wait_read1() { asm volatile("cp.async.bulk.wait_group.read 1;" ::: "memory"); }
-__device__ __forceinline__ void tma_wait_all0() { asm volatile("cp.async.bulk.wait_group 0;" ::: "memory"); }
-__device__ __forceinline__ void mma_bf16_16816(float* d, uint32_t a0, uint32_t a1, uint32_t a2, uint32_t a3, uint32_t b0, uint32_t b1) {
-  asm volatile("mma.sync.aligned.m16n8k16.row.col.f32.bf16.bf16.f32 {%0,%1,%2,%3}, {%4,%5,%6,%7}, {%8,%9}, {%0,%1,%2,%3};"
-               : "+f"(d[0]), "+f"(d[1]), "+f"(d[2]), "+f"(d[3]) : "r"(a0), "r"(a1), "r"(a2), "r"(a3), "r"(b0), "r"(b1));
-}
 __device__ __forceinline__ void ldmatrix_x4(uint32_t addr, uint32_t& r0, uint32_t& r1, uint32_t& r2, uint32_t& r3) {
   asm volatile("ldmatrix.sync.aligned.m8n8.x4.shared.b16 {%0,%1,%2,%3}, [%4];" : "=r"(r0), "=r"(r1), "=r"(r2), "=r"(r3) : "r"(addr) : "memory");
 }
 __device__ __forceinline__ void ldmatrix_x2(uint32_t addr, uint32_t& r0, uint32_t& r1) {
   asm volatile("ldmatrix.sync.aligned.m8n8.x2.shared.b16 {%0,%1}, [%2];" : "=r"(r0), "=r"(r1) : "r"(addr) : "memory");
 }
-// the four compute warps that share a TMEM lane quarter (= the same 32 pixel rows) exchange their LayerNorm / statistics partials
-__device__ __forceinline__ void epi_bar_sync(int q) { asm volatile("bar.sync %0, 128;" ::"r"(q + 1) : "memory"); }
 
 __global__ void __launch_bounds__(640, 1)
 ffn_tail_kernel(const __grid_constant__ CUtensorMap tm_h1, const __grid_constant__ CUtensorMap tm_x, const Params p) {
@@ -136,17 +122,12 @@ ffn_tail_kernel(const __grid_constant__ CUtensorMap tm_h1, const __grid_constant
   const uint32_t tmem_base = *tmem_ptr_smem;
   pdl_entry();                                           // up to here only weights (fc2 bias, norm2) were read
 
-  auto tile_xyb = [&](int t, int* x0, int* y0, int* b) {
-    const int tx = t % p.tiles_x; const int t2 = t / p.tiles_x;
-    *x0 = tx * 16; *y0 = (t2 % p.tiles_y) * 8; *b = t2 / p.tiles_y;
-  };
-
   if (warp == 0) {
     if (lane == 0) {
       // ===================== producer: per 64-channel slice one h1 halo box and one W2 slice =====================
       int it = 0;
       for (int t = blockIdx.x; t < p.total; t += gridDim.x, ++it) {
-        int x0, y0, b; tile_xyb(t, &x0, &y0, &b);
+        const auto [b, y0, x0] = conv_tile(t, p.tiles_x, p.tiles_y);
         for (int k = 0; k < 6; ++k) {
           const int h = k & 1;
           const uint32_t u = (uint32_t)(it * 3 + (k >> 1));
@@ -192,7 +173,7 @@ ffn_tail_kernel(const __grid_constant__ CUtensorMap tm_h1, const __grid_constant
     if (want_stats) {
       uint32_t u = 0;
       for (int t = blockIdx.x; t < p.total; t += gridDim.x) {
-        int x0, y0, b; tile_xyb(t, &x0, &y0, &b);
+        const auto [b, y0, x0] = conv_tile(t, p.tiles_x, p.tiles_y);
         for (int rr = lane; rr < 128; rr += 32) {
           const int y = y0 + (rr >> 4), x = x0 + (rr & 15);
           s_mult[rr] = (y < p.H && x < p.W) ? (float)(reflect_mult(y + p.yg0, p.Hf, p.Hp) * reflect_mult(x, p.W, p.Wp)) : 0.f;
@@ -234,7 +215,7 @@ ffn_tail_kernel(const __grid_constant__ CUtensorMap tm_h1, const __grid_constant
       // channels straight to global), which used to be a separate pass over the stream (cast_rows_bf16)
       uint32_t u = 0;
       for (int t = blockIdx.x; t < p.total; t += gridDim.x) {
-        int x0, y0, b; tile_xyb(t, &x0, &y0, &b);
+        const auto [b, y0, x0] = conv_tile(t, p.tiles_x, p.tiles_y);
         for (int j = 0; j < 6; ++j, ++u) {
           const int s = (int)(u % kNBox);
           mbar_wait_park(out_bar(s), (u / kNBox) & 1u);
@@ -267,13 +248,13 @@ ffn_tail_kernel(const __grid_constant__ CUtensorMap tm_h1, const __grid_constant
         ++u_store;
       };
       for (int t = blockIdx.x; t < p.total; t += gridDim.x) {
-        int x0, y0, b; tile_xyb(t, &x0, &y0, &b);
+        const auto [b, y0, x0] = conv_tile(t, p.tiles_x, p.tiles_y);
         for (int j = 0; j < 6; ++j) {
           const int s = (int)(u_prep % kNBox);
           if (u_prep >= (uint32_t)kNBox) {
             const uint32_t need = u_prep - (uint32_t)kNBox + 2u;
             while (u_store < need && u_store < u_prep) store_one();
-            tma_wait_read1();                              // bulk groups retire in order: store #(u_prep - kNBox) has left the box
+            tma_wait_read<1>();                            // bulk groups retire in order: store #(u_prep - kNBox) has left the box
             if (want_stats || want_shadow) mbar_wait_park(red_done(s), ((u_prep / kNBox) - 1u) & 1u);   // ... and the statistics warp has read it
           }
           c0s[s] = 32 * j; r0s[s] = x0; r1s[s] = y0; r2s[s] = b;
@@ -298,7 +279,7 @@ ffn_tail_kernel(const __grid_constant__ CUtensorMap tm_h1, const __grid_constant
     // are exchanged through s_part2 and flushed by the hs == 0 thread after the NEXT barrier of the compute warps (no extra barrier)
     auto flush_pixel_stats = [&](int tprev, int itprev) {
       if (hs != 0) return;
-      int x0, y0, b; tile_xyb(tprev, &x0, &y0, &b);
+      const auto [b, y0, x0] = conv_tile(tprev, p.tiles_x, p.tiles_y);
       const int y = y0 + (r >> 4), x = x0 + (r & 15);
       if (y >= p.H || x >= p.W) return;
       const float2* pp = s_part2 + (itprev & 1) * 512;
@@ -351,7 +332,7 @@ ffn_tail_kernel(const __grid_constant__ CUtensorMap tm_h1, const __grid_constant
       }
       float2* part = s_part + (e & 1) * 512;
       part[hs * 128 + r] = make_float2(mean, m2);
-      epi_bar_sync(q);
+      named_bar_sync(q + 1, 128);   // the four compute warps that share TMEM lane quarter q exchange their partials
       if (want_stats && tflush >= 0) flush_pixel_stats(tflush, e - 1);
 #pragma unroll
       for (int o = 1; o < 4; ++o) {
@@ -483,7 +464,7 @@ ffn_tail_kernel(const __grid_constant__ CUtensorMap tm_h1, const __grid_constant
       epi_begin(it - 1, tpp);
       for (int g = 0; g < 3; ++g) epi_group(it - 1, g);
     }
-    if (want_stats && tprev >= 0) { epi_bar_sync(q); flush_pixel_stats(tprev, it - 1); }
+    if (want_stats && tprev >= 0) { named_bar_sync(q + 1, 128); flush_pixel_stats(tprev, it - 1); }
   }
   tc_fence_before();
   __syncthreads();
@@ -504,7 +485,7 @@ int launch_ffn_tail(const bf16* h1, const uint32_t* dw_tbl_mma, const uint8_t* w
   if (ensure_dynamic_smem(ffn_tail_kernel, kSmemBytes, &configured)) return 1;
   Params p;
   p.B = B; p.H = H; p.W = W;
-  p.tiles_x = (W + 15) / 16; p.tiles_y = (H + 7) / 8;
+  p.tiles_x = cdiv(W, kConvTileW); p.tiles_y = cdiv(H, kConvTileH);
   const long long total = (long long)B * p.tiles_x * p.tiles_y;
   if (total > 2147483647LL / 8) { set_error("launch_ffn_tail: too many tiles"); return 1; }
   p.total = (int)total;

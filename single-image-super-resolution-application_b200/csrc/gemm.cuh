@@ -1,5 +1,6 @@
 // Dense-contraction front end of the tcgen05 kernels (umma_gemm.cu, umma_gemm_tma.cu, conv3_c64.cu): problem description + the
-// fused epilogue of the direct-store kernel.
+// pixel-shuffle epilogue of the direct-store kernel.  Each epilogue kind has one GEMM kernel: EPI_STORE and EPI_MSGATE run on the
+// TMA-staged kernel (umma_gemm_tma.cu), the pixel-shuffle heads EPI_SHUFFLE_* on the direct-store kernel (umma_gemm.cu).
 //
 // One "problem" is  D[M, N] = A[M, K] * Wp[N, K]^T  with bf16 operands and fp32 accumulation:
 //   * linear:  A is a token-major activation [M, K] (K padded to a multiple of 64);
@@ -17,7 +18,7 @@ enum EpiMode : int {
   EPI_SHUFFLE_NCHW = 3,  // pixel-shuffle(ps) + de-normalise -> NCHW fp32 image
   EPI_SHUFFLE_BF16 = 4,  // pixel-shuffle(ps) -> NHWC bf16 feature map with `shuf_c` channels
 };
-enum ActMode : int { ACT_NONE = 0, ACT_GELU = 1, ACT_LRELU = 2 };
+enum ActMode : int { ACT_NONE = 0, ACT_LRELU = 2 };
 
 struct GemmParams {
   // problem
@@ -44,40 +45,41 @@ struct GemmParams {
   float out_scale;   // 1 / img_range
   float mean[4];     // per-channel mean added after scaling (NCHW)
   const float* res_img;   // EPI_SHUFFLE_NCHW, ps == 1: NCHW fp32 image added INSTEAD of the mean (upsampler=None: x + conv_last(res), :1340-1342)
-  // operand views for debugging (no kernel reads them: the kernels take tensor maps)
-  const bf16* A; int lda;         // linear: [M, lda]; conv: NHWC base with lda = Cin_pad
-  const bf16* Wp; int ldw;        // [n_tiles*BN, ldw]
 };
+
+// Conv M tiles: 8 x 16 pixels = 128 GEMM rows, row r <-> pixel (y0 + r / 16, x0 + r % 16); tile t runs x fastest, then y, then the
+// image.  conv_last_fold (conv3_c64.cu) walks its own tile shape with the same order.
+constexpr int kConvTileH = 8, kConvTileW = 16;
+struct ConvTile { int b, y0, x0; };
+__host__ __device__ __forceinline__ ConvTile conv_tile(int t, int tiles_x, int tiles_y, int th = kConvTileH, int tw = kConvTileW) {
+  const int tx = t % tiles_x, t2 = t / tiles_x;
+  ConvTile c;
+  c.x0 = tx * tw; c.y0 = (t2 % tiles_y) * th; c.b = t2 / tiles_y;
+  return c;
+}
 
 // Row bookkeeping of the direct-store kernel
 struct RowInfo {
   bool valid;
-  long long grow;   // linear row / NHWC pixel index
   int b, y, x;      // conv coordinates (pixel)
 };
 
 __device__ __forceinline__ RowInfo row_info(const GemmParams& p, int m_tile, int r) {
   RowInfo ri;
   if (!p.conv) {
-    long long g = (long long)m_tile * 128 + r;
-    ri.valid = g < p.M;
-    ri.grow = g;
+    ri.valid = (long long)m_tile * 128 + r < p.M;
     ri.b = ri.y = ri.x = 0;
   } else {
-    int tx = m_tile % p.tiles_x;
-    int t2 = m_tile / p.tiles_x;
-    int ty = t2 % p.tiles_y;
-    int b = t2 / p.tiles_y;
-    int y = ty * 8 + (r >> 4), x = tx * 16 + (r & 15);
+    const ConvTile t = conv_tile(m_tile, p.tiles_x, p.tiles_y);
+    const int b = t.b, y = t.y0 + (r >> 4), x = t.x0 + (r & 15);
     ri.valid = (y < p.H) && (x < p.W);
     ri.b = b; ri.y = y; ri.x = x;
-    ri.grow = ((long long)b * p.H + y) * p.W + x;
   }
   return ri;
 }
 
 // ---------------------------------------------------------------------------
-// Fused epilogue for ONE output row (one thread).  `Acc::load16(col0, v)` returns the 16 raw
+// Pixel-shuffle epilogue for ONE output row (one thread).  `Acc::load16(col0, v)` returns the 16 raw
 // accumulators of columns [col0, col0+16) of this row for the current N tile.
 // All threads of a warp must call it together (TMEM loads are warp-collective), invalid rows
 // simply skip their global stores.
@@ -85,105 +87,26 @@ __device__ __forceinline__ RowInfo row_info(const GemmParams& p, int m_tile, int
 template <int BN, class Acc>
 __device__ __forceinline__ void epilogue_row(const GemmParams& p, Acc& acc, const RowInfo& ri, int n_tile) {
   const int n0 = n_tile * BN;
-  if (p.epi == EPI_STORE) {
+  // column co = c*ps*ps + i*ps + j  -> pixel (ps*y+i, ps*x+j), channel c
+  const int ps = p.ps, pss = ps * ps;
+  const int oh = p.H * ps, ow = p.W * ps;
 #pragma unroll 1
-    for (int c0 = 0; c0 < BN; c0 += 16) {
-      float v[16];
-      acc.load16(c0, v);
-      if (!ri.valid) continue;
-      const int gc = n0 + c0;
+  for (int c0 = 0; c0 < BN; c0 += 16) {
+    float v[16];
+    acc.load16(c0, v);
+    if (!ri.valid) continue;
 #pragma unroll
-      for (int i = 0; i < 16; ++i) {
-        float t = v[i] + __ldg(p.bias + gc + i);
-        if (p.act == ACT_GELU) t = gelu_erf(t);
-        else if (p.act == ACT_LRELU) t = lrelu(t, p.slope);
-        v[i] = t;
-      }
-      if (p.res != nullptr) {
-        const float* rr = p.res + ri.grow * p.ldr + gc;
-#pragma unroll
-        for (int i = 0; i < 16; ++i)
-          if (gc + i < p.n_real) v[i] += __ldg(rr + i);
-      }
-      if (p.out_f32 != nullptr) {
-        float* o = p.out_f32 + ri.grow * p.ldf + gc;
-        if (gc + 16 <= p.n_real && (p.ldf & 3) == 0) {
-#pragma unroll
-          for (int i = 0; i < 16; i += 4) *reinterpret_cast<float4*>(o + i) = make_float4(v[i], v[i + 1], v[i + 2], v[i + 3]);
-        } else {
-#pragma unroll
-          for (int i = 0; i < 16; ++i)
-            if (gc + i < p.n_real) o[i] = v[i];
-        }
-      }
-      if (p.out_bf16 != nullptr && gc < p.ldb) {
-        uint32_t w[8];
-#pragma unroll
-        for (int i = 0; i < 8; ++i) {
-          float a = (gc + 2 * i < p.n_real) ? v[2 * i] : 0.f;
-          float b = (gc + 2 * i + 1 < p.n_real) ? v[2 * i + 1] : 0.f;
-          w[i] = pack_bf16x2(a, b);
-        }
-        uint4* o = reinterpret_cast<uint4*>(p.out_bf16 + ri.grow * p.ldb + gc);
-        o[0] = make_uint4(w[0], w[1], w[2], w[3]);
-        o[1] = make_uint4(w[4], w[5], w[6], w[7]);
-      }
-    }
-  } else if (p.epi == EPI_MSGATE) {
-    // N tile `n_tile` (BN == 160) holds, for the 32 embedding channels c = 32*n_tile + i:
-    //   cols [32k, 32k+32), k=0..3 : conv3/5/7/9 outputs, cols [128,160): conv_x (1x1) output.
-    // g_k = x_k * sigmoid(x_1 * x_k) + x_k  (hit_sir_pro.py:83-92) -> out_bf16[row, 128*n_tile + 32*k + i]
-    // (the [tile][slot][channel] order the packed conv_first.conv_last expects, pack.cu pack_mslast_kernel).
-    float x1[32];
-    {
-      float v[16];
-#pragma unroll
-      for (int c0 = 128; c0 < 160; c0 += 16) {
-        acc.load16(c0, v);
-#pragma unroll
-        for (int i = 0; i < 16; ++i) x1[c0 + i - 128] = v[i] + __ldg(p.bias + n0 + c0 + i);
-      }
-    }
-#pragma unroll
-    for (int c0 = 0; c0 < 128; c0 += 16) {
-      float v[16];
-      acc.load16(c0, v);
-      if (ri.valid) {
-        uint32_t w[8];
-#pragma unroll
-        for (int i = 0; i < 16; i += 2) {
-          const float xa = v[i] + __ldg(p.bias + n0 + c0 + i), xb = v[i + 1] + __ldg(p.bias + n0 + c0 + i + 1);
-          const float ga = xa * sigmoidf_(x1[(c0 + i) & 31] * xa) + xa, gb = xb * sigmoidf_(x1[(c0 + i + 1) & 31] * xb) + xb;
-          w[i >> 1] = pack_bf16x2(ga, gb);
-        }
-        uint4* o = reinterpret_cast<uint4*>(p.out_bf16 + ri.grow * p.ldb + 128 * n_tile + c0);
-        o[0] = make_uint4(w[0], w[1], w[2], w[3]);
-        o[1] = make_uint4(w[4], w[5], w[6], w[7]);
-      }
-    }
-  } else {
-    // pixel-shuffle epilogues: column co = c*ps*ps + i*ps + j  -> pixel (ps*y+i, ps*x+j), channel c
-    const int ps = p.ps, pss = ps * ps;
-    const int oh = p.H * ps, ow = p.W * ps;
-#pragma unroll 1
-    for (int c0 = 0; c0 < BN; c0 += 16) {
-      float v[16];
-      acc.load16(c0, v);
-      if (!ri.valid) continue;
-#pragma unroll
-      for (int i = 0; i < 16; ++i) {
-        const int co = n0 + c0 + i;
-        if (co >= p.n_real) continue;
-        const int c = co / pss, rem = co - c * pss;
-        const int oy = ri.y * ps + rem / ps, ox = ri.x * ps + rem % ps;
-        float t = v[i] + __ldg(p.bias + co);
-        if (p.epi == EPI_SHUFFLE_NCHW) {
-          const long long oi = (((long long)ri.b * p.shuf_c + c) * oh + oy) * ow + ox;
-          p.out_f32[oi] = t * p.out_scale + (p.res_img != nullptr ? __ldg(p.res_img + oi) : p.mean[c & 3]);
-        } else {
-          if (p.act == ACT_LRELU) t = lrelu(t, p.slope);
-          p.out_bf16[(((long long)ri.b * oh + oy) * ow + ox) * p.ldb + c] = __float2bfloat16(t);
-        }
+    for (int i = 0; i < 16; ++i) {
+      const int co = n0 + c0 + i;
+      if (co >= p.n_real) continue;
+      const int c = co / pss, rem = co - c * pss;
+      const int oy = ri.y * ps + rem / ps, ox = ri.x * ps + rem % ps;
+      const float t = v[i] + __ldg(p.bias + co);
+      if (p.epi == EPI_SHUFFLE_NCHW) {
+        const long long oi = (((long long)ri.b * p.shuf_c + c) * oh + oy) * ow + ox;
+        p.out_f32[oi] = t * p.out_scale + (p.res_img != nullptr ? __ldg(p.res_img + oi) : p.mean[c & 3]);
+      } else {
+        p.out_bf16[(((long long)ri.b * oh + oy) * ow + ox) * p.ldb + c] = __float2bfloat16(t);
       }
     }
   }

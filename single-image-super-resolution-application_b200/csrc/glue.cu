@@ -10,10 +10,6 @@ namespace hitsir {
 
 namespace {
 
-__device__ __forceinline__ int reflect_src(int i, int n) { return i < n ? i : 2 * (n - 1) - i; }   // F.pad 'reflect' (:672)
-// number of positions of the padded axis [0, np) that read source index i: padded ip in [n, np) mirrors to 2(n-1) - ip
-__device__ __forceinline__ int reflect_mult(int i, int n, int np) { return 1 + ((i >= 2 * (n - 1) - (np - 1) && i <= n - 2) ? 1 : 0); }
-
 // ---------------------------------------------------------------------------------------------
 // Entry: mean shift (:1310-1311) + im2col of the f x f footprint.  CTA = (image, row, run of 64 pixels): the f rows x (64 + f - 1)
 // columns x in_ch window is staged once in shared memory as bf16((x - mean) * img_range) (zero outside the image = the conv's zero
@@ -322,10 +318,6 @@ __device__ __forceinline__ void split_bf16(float v, uint16_t* hi, uint16_t* lo) 
   const bf16 l = __float2bfloat16_rn(v - __bfloat162float(h));
   *hi = *reinterpret_cast<const uint16_t*>(&h); *lo = *reinterpret_cast<const uint16_t*>(&l);
 }
-__device__ __forceinline__ void mma_bf16_16816(float* d, const uint32_t* a, uint32_t b0, uint32_t b1) {
-  asm volatile("mma.sync.aligned.m16n8k16.row.col.f32.bf16.bf16.f32 {%0,%1,%2,%3}, {%4,%5,%6,%7}, {%8,%9}, {%0,%1,%2,%3};"
-               : "+f"(d[0]), "+f"(d[1]), "+f"(d[2]), "+f"(d[3]) : "r"(a[0]), "r"(a[1]), "r"(a[2]), "r"(a[3]), "r"(b0), "r"(b1));
-}
 // B fragments of both 3x3 filters in the k order above: img[n-tile 24][conv 2][k-step 2][reg 2][lane 32]
 __global__ void casa_bfrag_kernel(CasaW w, uint32_t* __restrict__ img) {
   const int idx = blockIdx.x * blockDim.x + threadIdx.x;
@@ -452,13 +444,14 @@ __global__ void __launch_bounds__(128, kQkvMinCtas) qkv_casa_mma_kernel(const fl
           const uint32_t* a0 = as + (v * kMmaRun + r0) * kMmaAS + s * 8 + tq;
           af[v][s][0] = a0[0]; af[v][s][1] = a0[8 * kMmaAS]; af[v][s][2] = a0[4]; af[v][s][3] = a0[8 * kMmaAS + 4];
         }
+      auto mma = [](float* d, const uint32_t* a, uint32_t b0, uint32_t b1) { mma_bf16_16816(d, a[0], a[1], a[2], a[3], b0, b1); };
 #pragma unroll
       for (int j = 0; j < 6; ++j) {
         float d1[4] = {0.f, 0.f, 0.f, 0.f}, d2[4] = {0.f, 0.f, 0.f, 0.f};
-        mma_bf16_16816(d1, af[0][0], bf[j][0][0][0], bf[j][0][0][1]);
-        mma_bf16_16816(d1, af[0][1], bf[j][0][1][0], bf[j][0][1][1]);
-        mma_bf16_16816(d2, af[1][0], bf[j][1][0][0], bf[j][1][0][1]);
-        mma_bf16_16816(d2, af[1][1], bf[j][1][1][0], bf[j][1][1][1]);
+        mma(d1, af[0][0], bf[j][0][0][0], bf[j][0][0][1]);
+        mma(d1, af[0][1], bf[j][0][1][0], bf[j][0][1][1]);
+        mma(d2, af[1][0], bf[j][1][0][0], bf[j][1][0][1]);
+        mma(d2, af[1][1], bf[j][1][1][0], bf[j][1][1][1]);
         const int pos0 = (warp * 6 + j) * 8 + tq * 2;
         const bool pad = ((pos0 + 1) & 15) == 15;
         const float padv = pos0 < 96 ? 1.0f : 0.f;        // q pads carry the constant 1 (k-gen bias rider), v pads 0
@@ -484,11 +477,11 @@ __global__ void __launch_bounds__(128, kQkvMinCtas) qkv_casa_mma_kernel(const fl
       const uint32_t os_addr = (uint32_t)__cvta_generic_to_shared(os);
       for (int px = 0; px < n; ++px)
         asm volatile("cp.async.bulk.global.shared::cta.bulk_group [%0], [%1], %2;" ::"l"(trow + (long long)px * kCp), "r"(os_addr + (uint32_t)(px * kMmaOS * 4)), "r"(kCp * 2) : "memory");
-      asm volatile("cp.async.bulk.commit_group;" ::: "memory");
-      asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");    // the tile may be rewritten after the next barrier
+      tma_commit();
+      tma_wait_read<0>();                                  // the tile may be rewritten after the next barrier
     }
   }
-  if (tid == 32) asm volatile("cp.async.bulk.wait_group 0;" ::: "memory");     // writes complete before the CTA exits
+  if (tid == 32) tma_wait_all0();                          // writes complete before the CTA exits
 }
 
 // ---------------------------------------------------------------------------------------------

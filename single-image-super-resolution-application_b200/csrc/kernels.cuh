@@ -1,6 +1,6 @@
 // Launch prototypes of the non-GEMM kernels (glue.cu, scc.cu, pack.cu).
 #pragma once
-#include "common.cuh"
+#include "gemm.cuh"
 
 namespace hitsir {
 
@@ -25,7 +25,7 @@ int launch_ln_rows(const float* x, const float* gamma, const float* beta, bf16* 
 // Optional by-product of ffn_tail: the casa statistics of the block output for the NEXT block (padded to Hp x Wp there):
 // cavg/cmax [B*H*W], part_sum/part_max [B * tiles][180] with tiles = ceil(H/8) * ceil(W/16) 8x16-pixel tiles per image
 struct FfnStats { float* cavg; float* cmax; float* part_sum; float* part_max; int Hp, Wp; };
-inline int ffn_tiles_per_image(int H, int W) { return ((H + 7) / 8) * ((W + 15) / 16); }
+inline int ffn_tiles_per_image(int H, int W) { return cdiv(H, kConvTileH) * cdiv(W, kConvTileW); }
 // dw_tbl_mma (launch_pack_dw_mma from the fp32 [26][384] tap-major table): the depthwise taps as B-fragment words of the tensor-core
 // conv, [384 channels][28 words]: bf16(w) in the low (c even) / high (c odd) half in MMA pairing order, word 26 = fp32 bias bits (pack.cu)
 int launch_pack_dw_mma(const float* dw_tbl, uint32_t* out, cudaStream_t st);
@@ -85,6 +85,11 @@ struct PadGeom {
   // Hpf; `top` / `bot` say that the per-pixel statistic maps carry one valid halo row of the neighbour band above / below
   int y0, Hf, Hpf, top, bot;
 };
+// F.pad 'reflect' (hit_sir_pro.py:672): source index of padded index i in [0, 2n - 1)
+__device__ __forceinline__ int reflect_src(int i, int n) { return i < n ? i : 2 * (n - 1) - i; }
+// number of positions of the padded axis [0, np) that read source index i: padded ip in [n, np) mirrors to 2(n-1) - ip.  The casa pool
+// statistics of sca_stats (glue.cu) and of the ffn_tail by-product both weight pixels by it, so both kernels give the same pools.
+__device__ __forceinline__ int reflect_mult(int i, int n, int np) { return 1 + ((i >= 2 * (n - 1) - (np - 1) && i <= n - 2) ? 1 : 0); }
 // per padded pixel channel mean / max + deterministic per-image per-channel (sum, max) partials
 int launch_sca_stats(const float* x, PadGeom g, float* cavg, float* cmax, float* part_sum, float* part_max, int nparts, cudaStream_t st);
 int launch_sca_mlp(const float* part_sum, const float* part_max, int nparts, PadGeom g, CasaW w, float* s1, float* s2, cudaStream_t st);

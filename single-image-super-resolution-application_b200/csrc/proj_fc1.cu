@@ -35,13 +35,6 @@ constexpr int kNumBars = 13 + 2 * kNBox;
 constexpr int kSmemBytes = kOffBar + kNumBars * 8 + 8 + 1024;
 static_assert(kSmemBytes <= 232448, "smem budget");
 
-__device__ __forceinline__ void tma_store_2d(const void* tmap, uint32_t src, int c0, int c1) {
-  asm volatile("cp.async.bulk.tensor.2d.global.shared::cta.bulk_group [%0, {%2, %3}], [%1];" ::"l"(tmap), "r"(src), "r"(c0), "r"(c1) : "memory");
-}
-__device__ __forceinline__ void tma_commit() { asm volatile("cp.async.bulk.commit_group;" ::: "memory"); }
-__device__ __forceinline__ void tma_wait_read1() { asm volatile("cp.async.bulk.wait_group.read 1;" ::: "memory"); }   // all but the newest group
-__device__ __forceinline__ void tma_wait_all0() { asm volatile("cp.async.bulk.wait_group 0;" ::: "memory"); }
-__device__ __forceinline__ void epi_bar_sync() { asm volatile("bar.sync 1, %0;" ::"n"(32 * kEpiWarps) : "memory"); }   // the epilogue threads only
 
 }  // namespace
 
@@ -181,7 +174,7 @@ proj_fc1_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constant_
             // #(u_prep - kNBox + 1) are issued, "at most one group pending" proves that store has finished reading shared memory.
             const uint32_t need = u_prep - (uint32_t)kNBox + 2u;
             while (u_store < need && u_store < u_prep) store_one();
-            tma_wait_read1();
+            tma_wait_read<1>();
           }
           if (is_f32(u_prep)) {
             mbar_expect_tx(in_bar(b), kBox);
@@ -253,7 +246,7 @@ proj_fc1_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constant_
           }
           part[hs * 128 + r] = make_float2(mean, m2);
         }
-        epi_bar_sync();
+        named_bar_sync(1, 32 * kEpiWarps);   // the epilogue threads only
         const int h0 = hs >> 1, ho = h0 ^ 1;   // column half of this warp's slices, and the other half
         const float2 own = part[h0 * 128 + r];
         float n = (float)slice_count(h0), mean = own.x, m2 = own.y;

@@ -46,65 +46,6 @@ struct Params {
   int H, W;
 };
 
-__host__ __device__ constexpr uint32_t make_idesc(int m, int n, int a_mn, int b_mn) {
-  return (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)a_mn << 15) | ((uint32_t)b_mn << 16) | ((uint32_t)(n >> 3) << 17) |
-         ((uint32_t)(m >> 4) << 24);
-}
-__device__ __forceinline__ uint64_t make_desc(uint32_t saddr, uint32_t lbo_bytes, uint32_t sbo_bytes) {
-  uint64_t d = 0;
-  d |= (uint64_t)((saddr & 0x3FFFFu) >> 4);
-  d |= (uint64_t)(lbo_bytes >> 4) << 16;
-  d |= (uint64_t)(sbo_bytes >> 4) << 32;
-  d |= (uint64_t)1 << 46;
-  d |= (uint64_t)2 << 61;
-  return d;
-}
-__device__ __forceinline__ uint64_t kdesc(uint32_t saddr) { return make_desc(saddr, 16, 1024); }
-__device__ __forceinline__ void tma_store_4d(const void* tmap, uint32_t src, int c0, int c1, int c2, int c3) {
-  asm volatile("cp.async.bulk.tensor.4d.global.shared::cta.bulk_group [%0, {%2, %3, %4, %5}], [%1];" ::"l"(tmap), "r"(src), "r"(c0), "r"(c1),
-               "r"(c2), "r"(c3) : "memory");
-}
-__device__ __forceinline__ void tma_commit() { asm volatile("cp.async.bulk.commit_group;" ::: "memory"); }
-__device__ __forceinline__ void tma_wait_read0() { asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory"); }
-__device__ __forceinline__ void tma_wait_all0() { asm volatile("cp.async.bulk.wait_group 0;" ::: "memory"); }
-
-__device__ __forceinline__ void wait_bar(uint32_t bar, uint32_t parity) {
-  uint32_t done = 0;
-  long long spins = 0;
-  while (true) {
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t"
-        "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"
-        "selp.u32 %0, 1, 0, p;\n\t}"
-        : "=r"(done) : "r"(bar), "r"(parity) : "memory");
-    if (done) break;
-    if (++spins > (1LL << 26)) {
-      printf("scc_dense: barrier timeout (block %d thread %d bar %u parity %u)\n", blockIdx.x, threadIdx.x, (bar >> 3) & 31u, parity);
-      __trap();
-    }
-  }
-}
-__device__ __forceinline__ uint8_t* swz(uint8_t* block, int row, int chunk) { return block + row * 128 + ((chunk ^ (row & 7)) << 4); }
-__device__ __forceinline__ void store16(uint8_t* block, int row, int chunk0, const float* v) {
-  *reinterpret_cast<uint4*>(swz(block, row, chunk0)) =
-      make_uint4(pack_bf16x2(v[0], v[1]), pack_bf16x2(v[2], v[3]), pack_bf16x2(v[4], v[5]), pack_bf16x2(v[6], v[7]));
-  *reinterpret_cast<uint4*>(swz(block, row, chunk0 + 1)) =
-      make_uint4(pack_bf16x2(v[8], v[9]), pack_bf16x2(v[10], v[11]), pack_bf16x2(v[12], v[13]), pack_bf16x2(v[14], v[15]));
-}
-template <int NG>
-__device__ __forceinline__ void tmem_ld_cols(uint32_t taddr, float (&v)[NG][16]) {
-  uint32_t r[NG][16];
-#pragma unroll
-  for (int i = 0; i < NG; ++i) tmem_ld16_nw(taddr + 16 * i, r[i]);
-  tmem_ld_wait();
-#pragma unroll
-  for (int i = 0; i < NG; ++i) {
-    reg_fence16(r[i]);
-#pragma unroll
-    for (int e = 0; e < 16; ++e) v[i][e] = __uint_as_float(r[i][e]);
-  }
-}
-
 // LT = tokens per window (16 or 64)
 template <int LT>
 __global__ void __launch_bounds__(384, 1)
@@ -171,8 +112,7 @@ scc_dense_kernel(const __grid_constant__ CUtensorMap tm_t, const __grid_constant
       };
       if (LT == 16) {          // all six 2 KB bias images fit the slot area: load them once
         mbar_expect_tx(b_full(0), (uint32_t)(kHeads * p.bias_bytes));
-        asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(sb + kOffBias), "l"(p.bias_img),
-                     "r"((uint32_t)(kHeads * p.bias_bytes)), "r"(b_full(0)) : "memory");
+        bulk_load(sb + kOffBias, p.bias_img, (uint32_t)(kHeads * p.bias_bytes), b_full(0));
       }
       if ((int)blockIdx.x < p.ntiles) load_tile(blockIdx.x, 0);
       for (int tile = blockIdx.x; tile < p.ntiles; tile += gridDim.x, ++cnt) {
@@ -182,8 +122,7 @@ scc_dense_kernel(const __grid_constant__ CUtensorMap tm_t, const __grid_constant
           const int slot = k & 1;
           wait_bar(b_empty(slot), (ub[slot] & 1u) ^ 1u);
           mbar_expect_tx(b_full(slot), (uint32_t)p.bias_bytes);
-          asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(sb + kOffBias + slot * 8192),
-                       "l"(p.bias_img + (size_t)(k - 1) * p.bias_bytes), "r"((uint32_t)p.bias_bytes), "r"(b_full(slot)) : "memory");
+          bulk_load(sb + kOffBias + slot * 8192, p.bias_img + (size_t)(k - 1) * p.bias_bytes, (uint32_t)p.bias_bytes, b_full(slot));
           ++ub[slot];
         }
       }
@@ -196,7 +135,7 @@ scc_dense_kernel(const __grid_constant__ CUtensorMap tm_t, const __grid_constant
       constexpr uint32_t id_oc = make_idesc(128, 96, 0, 1);      // out_c = P_c Q   (B = token tile, MN-major)
       constexpr uint32_t id_os = make_idesc(128, 16, 0, 1);      // out_s_h = P_h V_h
       const uint32_t kb = sb + kOffK, wb = sb + kOffW;
-      const uint64_t w1d = kdesc(wb), w2d = kdesc(wb + 32);
+      const uint64_t w1d = umma_desc_sw128(wb), w2d = umma_desc_sw128(wb + 32);
       uint32_t cnt = 0, us[2] = {0, 0}, up[2] = {0, 0};
       for (int tile = blockIdx.x; tile < p.ntiles; tile += gridDim.x, ++cnt) {
         const int s = (int)(cnt & 1u);
@@ -206,11 +145,11 @@ scc_dense_kernel(const __grid_constant__ CUtensorMap tm_t, const __grid_constant
         tc_fence_after();
         // ---- k-gen: K[:, 16h..] = Q_h W1^T (+ bias via the ones column) + V_h W2^T
 #pragma unroll
-        for (int h = 0; h < kHeads; ++h) umma_bf16(tmem + kTmS + 16 * h, kdesc(st + (h >> 2) * kBlk + (h & 3) * 32), w1d, id_k16, 0u);
+        for (int h = 0; h < kHeads; ++h) umma_bf16(tmem + kTmS + 16 * h, umma_desc_sw128(st + (h >> 2) * kBlk + (h & 3) * 32), w1d, id_k16, 0u);
 #pragma unroll
         for (int h = 0; h < kHeads; ++h) {
           const int cv = 96 + 16 * h;
-          umma_bf16(tmem + kTmS + 16 * h, kdesc(st + (cv >> 6) * kBlk + (cv & 63) * 2), w2d, id_k16, 1u);
+          umma_bf16(tmem + kTmS + 16 * h, umma_desc_sw128(st + (cv >> 6) * kBlk + (cv & 63) * 2), w2d, id_k16, 1u);
         }
         umma_commit(kt_full);
         wait_bar(k_ready, cnt & 1u);
@@ -224,13 +163,13 @@ scc_dense_kernel(const __grid_constant__ CUtensorMap tm_t, const __grid_constant
           if (j == 0) {
 #pragma unroll
             for (int ks = 0; ks < 8; ++ks)
-              umma_bf16(tmem + kTmD + 96, kdesc(pb + (ks >> 2) * kBlk + (ks & 3) * 32), make_desc(st + ks * 2048, kBlk, 1024), id_oc, ks ? 1u : 0u);
+              umma_bf16(tmem + kTmD + 96, umma_desc_sw128(pb + (ks >> 2) * kBlk + (ks & 3) * 32), make_desc(st + ks * 2048, kBlk, 1024), id_oc, ks ? 1u : 0u);
           } else {
             const int h = j - 1, cv = 96 + 16 * h;
             const uint32_t vb = st + (cv >> 6) * kBlk + (cv & 63) * 2;
 #pragma unroll
             for (int ks = 0; ks < 8; ++ks)
-              umma_bf16(tmem + kTmD + 16 * h, kdesc(pb + (ks >> 2) * kBlk + (ks & 3) * 32), make_desc(vb + ks * 2048, kBlk, 1024), id_os, ks ? 1u : 0u);
+              umma_bf16(tmem + kTmD + 16 * h, umma_desc_sw128(pb + (ks >> 2) * kBlk + (ks & 3) * 32), make_desc(vb + ks * 2048, kBlk, 1024), id_os, ks ? 1u : 0u);
           }
           umma_commit(p_empty(buf));
           ++up[buf];
@@ -244,11 +183,11 @@ scc_dense_kernel(const __grid_constant__ CUtensorMap tm_t, const __grid_constant
 #pragma unroll
             for (int ks = 0; ks < 6; ++ks) {             // St[l][l'] = sum_c v_l[c] k_l'[c]
               const int cv = 96 + 16 * ks;
-              umma_bf16(S, kdesc(st + (cv >> 6) * kBlk + (cv & 63) * 2), kdesc(kb + (ks >> 2) * kBlk + (ks & 3) * 32), id_s, ks ? 1u : 0u);
+              umma_bf16(S, umma_desc_sw128(st + (cv >> 6) * kBlk + (cv & 63) * 2), umma_desc_sw128(kb + (ks >> 2) * kBlk + (ks & 3) * 32), id_s, ks ? 1u : 0u);
             }
           } else {
             const int h = k - 1;                         // S_h[l][m] = q_lh . k_mh
-            umma_bf16(S, kdesc(st + (h >> 2) * kBlk + (h & 3) * 32), kdesc(kb + (h >> 2) * kBlk + (h & 3) * 32), id_s, 0u);
+            umma_bf16(S, umma_desc_sw128(st + (h >> 2) * kBlk + (h & 3) * 32), umma_desc_sw128(kb + (h >> 2) * kBlk + (h & 3) * 32), id_s, 0u);
           }
           umma_commit(s_full(buf));
           ++us[buf];
@@ -277,7 +216,7 @@ scc_dense_kernel(const __grid_constant__ CUtensorMap tm_t, const __grid_constant
             any = true;
           }
         }
-        if (any) { tma_commit(); tma_wait_read0(); }
+        if (any) { tma_commit(); tma_wait_read<0>(); }
         mbar_arrive(tok_empty(s));
       }
       tma_wait_all0();

@@ -71,78 +71,6 @@ struct Params {
   float* dbg;                // optional dump of window 0 (see hitsir_scc_debug layout in engine.cu)
 };
 
-__host__ __device__ constexpr uint32_t make_idesc(int m, int n, int a_mn, int b_mn) {
-  return (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)a_mn << 15) | ((uint32_t)b_mn << 16) | ((uint32_t)(n >> 3) << 17) |
-         ((uint32_t)(m >> 4) << 24);
-}
-// SWIZZLE_128B operand descriptor.  K-major: lbo ignored, sbo = 1024 (8 rows).  MN-major: lbo = stride between
-// 64-element blocks along M/N, sbo = stride between 8-row groups along K (cute/atom/mma_traits_sm100.hpp canonical forms).
-__device__ __forceinline__ uint64_t make_desc(uint32_t saddr, uint32_t lbo_bytes, uint32_t sbo_bytes) {
-  uint64_t d = 0;
-  d |= (uint64_t)((saddr & 0x3FFFFu) >> 4);
-  d |= (uint64_t)(lbo_bytes >> 4) << 16;
-  d |= (uint64_t)(sbo_bytes >> 4) << 32;
-  d |= (uint64_t)1 << 46;
-  d |= (uint64_t)2 << 61;
-  return d;
-}
-__device__ __forceinline__ uint64_t kdesc(uint32_t saddr) { return make_desc(saddr, 16, 1024); }
-
-__device__ __forceinline__ void bulk_load(uint32_t dst, const void* src, uint32_t bytes, uint32_t bar) {
-  asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(dst), "l"(src), "r"(bytes), "r"(bar)
-               : "memory");
-}
-__device__ __forceinline__ void tma_store_4d(const void* tmap, uint32_t src, int c0, int c1, int c2, int c3) {
-  asm volatile("cp.async.bulk.tensor.4d.global.shared::cta.bulk_group [%0, {%2, %3, %4, %5}], [%1];" ::"l"(tmap), "r"(src), "r"(c0), "r"(c1),
-               "r"(c2), "r"(c3) : "memory");
-}
-__device__ __forceinline__ void tma_commit() { asm volatile("cp.async.bulk.commit_group;" ::: "memory"); }
-__device__ __forceinline__ void tma_wait_read0() { asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory"); }
-__device__ __forceinline__ void tma_wait_all0() { asm volatile("cp.async.bulk.wait_group 0;" ::: "memory"); }
-
-// mbarrier wait with a watchdog: a protocol bug traps (-> launch error) instead of hanging the device
-__device__ __forceinline__ void wait_bar(uint32_t bar, uint32_t parity) {
-  uint32_t done = 0;
-  long long spins = 0;
-  while (true) {
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t"
-        "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"
-        "selp.u32 %0, 1, 0, p;\n\t}"
-        : "=r"(done) : "r"(bar), "r"(parity) : "memory");
-    if (done) break;
-    if (++spins > (1LL << 26)) {
-      printf("scc_umma: barrier timeout (block %d thread %d bar %u parity %u)\n", blockIdx.x, threadIdx.x, (bar >> 3) & 31u, parity);
-      __trap();
-    }
-  }
-}
-
-// 16-byte chunk address inside a SWIZZLE_128B block with 128-byte rows
-__device__ __forceinline__ uint8_t* swz(uint8_t* block, int row, int chunk) { return block + row * 128 + ((chunk ^ (row & 7)) << 4); }
-
-__device__ __forceinline__ void store16(uint8_t* block, int row, int chunk0, const float* v) {
-  *reinterpret_cast<uint4*>(swz(block, row, chunk0)) =
-      make_uint4(pack_bf16x2(v[0], v[1]), pack_bf16x2(v[2], v[3]), pack_bf16x2(v[4], v[5]), pack_bf16x2(v[6], v[7]));
-  *reinterpret_cast<uint4*>(swz(block, row, chunk0 + 1)) =
-      make_uint4(pack_bf16x2(v[8], v[9]), pack_bf16x2(v[10], v[11]), pack_bf16x2(v[12], v[13]), pack_bf16x2(v[14], v[15]));
-}
-
-// NG x 16 consecutive accumulator columns of this thread's TMEM lane -> registers with a single wait
-template <int NG>
-__device__ __forceinline__ void tmem_ld_cols(uint32_t taddr, float (&v)[NG][16]) {
-  uint32_t r[NG][16];
-#pragma unroll
-  for (int i = 0; i < NG; ++i) tmem_ld16_nw(taddr + 16 * i, r[i]);
-  tmem_ld_wait();
-#pragma unroll
-  for (int i = 0; i < NG; ++i) {
-    reg_fence16(r[i]);
-#pragma unroll
-    for (int e = 0; e < 16; ++e) v[i][e] = __uint_as_float(r[i][e]);
-  }
-}
-
 // optional phase timeline of the third window of CTA 0 (clock64 values, low 24 bits as floats) at dbg[63488 + slot]
 #define SCC_T(slot) do { if (p.dbg != nullptr && blockIdx.x == 0 && wi == 2) p.dbg[63488 + (slot)] = (float)(clock64() & 0xFFFFFF); } while (0)
 
@@ -267,7 +195,7 @@ scc_umma_kernel(const __grid_constant__ CUtensorMap tm_t, const __grid_constant_
             const uint32_t acc = (t | ks) != 0 ? 1u : 0u;
             const uint64_t da = make_desc(st + ks * 2048, (uint32_t)p.blk, 1024);
             const uint64_t da2 = make_desc(st + 2 * p.blk + ks * 2048, (uint32_t)p.blk, 1024);
-            const uint64_t dp = kdesc(pool + (ks >> 2) * 8192 + (ks & 3) * 32);
+            const uint64_t dp = umma_desc_sw128(pool + (ks >> 2) * 8192 + (ks & 3) * 32);
             umma_bf16(tmem + kTmG, da, da, id_G, acc);
             umma_bf16(tmem + kTmTlo, da, dp, id_T, acc);
             umma_bf16(tmem + kTmThi, da2, dp, id_T, acc);
@@ -286,16 +214,16 @@ scc_umma_kernel(const __grid_constant__ CUtensorMap tm_t, const __grid_constant_
           // every head's q slice carries its own ones column (position 16h+15), so the k-gen bias rides in the q-part contraction.
           // Issue order interleaves the 12 independent accumulators: back-to-back MMAs never accumulate into the same columns.
           const uint32_t gb = sb + kOffG, tb = sb + kOffTPT, wb = sb + kOffW;
-          const uint64_t w1d = kdesc(wb), w2d = kdesc(wb + 32);
+          const uint64_t w1d = umma_desc_sw128(wb), w2d = umma_desc_sw128(wb + 32);
 #pragma unroll
           for (int h = 0; h < kHeads; ++h) {
-            umma_bf16(tmem + kTmCorr + 16 * h, kdesc(gb + (h >> 2) * kGBlk + (h & 3) * 32), w1d, id_c16, 0u);
+            umma_bf16(tmem + kTmCorr + 16 * h, umma_desc_sw128(gb + (h >> 2) * kGBlk + (h & 3) * 32), w1d, id_c16, 0u);
             umma_bf16(tmem + kTmKP + 16 * h, make_desc(tb + 16 * h * 128, 1024, 1024), w1d, id_kp, 0u);
           }
 #pragma unroll
           for (int h = 0; h < kHeads; ++h) {
             const int cv = 96 + 16 * h;
-            umma_bf16(tmem + kTmCorr + 16 * h, kdesc(gb + (cv >> 6) * kGBlk + (cv & 63) * 2), w2d, id_c16, 1u);
+            umma_bf16(tmem + kTmCorr + 16 * h, umma_desc_sw128(gb + (cv >> 6) * kGBlk + (cv & 63) * 2), w2d, id_c16, 1u);
             umma_bf16(tmem + kTmKP + 16 * h, make_desc(sb + kOffKP + 16 * h * 128, 1024, 1024), w2d, id_kp, 1u);
           }
         }
@@ -306,7 +234,7 @@ scc_umma_kernel(const __grid_constant__ CUtensorMap tm_t, const __grid_constant_
         tc_fence_after();
         SCC_T(4);
         for (int ks = 0; ks < p.cell_ksteps; ++ks)
-          umma_bf16(tmem + kTmMblk, kdesc(sb + kOffTPT + 96 * 128 + ks * 32), make_desc(sb + kOffKP + ks * 2048, 8192, 1024), id_mb, ks ? 1u : 0u);
+          umma_bf16(tmem + kTmMblk, umma_desc_sw128(sb + kOffTPT + 96 * 128 + ks * 32), make_desc(sb + kOffKP + ks * 2048, 8192, 1024), id_mb, ks ? 1u : 0u);
         umma_commit(mid4_ready);
         SCC_T(5);
         // ---------- phase B
@@ -323,32 +251,32 @@ scc_umma_kernel(const __grid_constant__ CUtensorMap tm_t, const __grid_constant_
           const uint32_t st = sb + s * kStage, D = tmem + (uint32_t)(buf * 192);
           auto corr_step = [&](int ks) {
             const int ch = 96 + 16 * ks;
-            umma_bf16(D + 96, kdesc(st + (ch >> 6) * p.blk + (ch & 63) * 2), kdesc(sb + kOffCorr + ((ch >> 6) - 1) * kGBlk + (ch & 63) * 2), id_oc,
+            umma_bf16(D + 96, umma_desc_sw128(st + (ch >> 6) * p.blk + (ch & 63) * 2), umma_desc_sw128(sb + kOffCorr + ((ch >> 6) - 1) * kGBlk + (ch & 63) * 2), id_oc,
                       ks ? 1u : 0u);
           };
           if (p.resident) {
             // all six bias images are resident: interleave the seven independent accumulators (6 heads + out_c)
 #pragma unroll
             for (int h = 0; h < kHeads; ++h)
-              umma_bf16(D + 16 * h, kdesc(st + (h >> 2) * p.blk + (h & 3) * 32), kdesc(sb + kOffMblk + 16 * h * 128 + (h & 3) * 32), id_c16, 0u);
+              umma_bf16(D + 16 * h, umma_desc_sw128(st + (h >> 2) * p.blk + (h & 3) * 32), umma_desc_sw128(sb + kOffMblk + 16 * h * 128 + (h & 3) * 32), id_c16, 0u);
             corr_step(0);
             for (int ks = 0; ks < p.cell_ksteps; ++ks) {
 #pragma unroll
               for (int h = 0; h < kHeads; ++h)
-                umma_bf16(D + 16 * h, kdesc(sb + res_bias_off(h, p.bias_bytes) + ks * 32), kdesc(sb + kOffTPT + (96 + 16 * h) * 128 + ks * 32), id_c16, 1u);
+                umma_bf16(D + 16 * h, umma_desc_sw128(sb + res_bias_off(h, p.bias_bytes) + ks * 32), umma_desc_sw128(sb + kOffTPT + (96 + 16 * h) * 128 + ks * 32), id_c16, 1u);
               if (ks + 1 < 6) corr_step(ks + 1);
             }
             for (int ks = p.cell_ksteps + 1; ks < 6; ++ks) corr_step(ks);
           } else {
             for (int h = 0; h < kHeads; ++h) {
-              umma_bf16(D + 16 * h, kdesc(st + (h >> 2) * p.blk + (h & 3) * 32), kdesc(sb + kOffMblk + 16 * h * 128 + (h & 3) * 32), id_c16, 0u);
+              umma_bf16(D + 16 * h, umma_desc_sw128(st + (h >> 2) * p.blk + (h & 3) * 32), umma_desc_sw128(sb + kOffMblk + 16 * h * 128 + (h & 3) * 32), id_c16, 0u);
               corr_step(h);
               const int r = (int)(ring_cnt & 3u);
               wait_bar(ring_full(r), (ring_cnt >> 2) & 1u);
               tc_fence_after();
               const uint32_t bias = sb + kOffRing + r * kSlot, vp = sb + kOffTPT + (96 + 16 * h) * 128;
 #pragma unroll
-              for (int ks = 0; ks < 4; ++ks) umma_bf16(D + 16 * h, kdesc(bias + ks * 32), kdesc(vp + ks * 32), id_c16, 1u);
+              for (int ks = 0; ks < 4; ++ks) umma_bf16(D + 16 * h, umma_desc_sw128(bias + ks * 32), umma_desc_sw128(vp + ks * 32), id_c16, 1u);
               umma_commit(ring_empty(r));
               ++ring_cnt;
             }
@@ -377,7 +305,7 @@ scc_umma_kernel(const __grid_constant__ CUtensorMap tm_t, const __grid_constant_
 #pragma unroll
             for (int blk = 0; blk < 3; ++blk) tma_store_4d(&tm_o, sb + s * kStage + blk * p.blk, blk * 64, x0, y0, b);
             tma_commit();
-            tma_wait_read0();
+            tma_wait_read<0>();
           }
           mbar_arrive(tok_empty(s));
         }

@@ -5,9 +5,11 @@
 // TMEM lane r).  Operands are staged by TMA into 128B-swizzled K-major shared-memory tiles
 // (A: 128 rows x 64 bf16, B: BN rows x 64 bf16 per stage), the fp32 accumulator tile
 // (128 x BN) lives in TMEM and is double-buffered so the epilogue of tile i overlaps the MMAs
-// of tile i+1.  The same kernel serves token-major linears (2-D tensor map) and 3x3
-// convolutions as implicit GEMM (4-D NHWC tensor map, one TMA box per filter tap, zero padding
-// from TMA out-of-bounds fill).
+// of tile i+1.  The mainloop serves token-major linears (2-D tensor map) and 3x3 convolutions
+// as implicit GEMM (4-D NHWC tensor map, one TMA box per filter tap, zero padding from TMA
+// out-of-bounds fill); the epilogue stores each row's values straight to global memory, which
+// is what the pixel-shuffle heads (EPI_SHUFFLE_*, gemm.cuh) need.  Every other epilogue runs on
+// the TMA-staged kernel (umma_gemm_tma.cu).
 #include "gemm.cuh"
 
 namespace hitsir {
@@ -73,12 +75,7 @@ umma_gemm_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_consta
       int stage = 0; uint32_t phase = 0;
       for (int w = blockIdx.x; w < total; w += gridDim.x) {
         const int n_tile = w % p.n_tiles, m_tile = w / p.n_tiles;
-        int b = 0, y0 = 0, x0 = 0;
-        if (p.conv) {
-          const int tx = m_tile % p.tiles_x; const int t2 = m_tile / p.tiles_x;
-          const int ty = t2 % p.tiles_y; b = t2 / p.tiles_y;
-          y0 = ty * 8; x0 = tx * 16;
-        }
+        const ConvTile t = p.conv ? conv_tile(m_tile, p.tiles_x, p.tiles_y) : ConvTile{0, 0, 0};
         for (int kb = 0; kb < p.num_kb; ++kb) {
           mbar_wait(empty_bar(stage), phase ^ 1u);
           const uint32_t sa = smem_base + stage * Cfg::kStageBytes;
@@ -87,7 +84,7 @@ umma_gemm_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_consta
           if (p.conv) {
             const int tap = kb / p.cblocks, cb = kb - tap * p.cblocks;
             const int dy = tap / 3 - 1, dx = tap % 3 - 1;
-            tma_load_4d(sa, &tmap_a, full_bar(stage), cb * 64, x0 + dx, y0 + dy + p.a_y_off, b);
+            tma_load_4d(sa, &tmap_a, full_bar(stage), cb * 64, t.x0 + dx, t.y0 + dy + p.a_y_off, t.b);
           } else {
             tma_load_2d(sa, &tmap_a, full_bar(stage), kb * 64, m_tile * 128);
           }
@@ -239,12 +236,11 @@ static int launch_bn(const GemmParams& p, const CUtensorMap& ta, const CUtensorM
 }
 
 int launch_umma_gemm(int BN, const GemmParams& p, const CUtensorMap& ta, const CUtensorMap& tb, int num_sms, cudaStream_t st) {
+  if (p.epi != EPI_SHUFFLE_NCHW && p.epi != EPI_SHUFFLE_BF16) { set_error("launch_umma_gemm: epilogue %d is not a pixel shuffle", p.epi); return 1; }
   switch (BN) {
     case 16: return launch_bn<16>(p, ta, tb, num_sms, st);
     case 32: return launch_bn<32>(p, ta, tb, num_sms, st);
-    case 48: return launch_bn<48>(p, ta, tb, num_sms, st);
     case 64: return launch_bn<64>(p, ta, tb, num_sms, st);
-    case 160: return launch_bn<160>(p, ta, tb, num_sms, st);
     case 192: return launch_bn<192>(p, ta, tb, num_sms, st);
     case 256: return launch_bn<256>(p, ta, tb, num_sms, st);
     default: set_error("launch_umma_gemm: unsupported N tile %d", BN); return 1;

@@ -36,29 +36,14 @@ struct TmaCfg {
   static constexpr int kOutCols = kGroups * 64; // output columns produced per N tile
 };
 
-__device__ __forceinline__ void tma_store_2d(const void* tmap, uint32_t src, int c0, int c1) {
-  asm volatile("cp.async.bulk.tensor.2d.global.shared::cta.bulk_group [%0, {%2, %3}], [%1];" ::"l"(tmap), "r"(src), "r"(c0), "r"(c1) : "memory");
-}
-__device__ __forceinline__ void tma_store_4d(const void* tmap, uint32_t src, int c0, int c1, int c2, int c3) {
-  asm volatile("cp.async.bulk.tensor.4d.global.shared::cta.bulk_group [%0, {%2, %3, %4, %5}], [%1];" ::"l"(tmap), "r"(src), "r"(c0), "r"(c1),
-               "r"(c2), "r"(c3) : "memory");
-}
-__device__ __forceinline__ void tma_commit() { asm volatile("cp.async.bulk.commit_group;" ::: "memory"); }
-__device__ __forceinline__ void tma_wait_read1() { asm volatile("cp.async.bulk.wait_group.read 1;" ::: "memory"); }   // all but the newest group
-__device__ __forceinline__ void tma_wait_all0() { asm volatile("cp.async.bulk.wait_group 0;" ::: "memory"); }
-
 struct TileCoord {
   int m_tile, n_tile, b, y0, x0;
 };
 __device__ __forceinline__ TileCoord tile_coord(const GemmParams& p, int w) {
   TileCoord t;
   t.n_tile = w % p.n_tiles; t.m_tile = w / p.n_tiles;
-  t.b = 0; t.y0 = 0; t.x0 = 0;
-  if (p.conv) {
-    const int tx = t.m_tile % p.tiles_x; const int t2 = t.m_tile / p.tiles_x;
-    const int ty = t2 % p.tiles_y; t.b = t2 / p.tiles_y;
-    t.y0 = ty * 8; t.x0 = tx * 16;
-  }
+  const ConvTile c = p.conv ? conv_tile(t.m_tile, p.tiles_x, p.tiles_y) : ConvTile{0, 0, 0};
+  t.b = c.b; t.y0 = c.y0; t.x0 = c.x0;
   return t;
 }
 
@@ -234,7 +219,7 @@ umma_gemm_tma_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_co
             // newest store (waiting for group 0 here exposed one full store latency per box: ~6k cycles per fc1 tile).
             const uint32_t need = u_prep - (uint32_t)nb + 2u;
             while (u_store < need && u_store < u_prep) store_one();
-            tma_wait_read1();
+            tma_wait_read<1>();
           }
           c0s[s] = col;
           if (p.conv) { r0s[s] = t.x0; r1s[s] = t.y0; r2s[s] = t.b; } else { r0s[s] = t.m_tile * 128; r1s[s] = 0; r2s[s] = 0; }
@@ -301,10 +286,7 @@ umma_gemm_tma_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_co
             v[i] = fmaf(v[i], rcp_approx(1.0f + e), v[i]);
           }
         } else {
-          if (p.act == ACT_GELU) {
-#pragma unroll
-            for (int i = 0; i < SW; i += 2) { const float2 gl = gelu2(make_float2(v[i], v[i + 1])); v[i] = gl.x; v[i + 1] = gl.y; }
-          } else if (p.act == ACT_LRELU) {
+          if (p.act == ACT_LRELU) {
 #pragma unroll
             for (int i = 0; i < SW; ++i) v[i] = lrelu(v[i], p.slope);
           }
@@ -379,6 +361,7 @@ static int launch_tma_bn(const GemmParams& p, const CUtensorMap* maps, int num_s
 
 // maps: {A, B, out_f32, out_bf16, residual}; unused maps may be copies of any valid map
 int launch_umma_gemm_tma(int BN, const GemmParams& p, const CUtensorMap* maps, int num_sms, cudaStream_t st) {
+  if (p.epi != EPI_STORE && p.epi != EPI_MSGATE) { set_error("launch_umma_gemm_tma: unsupported epilogue %d", p.epi); return 1; }
   switch (BN) {
     case 64: return launch_tma_bn<64, 2>(p, maps, num_sms, st);     // 64-column tiles: the 8-warp epilogue is already hidden under the 9-tap mainloop
     case 160: return launch_tma_bn<160, 4>(p, maps, num_sms, st);
