@@ -5,7 +5,8 @@
     documented arithmetic;
 (c) plausible kernel bugs applied to the simulated kernel are rejected by the same assertion: the bound is tight enough to matter.
 
-tests/test_gpu_stage_fp64.py makes the same assertions on the CUDA kernels."""
+tests/test_gpu_stage_fp64.py and tests/test_gpu_stage_fp64_front.py (window self-correlation, casa gate, entry, fusion) make the same assertions on the
+CUDA kernels."""
 import pytest
 import torch
 
@@ -272,3 +273,119 @@ def test_resi_3conv(p):
     ref, bound = sr.resi_3conv(x, sd, p, sr.REF, res)
     sr.check_bound("3conv sim", sr.resi_3conv(x, sd, p, sr.SIM, res)[0], ref, bound)
     rejected("taps transposed", sr.resi_3conv(x, sd, p, sr.SIM, res, {"taps_transposed"})[0], ref, bound)
+
+
+# ---- casa gate ----------------------------------------------------------------------------------------------------------------
+WINDOWS = (4, 8, 16, 32, 48, 64)
+
+
+@pytest.mark.parametrize("j", range(6))
+def test_casa_qkv(net, j):
+    """Block input -> the gated, reflect-padded token map (tap `block0.j.qkv`).  At 33 x 37 every window size pads both axes, so
+    the reflected strips carry pixels that count twice in the pools and the gate convs read mirrored statistics at the edge.
+    Pools over the unpadded map are rejected at w = 4, 8, 16 and 48 only: at w = 32 and 64 they move no output element by more than
+    about half its bound (the bound there is dominated by the bf16 ulp of the stored token), so that mutant is not checked there."""
+    sd, taps = net
+    P, x, win = sr.block_params(sd, 0, j), block_input(taps, j), WINDOWS[j]
+    fp32_noise("qkv", sr.casa_qkv(x, P, win, sr.PIN)[0], taps[f"block0.{j}.qkv"])
+    ref, bound = sr.casa_qkv(x, P, win, sr.REF)
+    sr.check_bound(f"casa w={win} sim", sr.casa_qkv(x, P, win, sr.SIM)[0], ref, bound)
+    for mut in ("halo_zero", "lrelu_slope") + (() if win in (32, 64) else ("pool_unpadded",)):
+        rejected(mut, sr.casa_qkv(x, P, win, sr.SIM, {mut})[0], ref, bound)
+
+
+def test_casa_qkv_large_mean(net):
+    """The shifted case of the GPU test: block input + 256 on every channel, so the pooled means are large next to the gate."""
+    sd, taps = net
+    P, x = sr.block_params(sd, 0, 0), taps["embed"] + 256.0
+    ref, bound = sr.casa_qkv(x, P, 4, sr.REF)
+    sr.check_bound("casa sim, large mean", sr.casa_qkv(x, P, 4, sr.SIM)[0], ref, bound)
+
+
+# ---- entry: mean shift + conv_first -------------------------------------------------------------------------------------------
+def test_entry_multi_size(net):
+    sd, taps = net
+    x = synthetic_image(B, H, W, seed=4)
+    fp32_noise("shallow", sr.entry(x, sd, sr.PIN)[0], taps["shallow"])
+    ref, bound = sr.entry(x, sd, sr.REF)
+    sr.check_bound("entry sim", sr.entry(x, sd, sr.SIM)[0], ref, bound)
+    for mut in ("gate_no_residual", "mean_added"):
+        rejected(mut, sr.entry(x, sd, sr.SIM, mut={mut})[0], ref, bound)
+
+
+def saturating_entry(sd):
+    """conv_x scaled by 8: x1 x_k reaches |z| ~ 20, where the gate's sigmoid saturates (ex2 over- and underflows towards 0 and inf)."""
+    sd = dict(sd)
+    sd["conv_first.conv_x.weight"] = sd["conv_first.conv_x.weight"] * 8.0
+    return sd
+
+
+def test_entry_saturated_gate(net):
+    sd, _ = net
+    sd = saturating_entry(sd)
+    x = synthetic_image(B, H, W, seed=4)
+    ref, bound = sr.entry(x, sd, sr.REF)
+    sr.check_bound("entry sim, saturated gate", sr.entry(x, sd, sr.SIM)[0], ref, bound)
+    rejected("gate_no_residual", sr.entry(x, sd, sr.SIM, mut={"gate_no_residual"})[0], ref, bound)
+
+
+def test_entry_conv_first():
+    _, oracle = build_pair((0, 0, 0), "nearest+conv", 4, "stress", 21)
+    sd = oracle.sd
+    x = synthetic_image(B, H, W, seed=4)
+    taps = {}
+    with torch.no_grad():
+        oracle.forward(x, taps)
+    fp32_noise("shallow", sr.entry(x, sd, sr.PIN, ms=False)[0], taps["shallow"])
+    ref, bound = sr.entry(x, sd, sr.REF, ms=False)
+    sr.check_bound("conv_first sim", sr.entry(x, sd, sr.SIM, ms=False)[0], ref, bound)
+    rejected("mean_added", sr.entry(x, sd, sr.SIM, ms=False, mut={"mean_added"})[0], ref, bound)
+
+
+# ---- fusion ------------------------------------------------------------------------------------------------------------------
+def test_fusion(net):
+    sd, taps = net
+    cab, s = taps["conv_after_body"], taps["shallow"]
+    fp32_noise("fused", sr.fusion(cab, s, sd, sr.PIN)[0], taps["fused"])
+    ref, bound = sr.fusion(cab, s, sd, sr.REF)
+    sr.check_bound("fusion sim", sr.fusion(cab, s, sd, sr.SIM)[0], ref, bound)
+    for mut in ("swap", "sig_outside", "ch_h_not_transposed", "planes_swapped"):
+        rejected(mut, sr.fusion(cab, s, sd, sr.SIM, {mut})[0], ref, bound)
+
+
+# ---- window self-correlation --------------------------------------------------------------------------------------------------
+def pooled_bias(sd, j):
+    from oracle.hitsir_oracle import dynamic_pos_bias_table, pooled_rpe_bias
+    win = WINDOWS[j]
+    tbl = dynamic_pos_bias_table(sd, f"layers.0.residual_group.blocks.{j}.correlation.", (win, win))
+    return pooled_rpe_bias(tbl, (win, win), (min(win, 8), min(win, 8)))
+
+
+SCC_MUTANTS = ("no_bsl_vpt", "no_bsl_kp", "scale16", "inv_lb", "kgen_swapped", "no_ones", "bias_transposed", "bias_xy")
+SCC_UNREJECTED = {16: ("no_bsl_vpt", "no_bsl_kp", "no_ones"), 32: ("no_bsl_kp", "no_ones"), 48: ("no_bsl_vpt", "no_bsl_kp", "no_ones"),
+                  64: ("no_bsl_vpt", "no_bsl_kp", "no_ones")}
+
+
+@pytest.mark.parametrize("j", range(6))
+def test_scc(net, j):
+    """Tap `block0.j.qkv` (the padded token map) + the pooled bias -> tap `block0.j.scc`; SIM is `scc_dense` for w = 4, 8 and
+    `scc_umma` for w >= 16.  Mutants that do not apply to a kernel are skipped: "bias_transposed" needs the square L x L table of
+    `scc_dense`, "bias_xy" is its `scc_umma` counterpart, and "inv_lb" is no bug at r = 1 (Lb = L).
+    Not rejected at this shape (`SCC_UNREJECTED`): in `scc_umma` the bound is dominated by the bf16 rounding of G = Q^T T, a sum over
+    L tokens carried through |Wk| / L and |V|, and of KP; spatial_linear.bias and the k-gen bias move the output by less than that at
+    w = 16, 48, 64 (no_bsl_vpt, no_bsl_kp, no_ones; worst ratios 0.16 .. 1.0), and at w = 32 for no_bsl_kp (1.08, too close to 1 to
+    count) and no_ones.  Each of them is rejected at w = 4 and 8, and no_bsl_vpt also at w = 32."""
+    sd, taps = net
+    P, win = sr.block_params(sd, 0, j), WINDOWS[j]
+    bias = pooled_bias(sd, j)
+    tok = taps[f"block0.{j}.qkv"]
+    fp32_noise("scc", sr.scc(tok, bias, P, win, sr.PIN, (H, W))[0], taps[f"block0.{j}.scc"])
+    tok = sr.bf(tok).float()
+    ref, bound = sr.scc(tok, bias, P, win, sr.REF, (H, W))
+    sr.check_bound(f"scc w={win} sim", sr.scc(tok, bias, P, win, sr.SIM, (H, W))[0], ref, bound)
+    dense = win <= 8
+    for mut in SCC_MUTANTS:
+        if (mut == "bias_xy" and dense) or (mut in ("bias_transposed",) and not dense) or (mut == "inv_lb" and dense) \
+                or mut in SCC_UNREJECTED.get(win, ()):
+            continue
+        rejected(mut, sr.scc(tok, bias, P, win, sr.SIM, (H, W), {mut})[0], ref, bound)
