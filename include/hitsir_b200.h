@@ -169,6 +169,33 @@ HITSIR_API int hitsir_forward_x8_u8(HitsirHandle* h, const uint8_t* x_hwc, uint8
  * the fp32 bytes cross NVLink.  Needs no handle; asynchronous on `stream`. */
 HITSIR_API int hitsir_f32nchw_to_u8hwc(const float* src, uint8_t* dst, int B, int C, int H, int W, void* stream);
 
+/* The entry conversion alone, the mirror of hitsir_f32nchw_to_u8hwc: torchvision's to_tensor (utils/utils.py:143-145: value / 255 in
+ * fp32) of a uint8 HWC batch [B,H,W,C] into fp32 NCHW [B,C,H,W], both on the device; the conversion hitsir_forward_u8 applies to its
+ * input.  Needs no handle; asynchronous on `stream`. */
+HITSIR_API int hitsir_u8hwc_to_f32nchw(const uint8_t* src, float* dst, int B, int C, int H, int W, void* stream);
+
+/* ---- bicubic resizing: the LR synthesis of the evaluation (datasets/dataset.py:51-91) and the "Bicubic" baseline ------------------
+ * Two standard definitions over one separable resampler (horizontal pass, then vertical) with per-axis tap tables that the call builds
+ * on the device in `scratch` (hitsir_resize_scratch_bytes(mode, H, W, outH, outW) bytes of device memory, 4-byte aligned): no host copy, so a call
+ * can be captured in a CUDA graph.  No atomics (bitwise reproducible; an image's result does not depend on the rest of the batch),
+ * asynchronous on `stream`, no handle.  Null pointers, an empty batch, a zero-sized input or output and C not in {1, 3} are
+ * HITSIR_ERR_INVALID, and so is a downscale so strong that a tile's tap tables outgrow a CTA's shared memory (a factor above ~150). */
+enum { HITSIR_RESIZE_PIL = 0, HITSIR_RESIZE_MATLAB = 1 };
+/* For HITSIR_RESIZE_MATLAB pass outH = ceil(H * scale), outW = ceil(W * scale); an axis that shrinks to one sample is sized for
+ * scale >= 1 / max(its length, 16), and a smaller scale is HITSIR_ERR_INVALID.  0 for arguments the entries refuse. */
+HITSIR_API int64_t hitsir_resize_scratch_bytes(int mode, int H, int W, int outH, int outW);
+/* Pillow 12.2 Image.resize((outW, outH), Image.BICUBIC), modes "L" (C = 1) and "RGB" (C = 3), box and reducing_gap at their defaults:
+ * bit-exact.  Cubic a = -0.5 with support 2 * max(in/out, 1), weights normalised in double and rounded to 22-bit fixed point, int32
+ * sums, uint8 intermediate (libImaging/Resample.c).  uint8 HWC [B,H,W,C] -> uint8 HWC [B,outH,outW,C]. */
+HITSIR_API int hitsir_resize_u8_pil(const uint8_t* src_hwc, uint8_t* dst_hwc, int B, int H, int W, int C, int outH, int outW, void* scratch,
+                         void* stream);
+/* MATLAB imresize(x, scale, 'bicubic') as BasicSR's calculate_weights_indices + imresize compute it: cubic a = -0.5, antialiased
+ * (kernel width 4 / scale) when scale < 1, half-sample symmetric boundary, output ceil(H * scale) x ceil(W * scale).  Weights in fp64
+ * rounded to fp32, fp32 FMA accumulation in tap order: within a bound of the fp64 result that tests/resize_ref.py derives, not
+ * bit-exact to BasicSR (fp32 weights, unspecified summation order).  fp32 NCHW [B,C,H,W] -> fp32 NCHW, values not clipped. */
+HITSIR_API int hitsir_resize_f32_matlab(const float* src_nchw, float* dst_nchw, int B, int C, int H, int W, double scale, void* scratch,
+                             void* stream);
+
 /* The evaluation metric around the path on the device (experiments/experiment.py:436-463, called per batch from :743-755): both fp32
  * NCHW batches [B,3,H,W] in [0,1] are converted to the Y channel of YCbCr exactly as utils/utils.py:170-186 does
  * (16/255 + (65.738 R + 129.057 G + 25.064 B) / 256, fp32), `sr` clipped to [0,1] first when clip_sr != 0 (experiment.py:746-748),

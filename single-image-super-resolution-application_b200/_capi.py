@@ -18,6 +18,8 @@ UPSAMPLERS = {None: 0, "": 0, "pixelshuffle": 1, "pixelshuffledirect": 2, "neare
 
 ERR_CUDA, ERR_INVALID, ERR_UNSUPPORTED, ERR_INPUT_TOO_SMALL, ERR_WEIGHTS, ERR_WORKSPACE = 1, 2, 3, 4, 5, 6
 
+RESIZE_PIL, RESIZE_MATLAB = 0, 1
+
 
 class HitsirConfig(C.Structure):
     _fields_ = [
@@ -77,6 +79,10 @@ SYMBOLS = {
     "hitsir_ssim_y_scratch_doubles": (C.c_int64, [C.c_int, C.c_int, C.c_int, C.c_int]),
     "hitsir_ssim_y": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p,
                                 C.c_void_p]),
+    "hitsir_u8hwc_to_f32nchw": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p]),
+    "hitsir_resize_scratch_bytes": (C.c_int64, [C.c_int, C.c_int, C.c_int, C.c_int, C.c_int]),
+    "hitsir_resize_u8_pil": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p]),
+    "hitsir_resize_f32_matlab": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_double, C.c_void_p, C.c_void_p]),
     "hitsir_set_tap": (C.c_int, [C.c_void_p, C.c_char_p, C.c_void_p, C.c_int64, C.c_int]),
     "hitsir_set_inject": (C.c_int, [C.c_void_p, C.c_char_p, C.c_void_p, C.c_int64]),
     "hitsir_get_bias_table": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_int64, C.c_void_p]),

@@ -2,6 +2,7 @@
 // layout and the forward-pass orchestration of HiT_SIR.forward
 // (/root/reference/models/hit_sir_pro.py:1304-1344) behind the C ABI of include/hitsir_b200.h.
 #include <stdarg.h>
+#include <math.h>
 #include <stdlib.h>
 #include <string.h>
 
@@ -1307,6 +1308,49 @@ HITSIR_API int hitsir_forward_x8_u8(HitsirHandle* h, const uint8_t* x_hwc, uint8
 HITSIR_API int hitsir_f32nchw_to_u8hwc(const float* src, uint8_t* dst, int B, int C, int H, int W, void* stream) {
   if (!src || !dst || B <= 0 || C <= 0 || H <= 0 || W <= 0) { set_error("hitsir_f32nchw_to_u8hwc: bad argument"); return HITSIR_ERR_INVALID; }
   if (launch_f32nchw_to_u8hwc(src, dst, B, H, W, C, (cudaStream_t)stream)) return HITSIR_ERR_CUDA;
+  return 0;
+}
+
+HITSIR_API int hitsir_u8hwc_to_f32nchw(const uint8_t* src, float* dst, int B, int C, int H, int W, void* stream) {
+  if (!src || !dst || B <= 0 || C <= 0 || H <= 0 || W <= 0) { set_error("hitsir_u8hwc_to_f32nchw: bad argument"); return HITSIR_ERR_INVALID; }
+  if (launch_u8hwc_to_f32nchw(src, dst, B, H, W, C, (cudaStream_t)stream)) return HITSIR_ERR_CUDA;
+  return 0;
+}
+
+// ceil(in * scale) in double, as BasicSR's math.ceil(in_h * scale); 0 when it is not a positive int
+static int matlab_out_size(int in, double scale) {
+  const double o = ceil((double)in * scale);
+  return (o >= 1.0 && o <= 2147483647.0) ? (int)o : 0;
+}
+
+HITSIR_API int64_t hitsir_resize_scratch_bytes(int mode, int H, int W, int outH, int outW) {
+  if ((mode != HITSIR_RESIZE_PIL && mode != HITSIR_RESIZE_MATLAB) || H <= 0 || W <= 0 || outH <= 0 || outW <= 0) return 0;
+  return resize_scratch_bytes(mode == HITSIR_RESIZE_MATLAB, H, W, outH, outW);
+}
+
+HITSIR_API int hitsir_resize_u8_pil(const uint8_t* src_hwc, uint8_t* dst_hwc, int B, int H, int W, int C, int outH, int outW, void* scratch,
+                                    void* stream) {
+  if (!src_hwc || !dst_hwc || !scratch) { set_error("hitsir_resize_u8_pil: null argument"); return HITSIR_ERR_INVALID; }
+  if (B <= 0 || H <= 0 || W <= 0 || outH <= 0 || outW <= 0 || (C != 1 && C != 3) || B > 65535) {
+    set_error("hitsir_resize_u8_pil: bad shape B=%d %d x %d x %d -> %d x %d (C must be 1 or 3)", B, H, W, C, outH, outW);
+    return HITSIR_ERR_INVALID;
+  }
+  if (resize_check(0, C, H, W, outH, outW, 0.0)) return HITSIR_ERR_INVALID;
+  if (launch_resize_pil(src_hwc, dst_hwc, B, H, W, C, outH, outW, scratch, (cudaStream_t)stream)) return HITSIR_ERR_CUDA;
+  return 0;
+}
+
+HITSIR_API int hitsir_resize_f32_matlab(const float* src_nchw, float* dst_nchw, int B, int C, int H, int W, double scale, void* scratch,
+                                        void* stream) {
+  if (!src_nchw || !dst_nchw || !scratch) { set_error("hitsir_resize_f32_matlab: null argument"); return HITSIR_ERR_INVALID; }
+  const int outH = (scale > 0.0 && isfinite(scale)) ? matlab_out_size(H, scale) : 0;
+  const int outW = (scale > 0.0 && isfinite(scale)) ? matlab_out_size(W, scale) : 0;
+  if (B <= 0 || H <= 0 || W <= 0 || (C != 1 && C != 3) || (long long)B * C > 65535 || outH <= 0 || outW <= 0) {
+    set_error("hitsir_resize_f32_matlab: bad shape or scale B=%d C=%d %d x %d scale %g (C must be 1 or 3)", B, C, H, W, scale);
+    return HITSIR_ERR_INVALID;
+  }
+  if (resize_check(1, C, H, W, outH, outW, scale)) return HITSIR_ERR_INVALID;
+  if (launch_resize_matlab(src_nchw, dst_nchw, B, C, H, W, scale, outH, outW, scratch, (cudaStream_t)stream)) return HITSIR_ERR_CUDA;
   return 0;
 }
 

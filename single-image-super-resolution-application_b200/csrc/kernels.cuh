@@ -67,6 +67,14 @@ long long ssim_y_tiles(int H, int W, int gaussian);
 int launch_ssim_y(const float* sr, const float* hr, int B, int H, int W, int clip, int gaussian, int sample_cov, double* partial, double* ssim,
                   cudaStream_t st);
 
+// ---- resize.cu (bicubic resizing: Pillow's Image.resize(BICUBIC) on uint8 HWC, MATLAB imresize as BasicSR computes it on fp32 NCHW) ----
+// 0 when the shapes (and scale, matlab) are within what the kernel supports, else 1 with the error message set
+int resize_check(int matlab, int C, int H, int W, int outH, int outW, double scale);
+long long resize_scratch_bytes(int matlab, int H, int W, int outH, int outW);
+int launch_resize_pil(const uint8_t* src, uint8_t* dst, int B, int H, int W, int C, int outH, int outW, void* scratch, cudaStream_t st);
+int launch_resize_matlab(const float* src, float* dst, int B, int C, int H, int W, double scale, int outH, int outW, void* scratch,
+                         cudaStream_t st);
+
 // ---- casa (SpatialChannelAttention, hit_sir_pro.py:338-359) ------------------------------
 struct CasaW {
   const float* w1; const float* b1;      // linear1: Conv2d(1,C,3) as [9][C], [C]
