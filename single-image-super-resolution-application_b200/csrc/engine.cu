@@ -442,8 +442,8 @@ int finalize(HitsirHandle* h, cudaStream_t st) {
       if (launch_pos_table(pw, bw.win, tbl_scratch, st)) return 1;
       if (launch_pooled_bias(tbl_scratch, bw.win, bw.base, bw.bias_tbl, st)) return 1;
       bw.scc.bias_tbl = bw.bias_tbl;
-      if (dev_alloc(h, &bw.pool_img, scc_pool_image_bytes(bw.win)) || dev_alloc(h, &bw.bias_img, scc_bias_image_bytes(bw.win)) ||
-          dev_alloc(h, &bw.w_img, 2048)) return 1;
+      if (bw.r > 1 && dev_alloc(h, &bw.pool_img, scc_pool_image_bytes(bw.win))) return 1;     // only scc_umma (r > 1) reads it
+      if (dev_alloc(h, &bw.bias_img, scc_bias_image_bytes(bw.win)) || dev_alloc(h, &bw.w_img, 2048)) return 1;
       if (launch_scc_images(bw.scc, bw.win, bw.base, bw.pool_img, bw.bias_img, bw.w_img, st)) return 1;
       bw.scc.pool_img = bw.pool_img; bw.scc.bias_img = bw.bias_img; bw.scc.w_img = bw.w_img;
       // proj consumes the SCC output in its head-padded channel order (kernels.cuh scc_pos)
@@ -532,7 +532,6 @@ struct Workspace {
   bf16* T = nullptr;                                     // bf16 [NpMax,192] qkv tokens on the padded map
   float *cavg = nullptr, *cmax = nullptr;                // [NpMax]
   float *part_sum = nullptr, *part_max = nullptr, *s1 = nullptr, *s2 = nullptr;
-  float* scc_dbg = nullptr;
   bf16* outsc = nullptr;                                 // bf16 [N,192]
   bf16 *H1 = nullptr, *H2 = nullptr;                     // bf16 [N,384] (contiguous: also G [N,768], A1|A2 fp32)
   float *havg, *hmax, *wavg, *wmax, *c_att, *h_att, *w_att;
@@ -604,7 +603,6 @@ int layout_workspace(const HitsirHandle* h, int B, int H, int W, void* base, Wor
   }
   ws->s1 = b.take<float>((size_t)B * kC);
   ws->s2 = b.take<float>((size_t)B * kC);
-  ws->scc_dbg = b.take<float>((size_t)kSccDbgFloats);
   ws->outsc = b.take_ext<bf16>(N * kCp, hr * kCp);
   ws->H1 = b.take_ext<bf16>(N * kHidp * 2, 2 * hr * kHidp);  // H1 | H2 contiguous
   ws->H2 = ws->H1 ? ws->H1 + N * kHidp : nullptr;
@@ -822,7 +820,7 @@ int forward_block(Fwd& f, int i, int j, float* xin, float* xout) {
     g.pg.top = f.top ? 1 : 0; g.pg.bot = (f.bot && g.pg.Hp == f.H) ? 1 : 0;
   }
   g.w = w; g.base = bw.base; g.r = bw.r; g.L = w * w; g.Lb = bw.base * bw.base;
-  g.nWy = g.pg.Hp / w; g.nWx = g.pg.Wp / w; g.parts = 1;
+  g.nWy = g.pg.Hp / w; g.nWx = g.pg.Wp / w;
   const long long Np = (long long)f.B * g.pg.Hp * g.pg.Wp;
   {
     const Inject& in = h->inject;
@@ -852,14 +850,12 @@ int forward_block(Fwd& f, int i, int j, float* xin, float* xout) {
   LAUNCH("qkv_build", 1, launch_qkv_build(xin, g.pg, c.is_channel_spatial_attn, ws.cavg, ws.cmax, ws.s1, ws.s2, bw.casa, ws.T, f.st));
   TAPP((tn + ".qkv").c_str(), ws.T, 1, kCp, Np, kC);
   {
-    const bool want_dbg = h->tap.dst != nullptr && h->tap.name == tn + ".sccdbg";
     char cat[16]; snprintf(cat, sizeof(cat), "scc_w%d", w);
-    if (g.r == 1 && !want_dbg)
+    if (g.r == 1)
       LAUNCH(cat, 1, launch_scc_dense(ws.T, g, bw.scc, ws.outsc, h->num_sms, f.st));
     else
-      LAUNCH(cat, 1, launch_scc_umma(ws.T, g, bw.scc, ws.outsc, want_dbg ? ws.scc_dbg : nullptr, h->num_sms, f.st));
+      LAUNCH(cat, 1, launch_scc_umma(ws.T, g, bw.scc, ws.outsc, h->num_sms, f.st));
   }
-  TAP((tn + ".sccdbg").c_str(), ws.scc_dbg, 0, kSccDbgFloats, 1, kSccDbgFloats);
   TAPP((tn + ".scc").c_str(), ws.outsc, 1, kCp, f.N, kC);
   // proj + norm1 + residual (:597, :700-703) and ConvFFN fc1 + GELU (:39-41) in one kernel
   {
@@ -884,13 +880,12 @@ int forward_block(Fwd& f, int i, int j, float* xin, float* xout) {
     fs = FfnStats{ws.cavg, ws.cmax, ws.part_sum, ws.part_max, round_up(f.band ? f.Hf : f.H, wn), round_up(f.W, wn)};
     fsp = &fs;
   }
-  bf16* shadow = (need_shadow && fsp == nullptr) ? ws.xb0 : nullptr;      // emitted by the kernel's statistics warp
+  bf16* shadow = need_shadow ? ws.xb0 : nullptr;      // emitted by the kernel's statistics warp
   FfnBand fb{2, f.row0, f.Hf};
   if (f.band != nullptr) RUN(fill_halo(f, ws.H1, (size_t)f.W * kHidp * sizeof(bf16), f.H, 2));   // the depthwise 5x5 reads two rows across the band edge
   LAUNCH("ffn_tail", 1, launch_ffn_tail(ws.H1, bw.dw_mma, bw.w2_img, bw.fc2.b, bw.g2, bw.b2, xout, f.B, f.H, f.W, fsp, shadow, h->num_sms, f.st,
                                         f.band ? &fb : nullptr));
   if (fsp != nullptr) f.stats_nparts = ffn_tiles_per_image(f.H, f.W);
-  if (need_shadow && shadow == nullptr) LAUNCH("cast_shadow", 1, launch_cast_rows_bf16(xout, ws.xb0, f.N, f.st));
   TAP(tn.c_str(), xout, 0, kC, f.N, kC);
   return 0;
 }

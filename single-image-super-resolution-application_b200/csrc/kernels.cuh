@@ -124,7 +124,7 @@ struct SccW {
   const float* wk2; const float* bk2;    // k_generate2
   const float* wsl; float* bsl_dev;      // spatial_linear weight [r*r]; bias read from device (1 float)
   const float* bias_tbl;                 // pooled relative-position bias [6][L][Lb]
-  const uint8_t* pool_img;               // weights-only UMMA operand images (scc_umma.cu)
+  const uint8_t* pool_img;               // weights-only UMMA operand images (scc_umma.cu); pool_img: r > 1 only
   const uint8_t* bias_img;
   const uint8_t* w_img;
 };
@@ -133,14 +133,13 @@ struct SccGeom {
   int w, base, r;      // window, pooled grid side (min(w,8)), w/base
   int L, Lb;
   int nWy, nWx;        // windows per image
-  int parts;           // CTAs per window in the two-phase path (L / 256), 1 for the fused path
 };
 size_t scc_pool_image_bytes(int w);
 size_t scc_bias_image_bytes(int w);
+// pool_img == nullptr skips the pool image (r = 1: scc_dense reads only the bias and k-gen images)
 int launch_scc_images(const SccW& w, int win, int base, uint8_t* pool_img, uint8_t* bias_img, uint8_t* w_img, cudaStream_t st);
-// dbg (optional): fp32 dump of window 0: G[128][192] | TPT[192][64] | corr[128][96] | KP[128][96] | Mblk[128][16]
-constexpr int kSccDbgFloats = 63488 + 32;   // + phase timeline (clock64) of one window
-int launch_scc_umma(const bf16* t, const SccGeom& g, const SccW& w, bf16* out, float* dbg, int num_sms, cudaStream_t st);
+// windows with pooling ratio r > 1 (scc_dense serves r = 1)
+int launch_scc_umma(const bf16* t, const SccGeom& g, const SccW& w, bf16* out, int num_sms, cudaStream_t st);
 // scc_dense.cu: windows of 4x4 / 8x8 tokens (pooling ratio 1), several windows per 128-token tile
 int launch_scc_dense(const bf16* t, const SccGeom& g, const SccW& w, bf16* out, int num_sms, cudaStream_t st);
 

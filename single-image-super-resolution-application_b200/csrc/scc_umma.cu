@@ -21,6 +21,8 @@
 // The token layout is head-padded (6 x 16 | 6 x 16 = 192 channels, kernels.cuh scc_pos); position 15 holds a
 // constant 1 so that the k-gen bias rides along in the contractions.
 //
+// Serves the windows with pooling ratio r > 1: w = 16, 32, 48, 64 (two or more 128-token tiles of 16x8 pixels), and w = 4 / 8 when
+// base_win_size is below the window (one tile: resident mode).  Windows with r = 1 run in scc_dense.cu.
 // One persistent CTA per SM walks whole windows.  Warp roles: warp 0 = TMA producer, warp 1 = MMA issuer,
 // warp 2 = TMEM allocator, warp 3 = TMA-store thread, warps 4..11 = TMEM->register->smem converters / epilogue.
 #include "gemm.cuh"
@@ -68,11 +70,7 @@ struct Params {
   const uint8_t* w_img;      // 2 KB
   const float* bsl;          // spatial_linear.bias (device scalar)
   int H, W;                  // unpadded image size (stores outside are skipped / clipped)
-  float* dbg;                // optional dump of window 0 (see hitsir_scc_debug layout in engine.cu)
 };
-
-// optional phase timeline of the third window of CTA 0 (clock64 values, low 24 bits as floats) at dbg[63488 + slot]
-#define SCC_T(slot) do { if (p.dbg != nullptr && blockIdx.x == 0 && wi == 2) p.dbg[63488 + (slot)] = (float)(clock64() & 0xFFFFFF); } while (0)
 
 __global__ void __launch_bounds__(384, 1)
 scc_umma_kernel(const __grid_constant__ CUtensorMap tm_t, const __grid_constant__ CUtensorMap tm_o, const Params p) {
@@ -182,7 +180,6 @@ scc_umma_kernel(const __grid_constant__ CUtensorMap tm_t, const __grid_constant_
           if (d_cnt > buf) { const uint32_t last = ((d_cnt - 1 - buf) >> 1 << 1) + buf; wait_bar(d_empty((int)buf), (last >> 1) & 1u); }
         tc_fence_after();
         const uint32_t a0 = tok_cnt;
-        SCC_T(0);
         // ---------- phase A
         for (int t = 0; t < p.tiles; ++t) {
           const int s = (int)(tok_cnt & 1u);
@@ -205,11 +202,9 @@ scc_umma_kernel(const __grid_constant__ CUtensorMap tm_t, const __grid_constant_
           ++tok_cnt;
         }
         umma_commit(a_done);
-        SCC_T(1);
         // ---------- mid2: corr = G Wk^T, KP = TPT^T Wk^T (per head: q part, v part, bias via the ones channel)
         wait_bar(mid1_done, (uint32_t)(wi & 1));
         tc_fence_after();
-        SCC_T(2);
         {
           // every head's q slice carries its own ones column (position 16h+15), so the k-gen bias rides in the q-part contraction.
           // Issue order interleaves the 12 independent accumulators: back-to-back MMAs never accumulate into the same columns.
@@ -228,19 +223,15 @@ scc_umma_kernel(const __grid_constant__ CUtensorMap tm_t, const __grid_constant_
           }
         }
         umma_commit(mid2_ready);
-        SCC_T(3);
         // ---------- mid4: Mfull[(h,j)][(h',i)] = sum_m VPT[(h,j)][m] KP[m][(h',i)]
         wait_bar(mid3_done, (uint32_t)(wi & 1));
         tc_fence_after();
-        SCC_T(4);
         for (int ks = 0; ks < p.cell_ksteps; ++ks)
           umma_bf16(tmem + kTmMblk, umma_desc_sw128(sb + kOffTPT + 96 * 128 + ks * 32), make_desc(sb + kOffKP + ks * 2048, 8192, 1024), id_mb, ks ? 1u : 0u);
         umma_commit(mid4_ready);
-        SCC_T(5);
         // ---------- phase B
         wait_bar(mid5_done, (uint32_t)(wi & 1));
         tc_fence_after();
-        SCC_T(6);
         for (int t = 0; t < p.tiles; ++t) {
           const uint32_t idx = p.streaming ? tok_cnt : a0 + (uint32_t)t;
           const int s = (int)(idx & 1u);
@@ -284,7 +275,6 @@ scc_umma_kernel(const __grid_constant__ CUtensorMap tm_t, const __grid_constant_
           umma_commit(d_full(buf));
           ++d_cnt;
         }
-        SCC_T(7);
       }
     }
   } else if (warp == 3) {
@@ -322,12 +312,10 @@ scc_umma_kernel(const __grid_constant__ CUtensorMap tm_t, const __grid_constant_
     uint32_t tok_cnt = 0, d_cnt = 0;
     int wi = 0;
     for (int win = blockIdx.x; win < p.nwin; win += gridDim.x, ++wi) {
-      float* dbg = (p.dbg != nullptr && win == 0) ? p.dbg : nullptr;
       const uint32_t par = (uint32_t)(wi & 1);
       // ---------- mid1: G, TPT -> bf16 operand images
       wait_bar(a_done, par);
       tc_fence_after();
-      if (threadIdx.x == 128) SCC_T(8);
       if (q < 3) {
         float v[6][16];
         tmem_ld_cols<6>(tl + kTmG + hs * 96, v);
@@ -335,7 +323,6 @@ scc_umma_kernel(const __grid_constant__ CUtensorMap tm_t, const __grid_constant_
         for (int i = 0; i < 6; ++i) {
           const int c0 = hs * 96 + 16 * i;
           store16(sp + kOffG + (c0 >> 6) * kGBlk, row, (c0 & 63) >> 3, v[i]);
-          if (dbg) for (int e = 0; e < 16; ++e) dbg[row * 192 + c0 + e] = v[i][e];
         }
       }
       if (hs == 0 || q < 2) {
@@ -354,17 +341,14 @@ scc_umma_kernel(const __grid_constant__ CUtensorMap tm_t, const __grid_constant_
             for (int e = 0; e < 16; ++e) v[i][e] = (16 * i + e < p.Lb && !padrow) ? v[i][e] + bsl : 0.f;
           }
           store16(sp + kOffTPT, crow, 2 * i, v[i]);
-          if (dbg) for (int e = 0; e < 16; ++e) dbg[24576 + crow * 64 + 16 * i + e] = v[i][e];
         }
       }
       tc_fence_before();
       fence_proxy_async_smem();
       mbar_arrive_warp(mid1_done);
-      if (threadIdx.x == 128) SCC_T(9);
       // ---------- mid3: corr, KP -> bf16 operand images
       wait_bar(mid2_ready, par);
       tc_fence_after();
-      if (threadIdx.x == 128) SCC_T(10);
       if (q < 3) {
         float v[3][16];
         tmem_ld_cols<3>(tl + kTmCorr + hs * 48, v);
@@ -374,7 +358,6 @@ scc_umma_kernel(const __grid_constant__ CUtensorMap tm_t, const __grid_constant_
 #pragma unroll
           for (int e = 0; e < 16; ++e) v[i][e] *= p.invL;
           store16(sp + kOffCorr + ((ch >> 6) - 1) * kGBlk, row, (ch & 63) >> 3, v[i]);
-          if (dbg) for (int e = 0; e < 16; ++e) dbg[36864 + row * 96 + c0 + e] = v[i][e];
         }
       }
       if (q < 2) {
@@ -386,17 +369,14 @@ scc_umma_kernel(const __grid_constant__ CUtensorMap tm_t, const __grid_constant_
 #pragma unroll
           for (int e = 0; e < 16; ++e) v[i][e] = (row < p.Lb && e != 15) ? v[i][e] + bsl : 0.f;
           store16(sp + kOffKP + (c0 >> 6) * 8192, row, (c0 & 63) >> 3, v[i]);
-          if (dbg) for (int e = 0; e < 16; ++e) dbg[49152 + row * 96 + c0 + e] = v[i][e];
         }
       }
       tc_fence_before();
       fence_proxy_async_smem();
       mbar_arrive_warp(mid3_done);
-      if (threadIdx.x == 128) SCC_T(11);
       // ---------- mid5: diagonal blocks of Mfull / 15 -> Mblk operand image
       wait_bar(mid4_ready, par);
       tc_fence_after();
-      if (threadIdx.x == 128) SCC_T(12);
       if (hs == 0 && q < 3) {
         float v[2][16];
         tmem_ld_cols<2>(tl + kTmMblk + 32 * q, v);
@@ -405,12 +385,10 @@ scc_umma_kernel(const __grid_constant__ CUtensorMap tm_t, const __grid_constant_
 #pragma unroll
         for (int e = 0; e < 16; ++e) o[e] = ((lane & 16) ? v[1][e] : v[0][e]) * (1.0f / 15.0f);
         store16(sp + kOffMblk, row, 2 * (h & 3), o);
-        if (dbg) for (int e = 0; e < 16; ++e) dbg[61440 + row * 16 + e] = o[e];
       }
       tc_fence_before();
       fence_proxy_async_smem();
       mbar_arrive_warp(mid5_done);
-      if (threadIdx.x == 128) SCC_T(13);
       // ---------- phase B epilogue: accumulator -> bf16, in place over the consumed token tile, then TMA store
       const uint32_t a0 = tok_cnt;
       for (int t = 0; t < p.tiles; ++t) {
@@ -419,7 +397,6 @@ scc_umma_kernel(const __grid_constant__ CUtensorMap tm_t, const __grid_constant_
         const int buf = (int)(d_cnt & 1u);
         wait_bar(d_full(buf), (d_cnt >> 1) & 1u);
         tc_fence_after();
-        if (threadIdx.x == 128) SCC_T(14);
         uint8_t* stp = sp + s * kStage;
         {
           float v[6][16];
@@ -437,7 +414,6 @@ scc_umma_kernel(const __grid_constant__ CUtensorMap tm_t, const __grid_constant_
         }
         fence_proxy_async_smem();
         mbar_arrive_warp(st_ready(s));
-        if (threadIdx.x == 128) SCC_T(15);
         ++d_cnt;
       }
       tok_cnt = a0 + (uint32_t)(mult * p.tiles);
@@ -519,7 +495,7 @@ size_t scc_bias_image_bytes(int w) { const SccTile g = scc_tile(w); return (size
 int launch_scc_images(const SccW& w, int win, int base, uint8_t* pool_img, uint8_t* bias_img, uint8_t* w_img, cudaStream_t st) {
   const SccTile g = scc_tile(win);
   const int pool_bytes = (g.TT > 64 ? g.TT / 64 : 1) * 8192;
-  {
+  if (pool_img != nullptr) {
     const long long total = (long long)g.tiles * (pool_bytes / 8192) * 4096;
     const int grid = (int)((total + 255) / 256 < 4096 ? (total + 255) / 256 : 4096);
     scc_pool_image_kernel<<<grid, 256, 0, st>>>(w.wsl, win, base, pool_img, pool_bytes);
@@ -536,7 +512,7 @@ int launch_scc_images(const SccW& w, int win, int base, uint8_t* pool_img, uint8
   return 0;
 }
 
-int launch_scc_umma(const bf16* t, const SccGeom& g, const SccW& w, bf16* out, float* dbg, int num_sms, cudaStream_t st) {
+int launch_scc_umma(const bf16* t, const SccGeom& g, const SccW& w, bf16* out, int num_sms, cudaStream_t st) {
   static unsigned long long configured = 0;
   if (ensure_dynamic_smem(scc_umma_kernel, kSmemBytes, &configured)) return 1;
   const SccTile tg = scc_tile(g.w);
@@ -553,7 +529,6 @@ int launch_scc_umma(const bf16* t, const SccGeom& g, const SccW& w, bf16* out, f
   p.bias_bytes = tg.TT * 128;
   p.pool_img = w.pool_img; p.bias_img = w.bias_img; p.w_img = w.w_img; p.bsl = w.bsl_dev;
   p.H = g.pg.H; p.W = g.pg.W;
-  p.dbg = dbg;
   CUtensorMap tm_t, tm_o;
   if (make_tmap_nhwc(&tm_t, t, g.pg.B, g.pg.Hp, g.pg.Wp, kCp, 64, (uint32_t)tg.bx, (uint32_t)tg.by)) return 1;
   if (make_tmap_nhwc(&tm_o, out, g.pg.B, g.pg.H, g.pg.W, kCp, 64, (uint32_t)tg.bx, (uint32_t)tg.by)) return 1;

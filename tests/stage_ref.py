@@ -20,6 +20,7 @@ propagate the bound of their input as derived at `ln_bound` and `gelu_bound`.  N
 """
 from __future__ import annotations
 
+import math
 from dataclasses import dataclass
 
 import torch
@@ -682,6 +683,12 @@ def fusion(cab, shallow, sd, ar: Arith, mut=()):
 HEADS, HD = 6, 15
 
 
+def _pool_geom(P, win: int):
+    """(pooled grid side, pooling ratio r) of a window, read off spatial_linear = Linear(r^2, 1): base = min(w, base_win_size)."""
+    r = math.isqrt(P["spatial_linear.weight"].numel())
+    return win // r, r
+
+
 def _scc_operands(P, win: int, ar: Arith, mut=()):
     """The weight operands of both SCC kernels: the k-gen image (`scc_w_image_kernel`) holds bf16(0.5 w1), bf16(0.5 w2) and
     bf16(0.5 (b1 + b2)) (fp32 sum, on the ones column of each head's q slice); the pool weights are a bf16 operand image when r > 1
@@ -696,8 +703,7 @@ def _scc_operands(P, win: int, ar: Arith, mut=()):
         bk = torch.zeros_like(bk)
     W1x = torch.cat([ar.op(0.5 * w1.float()), ar.op(bk)[:, None]], 1)
     W2 = ar.op(0.5 * w2.float())
-    base = min(win, 8)
-    r = win // base
+    base, r = _pool_geom(P, win)
     wsl = P["spatial_linear.weight"].reshape(-1)
     wsl = ar.op(wsl) if r > 1 else ar.f32(wsl)
     ly, lx = torch.div(torch.arange(win * win), win, rounding_mode="floor"), torch.arange(win * win) % win
@@ -831,8 +837,7 @@ def scc(tok, bias, P, win: int, ar: Arith, hw, mut=()):
     and one bf16 ulp of the stored output.  Mutants of SIM: "no_bsl_vpt", "no_bsl_kp", "scale16", "inv_lb", "kgen_swapped",
     "no_ones", "bias_transposed" (scc_dense: the L x L table read (m, l)), "bias_xy" (scc_umma: the L x Lb table's token rows read
     with x and y exchanged -- an (m, l) read of a non-square table is not a plausible kernel bug)."""
-    base = min(win, 8)
-    r = win // base
+    base, r = _pool_geom(P, win)
     if ar is SIM:
         out_s, out_c = (_scc_dense_sim if r == 1 else _scc_umma_sim)(tok, bias, P, win, mut)
     else:

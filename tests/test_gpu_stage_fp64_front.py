@@ -27,8 +27,8 @@ SHAPES = {"trunk": (2, 98, 146), "small": (1, 37, 53)}
 WINDOWS = (4, 8, 16, 32, 48, 64)
 
 
-def make_model(flags=(1, 1, 1), edit=None):
-    model, oracle = build_pair(flags, "nearest+conv", 4, "stress", 21, edit=edit)
+def make_model(flags=(1, 1, 1), edit=None, **extra):
+    model, oracle = build_pair(flags, "nearest+conv", 4, "stress", 21, edit=edit, **extra)
     return model.to(DEV), oracle.sd
 
 
@@ -83,6 +83,16 @@ def test_scc_common_mode(j):
         check_scc(model, sd, x, j, "casa off, +64")
     finally:
         model.set_inject(DEV, None)
+
+
+@pytest.mark.parametrize("base,j", [(4, 1), (4, 2), (2, 0), (2, 1)])
+def test_scc_pooled_base(base, j):
+    """base_win_size below 8, windows 4..64 as in the pro model: the w = 4 / 8 windows pool inside their one token tile and run
+    `scc_umma`'s resident mode (base 4: w = 8 at r = 2; base 2: w = 4 at r = 2, w = 8 at r = 4); base 4, w = 16 runs the two-tile
+    mode over 16 pooled cells (one cell k-step)."""
+    model, sd = make_model(base_win_size=[base, base], hier_win_ratios=[w / base for w in WINDOWS])
+    B, H, W = SHAPES["trunk"]
+    check_scc(model, sd, synthetic_image(B, H, W, seed=4).to(DEV), j, f"base_win_size {base}")
 
 
 # ---- casa gate --------------------------------------------------------------------------------------------------------------
