@@ -168,6 +168,9 @@ HITSIR_API int hitsir_forward_x8_u8(HitsirHandle* h, const uint8_t* x_hwc, uint8
  * an fp32 NCHW batch [B,C,H,W] into uint8 HWC [B,H,W,C], both on the device.  Used before the multi-GPU output gather: a quarter of
  * the fp32 bytes cross NVLink.  Needs no handle; asynchronous on `stream`. */
 HITSIR_API int hitsir_f32nchw_to_u8hwc(const float* src, uint8_t* dst, int B, int C, int H, int W, void* stream);
+/* The same with BasicSR's tensor2img rounding (basicsr/utils/img_util.py, uint8 output): clip(0,1), value * 255 in fp32, rounded half
+ * to even, of an fp32 NCHW batch [B,C,H,W] into uint8 HWC [B,H,W,C].  Needs no handle; asynchronous on `stream`. */
+HITSIR_API int hitsir_f32nchw_to_u8hwc_round(const float* src, uint8_t* dst, int B, int C, int H, int W, void* stream);
 
 /* The entry conversion alone, the mirror of hitsir_f32nchw_to_u8hwc: torchvision's to_tensor (utils/utils.py:143-145: value / 255 in
  * fp32) of a uint8 HWC batch [B,H,W,C] into fp32 NCHW [B,C,H,W], both on the device; the conversion hitsir_forward_u8 applies to its
@@ -222,6 +225,28 @@ HITSIR_API int hitsir_psnr_y(const float* sr, const float* hr, int B, int H, int
 HITSIR_API int64_t hitsir_ssim_y_scratch_doubles(int B, int H, int W, int gaussian);
 HITSIR_API int hitsir_ssim_y(const float* sr, const float* hr, int B, int H, int W, int clip_sr, int gaussian, int sample_cov,
                   double* scratch, double* ssim_out, void* stream);
+
+/* The metrics of published SR tables: BasicSR 1.4.2's calculate_psnr and calculate_ssim (basicsr/metrics/psnr_ssim.py, with
+ * to_y_channel of basicsr/metrics/metric_util.py and bgr2ycbcr of basicsr/utils/color_util.py) of two uint8 RGB HWC batches
+ * [B,H,W,3] on the device (SR rounded to uint8 first, as tensor2img does: hitsir_f32nchw_to_u8hwc_round).
+ *   crop:   crop_border pixels are dropped on every side (none when 0).
+ *   planes: y_only != 0 -> one plane, BasicSR's Y on the 0-255 scale: t = fp32(v) / 255 (fp32), y = ((24.966 t_B + 128.553 t_G)
+ *           + 65.481 t_R) + 16 (double), Y = fp32(fp32(y / 255) * 255); y_only == 0 -> the three colour channels.
+ *   mse_out[b] = the mean over every kept value of (sr - hr)^2 in double: PSNR_b = 10 log10(255^2 / mse_out[b]), +inf when 0.  In RGB
+ *           mode the squares are integers summed exactly, so mse_out equals numpy's bit for bit.
+ *   ssim_out[b] = per plane, the mean over the valid region [5, Hc-5) x [5, Wc-5) of the crop of
+ *           S = ((2 mu1 mu2 + c1)(2 s12 + c2)) / ((mu1^2 + mu2^2 + c1)(s11 + s22 + c2)),  c1 = (0.01 * 255)^2, c2 = (0.03 * 255)^2,
+ *           with window means under outer(k, k), k = cv2.getGaussianKernel(11, 1.5), and s = E[ab] - mu_a mu_b; then the mean of the
+ *           planes in BasicSR's BGR order ((B + G) + R) / 3.  Double throughout; direct (separable) window sums rather than
+ *           cv2.filter2D's DFT, so within a derived per-image bound of BasicSR (1e-13 to 1e-11) rather than bit-exact;
+ *           ssim(x, x) is exactly 1.
+ * Null pointers, B outside 1..65535, crop_border < 0 and H - 2 crop_border < 11 or W - 2 crop_border < 11 (BasicSR returns nan with a
+ * warning) are HITSIR_ERR_INVALID.  `scratch`: device buffer of hitsir_basicsr_metrics_scratch_doubles(B,H,W,crop_border,y_only) doubles
+ * (0 for arguments the entry refuses).  No host copy (graph-capturable), fixed-order reduction (bitwise reproducible, independent of the
+ * other images of the batch); asynchronous on `stream`; needs no handle. */
+HITSIR_API int64_t hitsir_basicsr_metrics_scratch_doubles(int B, int H, int W, int crop_border, int y_only);
+HITSIR_API int hitsir_psnr_ssim_basicsr(const uint8_t* sr_hwc, const uint8_t* hr_hwc, int B, int H, int W, int crop_border, int y_only,
+                             double* scratch, double* mse_out, double* ssim_out, void* stream);
 
 /* Test hook standing in for PyTorch forward hooks on reference sub-modules: the next
  * hitsir_forward copies the named intermediate activation (fp32, NHWC, real channels only) into

@@ -11,9 +11,9 @@ from .hit_sir_pro import HiT_SIR, PRO_KWARGS  # noqa: F401
 from . import _capi  # noqa: F401
 from .sharding import ShardedSR, PeerGather, tile_plan, stitch_tiles  # noqa: F401
 from .host_pipeline import HostPipeline  # noqa: F401
-from .metrics import mse_y, psnr_y, ssim_y, to_uint8_hwc  # noqa: F401
+from .metrics import mse_y, psnr_y, ssim_y, psnr_ssim_basicsr, to_uint8_hwc  # noqa: F401
 from .resize import resize_bicubic, to_float_nchw, evaluate  # noqa: F401
 from .graphed import GraphedForward  # noqa: F401
 from .banded import BandedSR, LocalBandedSR, band_plan  # noqa: F401
 
-__all__ = ["HiT_SIR", "PRO_KWARGS", "ShardedSR", "tile_plan", "stitch_tiles", "HostPipeline", "mse_y", "psnr_y", "ssim_y", "to_uint8_hwc", "resize_bicubic", "to_float_nchw", "evaluate", "GraphedForward", "BandedSR", "LocalBandedSR", "band_plan", "PeerGather"]
+__all__ = ["HiT_SIR", "PRO_KWARGS", "ShardedSR", "tile_plan", "stitch_tiles", "HostPipeline", "mse_y", "psnr_y", "ssim_y", "psnr_ssim_basicsr", "to_uint8_hwc", "resize_bicubic", "to_float_nchw", "evaluate", "GraphedForward", "BandedSR", "LocalBandedSR", "band_plan", "PeerGather"]

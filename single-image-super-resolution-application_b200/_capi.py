@@ -74,7 +74,11 @@ SYMBOLS = {
     "hitsir_forward_x8_u8": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_size_t,
                                        C.c_void_p]),
     "hitsir_f32nchw_to_u8hwc": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p]),
-    "hitsir_psnr_y_scratch_doubles": (C.c_int64, [C.c_int, C.c_int, C.c_int]),
+    "hitsir_f32nchw_to_u8hwc_round": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p]),
+    "hitsir_basicsr_metrics_scratch_doubles": (C.c_int64, [C.c_int, C.c_int, C.c_int, C.c_int, C.c_int]),
+    "hitsir_psnr_ssim_basicsr": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p,
+                                           C.c_void_p, C.c_void_p]),
+    "hitsir_psnr_y_scratch_doubles":(C.c_int64, [C.c_int, C.c_int, C.c_int]),
     "hitsir_psnr_y": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p]),
     "hitsir_ssim_y_scratch_doubles": (C.c_int64, [C.c_int, C.c_int, C.c_int, C.c_int]),
     "hitsir_ssim_y": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p,

@@ -1306,6 +1306,12 @@ HITSIR_API int hitsir_f32nchw_to_u8hwc(const float* src, uint8_t* dst, int B, in
   return 0;
 }
 
+HITSIR_API int hitsir_f32nchw_to_u8hwc_round(const float* src, uint8_t* dst, int B, int C, int H, int W, void* stream) {
+  if (!src || !dst || B <= 0 || C <= 0 || H <= 0 || W <= 0) { set_error("hitsir_f32nchw_to_u8hwc_round: bad argument"); return HITSIR_ERR_INVALID; }
+  if (launch_f32nchw_to_u8hwc_round(src, dst, B, H, W, C, (cudaStream_t)stream)) return HITSIR_ERR_CUDA;
+  return 0;
+}
+
 HITSIR_API int hitsir_u8hwc_to_f32nchw(const uint8_t* src, float* dst, int B, int C, int H, int W, void* stream) {
   if (!src || !dst || B <= 0 || C <= 0 || H <= 0 || W <= 0) { set_error("hitsir_u8hwc_to_f32nchw: bad argument"); return HITSIR_ERR_INVALID; }
   if (launch_u8hwc_to_f32nchw(src, dst, B, H, W, C, (cudaStream_t)stream)) return HITSIR_ERR_CUDA;
@@ -1375,6 +1381,19 @@ HITSIR_API int hitsir_ssim_y(const float* sr, const float* hr, int B, int H, int
     return HITSIR_ERR_INVALID;
   }
   if (launch_ssim_y(sr, hr, B, H, W, clip_sr, gaussian, sample_cov, scratch, ssim_out, (cudaStream_t)stream)) return HITSIR_ERR_CUDA;
+  return 0;
+}
+
+HITSIR_API int64_t hitsir_basicsr_metrics_scratch_doubles(int B, int H, int W, int crop_border, int y_only) {
+  if (basicsr_metrics_check(B, H, W, crop_border)) return 0;
+  return basicsr_metrics_scratch_doubles(B, H, W, crop_border, y_only);
+}
+
+HITSIR_API int hitsir_psnr_ssim_basicsr(const uint8_t* sr_hwc, const uint8_t* hr_hwc, int B, int H, int W, int crop_border, int y_only,
+                                        double* scratch, double* mse_out, double* ssim_out, void* stream) {
+  if (!sr_hwc || !hr_hwc || !scratch || !mse_out || !ssim_out) { set_error("hitsir_psnr_ssim_basicsr: null argument"); return HITSIR_ERR_INVALID; }
+  if (basicsr_metrics_check(B, H, W, crop_border)) return HITSIR_ERR_INVALID;
+  if (launch_psnr_ssim_basicsr(sr_hwc, hr_hwc, B, H, W, crop_border, y_only, scratch, mse_out, ssim_out, (cudaStream_t)stream)) return HITSIR_ERR_CUDA;
   return 0;
 }
 

@@ -94,13 +94,15 @@ __global__ void u8hwc_to_f32nchw_kernel(const uint8_t* __restrict__ in, float* _
     out[i] = (float)in[(((long long)b * H + y) * W + x) * C + c] / 255.0f;
   }
 }
-// fp32 NCHW -> clip(0,1) (experiments/experiment.py:746-748, test_experiment.py:75) -> uint8 HWC with to_pil_image's mul(255).byte() truncation
+// fp32 NCHW -> clip(0,1) (experiments/experiment.py:746-748, test_experiment.py:75) -> uint8 HWC with to_pil_image's mul(255).byte() truncation,
+// or (Round) with BasicSR's tensor2img (basicsr/utils/img_util.py): (v * 255.0).round() in fp32, half to even
+template <bool Round>
 __global__ void f32nchw_to_u8hwc_kernel(const float* __restrict__ in, uint8_t* __restrict__ out, int B, int H, int W, int C) {
   const long long total = (long long)B * H * W * C;
   for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (long long)gridDim.x * blockDim.x) {
     const int c = (int)(i % C); long long t = i / C; const int x = (int)(t % W); t /= W; const int y = (int)(t % H); const int b = (int)(t / H);
     const float v = fminf(fmaxf(in[(((long long)b * C + c) * H + y) * W + x], 0.f), 1.f);
-    out[i] = (uint8_t)(v * 255.0f);
+    out[i] = Round ? (uint8_t)rintf(__fmul_rn(v, 255.0f)) : (uint8_t)(v * 255.0f);
   }
 }
 
@@ -671,7 +673,12 @@ int launch_u8hwc_to_f32nchw(const uint8_t* in, float* out, int B, int H, int W, 
   return 0;
 }
 int launch_f32nchw_to_u8hwc(const float* in, uint8_t* out, int B, int H, int W, int C, cudaStream_t st) {
-  f32nchw_to_u8hwc_kernel<<<grid_for((long long)B * C * H * W, 256), 256, 0, st>>>(in, out, B, H, W, C);
+  f32nchw_to_u8hwc_kernel<false><<<grid_for((long long)B * C * H * W, 256), 256, 0, st>>>(in, out, B, H, W, C);
+  HITSIR_CHECK(cudaGetLastError());
+  return 0;
+}
+int launch_f32nchw_to_u8hwc_round(const float* in, uint8_t* out, int B, int H, int W, int C, cudaStream_t st) {
+  f32nchw_to_u8hwc_kernel<true><<<grid_for((long long)B * C * H * W, 256), 256, 0, st>>>(in, out, B, H, W, C);
   HITSIR_CHECK(cudaGetLastError());
   return 0;
 }

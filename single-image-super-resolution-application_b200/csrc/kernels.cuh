@@ -44,6 +44,8 @@ int launch_psnr_y(const float* sr, const float* hr, int B, int H, int W, int cli
 // uint8 HWC <-> fp32 NCHW entry / exit (to_tensor: /255; clip(0,1) then to_pil_image: *255 truncated)
 int launch_u8hwc_to_f32nchw(const uint8_t* in, float* out, int B, int H, int W, int C, cudaStream_t st);
 int launch_f32nchw_to_u8hwc(const float* in, uint8_t* out, int B, int H, int W, int C, cudaStream_t st);
+// the same with BasicSR's tensor2img rounding: clip(0,1), fp32 * 255, round half to even
+int launch_f32nchw_to_u8hwc_round(const float* in, uint8_t* out, int B, int H, int W, int C, cudaStream_t st);
 // perm != 0: column c is read from the head-padded position scc_pos(c)
 int launch_f32_to_f32_tap(const void* src, int src_is_bf16, int ld_src, float* dst, long long rows, int cols, int perm, cudaStream_t st);
 // out_bf16[N,192] = bf16(a) (pad 0): GEMM operand shadow of the fp32 stream
@@ -66,6 +68,12 @@ long long ssim_y_tiles(int H, int W, int gaussian);
 // partial: B * ssim_y_tiles doubles; ssim[b] = mean of the SSIM map over the interior of image b
 int launch_ssim_y(const float* sr, const float* hr, int B, int H, int W, int clip, int gaussian, int sample_cov, double* partial, double* ssim,
                   cudaStream_t st);
+// BasicSR 1.4.2's calculate_psnr / calculate_ssim of two uint8 RGB HWC batches (crop_border, test_y_channel = y_only).
+// basicsr_metrics_check: 0 when B, the shape and the crop are supported, else 1 with the error message set.
+int basicsr_metrics_check(int B, int H, int W, int crop);
+long long basicsr_metrics_scratch_doubles(int B, int H, int W, int crop, int y_only);
+int launch_psnr_ssim_basicsr(const uint8_t* sr, const uint8_t* hr, int B, int H, int W, int crop, int y_only, double* scratch, double* mse,
+                             double* ssim, cudaStream_t st);
 
 // ---- resize.cu (bicubic resizing: Pillow's Image.resize(BICUBIC) on uint8 HWC, MATLAB imresize as BasicSR computes it on fp32 NCHW) ----
 // 0 when the shapes (and scale, matlab) are within what the kernel supports, else 1 with the error message set

@@ -4,7 +4,9 @@
 (`utils/utils.py:170-186`) and calls `skimage.metrics.peak_signal_noise_ratio(hr_y, sr_y, data_range=1)` on the CPU, image by
 image.  `psnr_y` does the same arithmetic in one fused CUDA pass over the two batches (C ABI `hitsir_psnr_y`), so evaluation
 never copies the SR images to the host.  `ssim_y` does the same for the second score, `skimage.metrics.structural_similarity(hr_y,
-sr_y, data_range=1)` (:575-640), in one fused CUDA pass plus a fixed-order reduction (C ABI `hitsir_ssim_y`).  There is no CPU path.
+sr_y, data_range=1)` (:575-640), in one fused CUDA pass plus a fixed-order reduction (C ABI `hitsir_ssim_y`).  `psnr_ssim_basicsr`
+scores by the other convention, BasicSR's `calculate_psnr` / `calculate_ssim` on rounded uint8 images, which published SR tables use.
+There is no CPU path.
 """
 from __future__ import annotations
 
@@ -69,16 +71,54 @@ def ssim_y(sr: torch.Tensor, hr: torch.Tensor, clip: bool = True, gaussian_weigh
     return out
 
 
-def to_uint8_hwc(y: torch.Tensor) -> torch.Tensor:
+def psnr_ssim_basicsr(sr_u8: torch.Tensor, hr_u8: torch.Tensor, crop_border: int, test_y_channel: bool = True):
+    """BasicSR 1.4.2's `calculate_psnr` and `calculate_ssim` (basicsr/metrics/psnr_ssim.py), the scores of published SR tables, of
+    every image of two uint8 (B,H,W,3) RGB CUDA batches, on the device (C ABI `hitsir_psnr_ssim_basicsr`).
+
+    `crop_border` pixels are dropped on every side (BasicSR passes the scale factor); `test_y_channel` scores BasicSR's Y on the 0-255
+    scale, else the three colour channels.  SSIM is the 11x11 Gaussian (sigma 1.5) window over the valid region, in float64.  Round an
+    fp32 SR batch as BasicSR's `tensor2img` does first: ``to_uint8_hwc(sr, rounding="nearest")``.  Returns ``(psnr, ssim)``, float64
+    (B,) CUDA tensors; psnr = 10 log10(255^2 / mse), +inf for identical images."""
+    if sr_u8.device.type != "cuda" or hr_u8.device != sr_u8.device:
+        raise RuntimeError("psnr_ssim_basicsr expects CUDA tensors on the same device: there is no CPU path.")
+    if sr_u8.dtype != torch.uint8 or hr_u8.dtype != torch.uint8:
+        raise ValueError(f"psnr_ssim_basicsr takes uint8 images, got {sr_u8.dtype} and {hr_u8.dtype}")
+    if sr_u8.dim() != 4 or sr_u8.shape[3] != 3 or sr_u8.shape != hr_u8.shape:
+        raise ValueError(f"expected two (B,H,W,3) batches of the same shape, got {tuple(sr_u8.shape)} and {tuple(hr_u8.shape)}")
+    c = int(crop_border)
+    B, H, W, _ = sr_u8.shape
+    if B == 0 or c < 0 or H - 2 * c < 11 or W - 2 * c < 11:
+        raise ValueError(f"psnr_ssim_basicsr needs a non-empty batch, crop_border >= 0 and images of at least 11x11 after the crop, "
+                         f"got {tuple(sr_u8.shape)} with crop_border={c}")
+    sr_u8 = sr_u8.contiguous()
+    hr_u8 = hr_u8.contiguous()
+    y = 1 if test_y_channel else 0
+    lib = _capi.load()
+    with torch.cuda.device(sr_u8.device):
+        stream = torch.cuda.current_stream(sr_u8.device).cuda_stream
+        scratch = torch.empty(int(lib.hitsir_basicsr_metrics_scratch_doubles(B, H, W, c, y)), dtype=torch.float64, device=sr_u8.device)
+        mse = torch.empty(B, dtype=torch.float64, device=sr_u8.device)
+        ssim = torch.empty(B, dtype=torch.float64, device=sr_u8.device)
+        _capi.check(lib.hitsir_psnr_ssim_basicsr(ctypes.c_void_p(sr_u8.data_ptr()), ctypes.c_void_p(hr_u8.data_ptr()), B, H, W, c, y,
+                                                 ctypes.c_void_p(scratch.data_ptr()), ctypes.c_void_p(mse.data_ptr()),
+                                                 ctypes.c_void_p(ssim.data_ptr()), ctypes.c_void_p(stream)))
+    return 10.0 * torch.log10(65025.0 / mse), ssim
+
+
+def to_uint8_hwc(y: torch.Tensor, rounding: str = "truncate") -> torch.Tensor:
     """`to_pil_image(y.clip(0, 1))` of test_experiment.py:75-77 on the device: fp32 (B,C,H,W) -> uint8 (B,H,W,C), value * 255 truncated
-    (C ABI `hitsir_f32nchw_to_u8hwc`).  The multi-GPU output gather moves this form: a quarter of the fp32 bytes."""
+    (C ABI `hitsir_f32nchw_to_u8hwc`).  The multi-GPU output gather moves this form: a quarter of the fp32 bytes.
+    ``rounding="nearest"`` rounds half to even instead, as BasicSR's `tensor2img` does before its metrics (`hitsir_f32nchw_to_u8hwc_round`)."""
+    if rounding not in ("truncate", "nearest"):
+        raise ValueError(f"to_uint8_hwc: rounding must be 'truncate' or 'nearest', got {rounding!r}")
     if y.device.type != "cuda" or y.dim() != 4:
         raise RuntimeError("to_uint8_hwc expects a (B,C,H,W) CUDA tensor: there is no CPU path.")
     y = y.contiguous().float()
     B, C, H, W = y.shape
     out = torch.empty((B, H, W, C), dtype=torch.uint8, device=y.device)
+    lib = _capi.load()
+    fn = lib.hitsir_f32nchw_to_u8hwc if rounding == "truncate" else lib.hitsir_f32nchw_to_u8hwc_round
     with torch.cuda.device(y.device):
         stream = torch.cuda.current_stream(y.device).cuda_stream
-        _capi.check(_capi.load().hitsir_f32nchw_to_u8hwc(ctypes.c_void_p(y.data_ptr()), ctypes.c_void_p(out.data_ptr()), B, C, H, W,
-                                                          ctypes.c_void_p(stream)))
+        _capi.check(fn(ctypes.c_void_p(y.data_ptr()), ctypes.c_void_p(out.data_ptr()), B, C, H, W, ctypes.c_void_p(stream)))
     return out

@@ -19,7 +19,7 @@ from typing import Dict, Optional, Sequence
 import torch
 
 from . import _capi
-from .metrics import psnr_y, ssim_y
+from .metrics import psnr_ssim_basicsr, psnr_y, ssim_y, to_uint8_hwc
 
 
 def to_float_nchw(x_u8: torch.Tensor) -> torch.Tensor:
@@ -87,16 +87,30 @@ def resize_bicubic(x: torch.Tensor, size: Optional[Sequence[int]] = None, scale:
 
 
 def evaluate(model, hr_u8: torch.Tensor, lr_kernel: str = "pil", self_ensemble: bool = False, bicubic_baseline: bool = False,
-             gaussian_weights: bool = False, use_sample_covariance: bool = True) -> Dict[str, torch.Tensor]:
+             gaussian_weights: Optional[bool] = None, use_sample_covariance: Optional[bool] = None, protocol: str = "skimage",
+             crop_border: Optional[int] = None, lr_u8: Optional[torch.Tensor] = None) -> Dict[str, torch.Tensor]:
     """Score `model` on a batch of HR images without leaving the device: the loop of experiments/experiment.py:681-790.
 
     `hr_u8`: uint8 (B,H,W,3) CUDA images, H and W multiples of ``model.upscale`` (crop by slicing first).  HR is
     ``to_float_nchw(hr_u8)``; the LR is the Pillow resize of `hr_u8` converted the same way (``lr_kernel="pil"``) or
-    ``resize_bicubic(hr, scale=1/upscale, kernel="matlab")`` kept in fp32 (``lr_kernel="matlab"``).  SR is ``model(lr)`` (or
-    ``model.forward_x8(lr)``), clipped to [0, 1] by the metrics.  Returns ``{"psnr_y", "ssim_y"}``, float64 (B,) CUDA tensors, plus
-    ``"bicubic_psnr_y"`` / ``"bicubic_ssim_y"`` with `bicubic_baseline`: the LR upscaled back to H x W by the same bicubic."""
+    ``resize_bicubic(hr, scale=1/upscale, kernel="matlab")`` kept in fp32 (``lr_kernel="matlab"``); or, when given, `lr_u8`: uint8
+    (B,H/upscale,W/upscale,3) LR images such as the MATLAB-made ones benchmark sets ship, converted by ``to_float_nchw``.  SR is
+    ``model(lr)`` (or ``model.forward_x8(lr)``).  With `bicubic_baseline`, the LR is also upscaled back to H x W by the `lr_kernel`
+    bicubic and scored the same way.
+
+    ``protocol="skimage"`` (the reference harness): SR clipped to [0, 1] by the metrics, ``psnr_y`` and ``ssim_y`` with
+    `gaussian_weights` / `use_sample_covariance` (default False / True).  ``protocol="basicsr"`` (published SR tables):
+    ``to_uint8_hwc(sr, rounding="nearest")`` scored by ``psnr_ssim_basicsr(., hr_u8, crop_border, test_y_channel=True)``,
+    `crop_border` defaulting to ``upscale``.  Returns ``{"psnr_y", "ssim_y"}``, float64 (B,) CUDA tensors, plus
+    ``"bicubic_psnr_y"`` / ``"bicubic_ssim_y"`` with `bicubic_baseline`."""
     if lr_kernel not in ("pil", "matlab"):
         raise ValueError(f"evaluate: lr_kernel must be 'pil' or 'matlab', got {lr_kernel!r}")
+    if protocol not in ("skimage", "basicsr"):
+        raise ValueError(f"evaluate: protocol must be 'skimage' or 'basicsr', got {protocol!r}")
+    if protocol == "basicsr" and (gaussian_weights is not None or use_sample_covariance is not None):
+        raise ValueError("evaluate: gaussian_weights / use_sample_covariance are skimage options; protocol='basicsr' fixes its window")
+    if protocol == "skimage" and crop_border is not None:
+        raise ValueError("evaluate: crop_border applies to protocol='basicsr' only; the skimage protocol scores the whole image")
     if hr_u8.device.type != "cuda" or hr_u8.dtype != torch.uint8 or hr_u8.dim() != 4 or hr_u8.shape[3] != 3:
         raise ValueError(f"evaluate expects uint8 (B,H,W,3) CUDA images, got {hr_u8.dtype} {tuple(hr_u8.shape)} on {hr_u8.device}")
     s = int(model.upscale)
@@ -105,21 +119,32 @@ def evaluate(model, hr_u8: torch.Tensor, lr_kernel: str = "pil", self_ensemble: 
     B, H, W, _ = hr_u8.shape
     if H % s or W % s:
         raise ValueError(f"evaluate: H and W must be multiples of upscale={s}, got {H} x {W}; crop the HR images first")
+    c = s if crop_border is None else int(crop_border)
+    if protocol == "basicsr" and (c < 0 or H - 2 * c < 11 or W - 2 * c < 11):
+        raise ValueError(f"evaluate: crop_border={c} leaves less than the 11x11 SSIM window of {H} x {W} images")
     hr = to_float_nchw(hr_u8)
-    if lr_kernel == "pil":
+    if lr_u8 is not None:
+        if lr_u8.dtype != torch.uint8 or lr_u8.device != hr_u8.device or tuple(lr_u8.shape) != (B, H // s, W // s, 3):
+            raise ValueError(f"evaluate: lr_u8 must be uint8 {(B, H // s, W // s, 3)} on {hr_u8.device}, got {lr_u8.dtype} "
+                             f"{tuple(lr_u8.shape)} on {lr_u8.device}")
+        lr = to_float_nchw(lr_u8)
+    elif lr_kernel == "pil":
         lr_u8 = resize_bicubic(hr_u8, size=(H // s, W // s), kernel="pil")
         lr = to_float_nchw(lr_u8)
     else:
         lr = resize_bicubic(hr, scale=1.0 / s, kernel="matlab")
     with torch.no_grad():
         sr = model.forward_x8(lr) if self_ensemble else model(lr)
-    kw = dict(gaussian_weights=gaussian_weights, use_sample_covariance=use_sample_covariance)
-    out = {"psnr_y": psnr_y(sr, hr), "ssim_y": ssim_y(sr, hr, **kw)}
+    if protocol == "skimage":
+        kw = dict(gaussian_weights=bool(gaussian_weights), use_sample_covariance=use_sample_covariance is None or bool(use_sample_covariance))
+        score = lambda y: (psnr_y(y, hr), ssim_y(y, hr, **kw))     # noqa: E731
+    else:
+        score = lambda y: psnr_ssim_basicsr(to_uint8_hwc(y, rounding="nearest"), hr_u8, c, test_y_channel=True)     # noqa: E731
+    out = dict(zip(("psnr_y", "ssim_y"), score(sr)))
     if bicubic_baseline:
         if lr_kernel == "pil":
             up = to_float_nchw(resize_bicubic(lr_u8, size=(H, W), kernel="pil"))
         else:
             up = resize_bicubic(lr, scale=float(s), kernel="matlab")
-        out["bicubic_psnr_y"] = psnr_y(up, hr)
-        out["bicubic_ssim_y"] = ssim_y(up, hr, **kw)
+        out["bicubic_psnr_y"], out["bicubic_ssim_y"] = score(up)
     return out
