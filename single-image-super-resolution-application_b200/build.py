@@ -19,7 +19,7 @@ CSRC = os.path.join(HERE, "csrc")
 BUILD = os.path.join(HERE, "build")
 LIB = os.path.join(HERE, "libhitsir_b200.so")
 SOURCES = ["engine.cu", "umma_gemm.cu", "umma_gemm_tma.cu", "proj_fc1.cu", "conv3_c64.cu", "ffn_tail.cu", "scc_umma.cu", "scc_dense.cu", "glue.cu", "pack.cu",
-           "ensemble.cu", "ssim.cu", "resize.cu"]
+           "ensemble.cu", "metrics.cu", "resize.cu"]
 HEADERS = ["common.cuh", "gemm.cuh", "kernels.cuh", "ycbcr.cuh", os.path.join("..", "..", "include", "hitsir_b200.h")]
 NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
 FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",

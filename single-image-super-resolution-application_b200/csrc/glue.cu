@@ -4,7 +4,6 @@
 // gating, nearest upsampling.  Token-major (NHWC) throughout; 128-bit accesses where rows allow.
 #include "gemm.cuh"
 #include "kernels.cuh"
-#include "ycbcr.cuh"
 
 namespace hitsir {
 
@@ -104,47 +103,6 @@ __global__ void f32nchw_to_u8hwc_kernel(const float* __restrict__ in, uint8_t* _
     const float v = fminf(fmaxf(in[(((long long)b * C + c) * H + y) * W + x], 0.f), 1.f);
     out[i] = Round ? (uint8_t)rintf(__fmul_rn(v, 255.0f)) : (uint8_t)(v * 255.0f);
   }
-}
-
-// Evaluation metric on the device (experiments/experiment.py:436-463): Y channel of both [0,1] RGB batches exactly as
-// utils/utils.py:170-186 writes it (y_channel, ycbcr.cuh), then the squared fp32 difference accumulated in double (skimage
-// mean_squared_error: float32 squares, float64 mean).  Two fixed-order levels (thread -> warp tree -> CTA partial -> per-image sum):
-// bitwise reproducible, no atomics.
-constexpr int kPsnrChunk = 4096;                           // pixels per CTA
-__global__ void __launch_bounds__(256) psnr_y_partial_kernel(const float* __restrict__ sr, const float* __restrict__ hr, long long HW, int clip,
-                                                             double* __restrict__ partial) {
-  __shared__ double s_w[8];
-  const int b = blockIdx.y;
-  const float* s0 = sr + (long long)b * 3 * HW;
-  const float* h0 = hr + (long long)b * 3 * HW;
-  double acc = 0.0;
-  const long long base = (long long)blockIdx.x * kPsnrChunk;
-#pragma unroll 4
-  for (int i = 0; i < kPsnrChunk / 256; ++i) {
-    const long long px = base + threadIdx.x + 256 * i;
-    if (px < HW) {
-      float r = s0[px], g = s0[HW + px], bl = s0[2 * HW + px];
-      if (clip) { r = fminf(fmaxf(r, 0.f), 1.f); g = fminf(fmaxf(g, 0.f), 1.f); bl = fminf(fmaxf(bl, 0.f), 1.f); }   // sr_imgs.clip(0, 1) (:748)
-      const float d = __fsub_rn(y_channel(h0[px], h0[HW + px], h0[2 * HW + px]), y_channel(r, g, bl));
-      acc += (double)__fmul_rn(d, d);
-    }
-  }
-#pragma unroll
-  for (int o = 16; o > 0; o >>= 1) acc += __shfl_xor_sync(0xffffffffu, acc, o);
-  if ((threadIdx.x & 31) == 0) s_w[threadIdx.x >> 5] = acc;
-  __syncthreads();
-  if (threadIdx.x == 0) {
-    double t = 0.0;
-#pragma unroll
-    for (int w = 0; w < 8; ++w) t += s_w[w];
-    partial[(long long)b * gridDim.x + blockIdx.x] = t;
-  }
-}
-__global__ void psnr_y_final_kernel(const double* __restrict__ partial, int chunks, long long HW, double* __restrict__ mse) {
-  if (threadIdx.x != 0) return;
-  double t = 0.0;
-  for (int c = 0; c < chunks; ++c) t += partial[(long long)blockIdx.x * chunks + c];
-  mse[blockIdx.x] = t / (double)HW;
 }
 
 __global__ void tap_kernel(const void* src, int is_bf16, int ld, float* dst, long long rows, int cols, int perm) {
@@ -679,16 +637,6 @@ int launch_f32nchw_to_u8hwc(const float* in, uint8_t* out, int B, int H, int W, 
 }
 int launch_f32nchw_to_u8hwc_round(const float* in, uint8_t* out, int B, int H, int W, int C, cudaStream_t st) {
   f32nchw_to_u8hwc_kernel<true><<<grid_for((long long)B * C * H * W, 256), 256, 0, st>>>(in, out, B, H, W, C);
-  HITSIR_CHECK(cudaGetLastError());
-  return 0;
-}
-long long psnr_y_chunks(int H, int W) { return ((long long)H * W + kPsnrChunk - 1) / kPsnrChunk; }
-int launch_psnr_y(const float* sr, const float* hr, int B, int H, int W, int clip, double* partial, double* mse, cudaStream_t st) {
-  const long long HW = (long long)H * W, chunks = psnr_y_chunks(H, W);
-  if (chunks > 2147483647LL || B > 65535) { set_error("launch_psnr_y: image or batch too large"); return 1; }
-  psnr_y_partial_kernel<<<dim3((unsigned)chunks, (unsigned)B), 256, 0, st>>>(sr, hr, HW, clip, partial);
-  HITSIR_CHECK(cudaGetLastError());
-  psnr_y_final_kernel<<<B, 32, 0, st>>>(partial, (int)chunks, HW, mse);
   HITSIR_CHECK(cudaGetLastError());
   return 0;
 }

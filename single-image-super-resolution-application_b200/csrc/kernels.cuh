@@ -38,9 +38,6 @@ struct FfnBand { int halo, yg0, Hf; };
 int launch_ffn_tail(const bf16* h1, const uint32_t* dw_tbl_mma, const uint8_t* w2_img, const float* b2, const float* gamma,
                     const float* beta, float* x, int B, int H, int W, const FfnStats* stats, bf16* shadow, int num_sms, cudaStream_t st,
                     const FfnBand* band = nullptr);
-// per-image mean squared difference of the YCbCr Y channels of two [0,1] fp32 NCHW RGB batches (utils/utils.py:170-186, experiment.py:436-463)
-long long psnr_y_chunks(int H, int W);
-int launch_psnr_y(const float* sr, const float* hr, int B, int H, int W, int clip, double* partial, double* mse, cudaStream_t st);
 // uint8 HWC <-> fp32 NCHW entry / exit (to_tensor: /255; clip(0,1) then to_pil_image: *255 truncated)
 int launch_u8hwc_to_f32nchw(const uint8_t* in, float* out, int B, int H, int W, int C, cudaStream_t st);
 int launch_f32nchw_to_u8hwc(const float* in, uint8_t* out, int B, int H, int W, int C, cudaStream_t st);
@@ -61,7 +58,11 @@ int launch_x8_entry(const float* x, const uint8_t* x_u8hwc, float* xt, int B, in
 // first term; last: * 0.125f, and y_u8hwc != nullptr writes uint8 [B,Hd,Wd,C] as launch_f32nchw_to_u8hwc instead of acc
 int launch_x8_combine(const float* z, float* acc, uint8_t* y_u8hwc, int B, int C, int Hd, int Wd, int k0, int g, int first, int last, cudaStream_t st);
 
-// ---- ssim.cu (Y-channel SSIM of two [0,1] fp32 NCHW RGB batches, skimage structural_similarity(hr_y, sr_y, data_range=1)) ----
+// ---- metrics.cu (evaluation metrics of two batches, per image) ----
+// per-image mean squared difference of the YCbCr Y channels of two [0,1] fp32 NCHW RGB batches (utils/utils.py:170-186, experiment.py:436-463)
+long long psnr_y_chunks(int H, int W);
+int launch_psnr_y(const float* sr, const float* hr, int B, int H, int W, int clip, double* partial, double* mse, cudaStream_t st);
+// Y-channel SSIM of two [0,1] fp32 NCHW RGB batches, skimage structural_similarity(hr_y, sr_y, data_range=1)
 // window radius 3 (uniform 7x7) or 5 (Gaussian sigma 1.5, 11 taps); tiles per image of the interior, 0 when H or W < the window
 int ssim_y_radius(int gaussian);
 long long ssim_y_tiles(int H, int W, int gaussian);

@@ -1,5 +1,5 @@
-// Y channel of YCbCr as the reference evaluation computes it, shared by the metrics on the device (psnr_y in glue.cu, ssim_y in
-// ssim.cu): utils/utils.py:170-186 writes 16/255 + (65.738 R + 129.057 G + 25.064 B) / 256, every operation rounded to fp32 in that
+// Y channel of YCbCr as the reference evaluation computes it, shared by the metrics on the device (psnr_y and ssim_y in
+// metrics.cu): utils/utils.py:170-186 writes 16/255 + (65.738 R + 129.057 G + 25.064 B) / 256, every operation rounded to fp32 in that
 // order (no FMA contraction).
 #pragma once
 #include <cuda_runtime.h>

@@ -17,22 +17,35 @@ import torch
 from . import _capi
 
 
+def _check_pair(sr: torch.Tensor, hr: torch.Tensor, who: str, u8_hwc: bool = False) -> None:
+    """Raise unless `sr` and `hr` are CUDA tensors on one device with one shape: (B,3,H,W), or (B,H,W,3) and uint8 when `u8_hwc`.
+    `who` names the caller and its verb in the device error ("ssim_y expects")."""
+    if sr.device.type != "cuda" or hr.device != sr.device:
+        raise RuntimeError(f"{who} CUDA tensors on the same device: there is no CPU path.")
+    if u8_hwc and (sr.dtype != torch.uint8 or hr.dtype != torch.uint8):
+        raise ValueError(f"{who.split()[0]} takes uint8 images, got {sr.dtype} and {hr.dtype}")
+    layout, c = ("(B,H,W,3)", 3) if u8_hwc else ("(B,3,H,W)", 1)
+    if sr.dim() != 4 or sr.shape[c] != 3 or sr.shape != hr.shape:
+        raise ValueError(f"expected two {layout} batches of the same shape, got {tuple(sr.shape)} and {tuple(hr.shape)}")
+
+
+def _call(fn, device: torch.device, *args) -> None:
+    """Call the C ABI function `fn` on `device`, tensors passed by address and the current stream of `device` as the last argument."""
+    with torch.cuda.device(device):
+        stream = torch.cuda.current_stream(device).cuda_stream
+        _capi.check(fn(*[ctypes.c_void_p(a.data_ptr()) if isinstance(a, torch.Tensor) else a for a in args], ctypes.c_void_p(stream)))
+
+
 def mse_y(sr: torch.Tensor, hr: torch.Tensor, clip: bool = True) -> torch.Tensor:
     """Per-image mean squared difference of the Y channels, float64 CUDA tensor of shape (B,)."""
-    if sr.device.type != "cuda" or hr.device != sr.device:
-        raise RuntimeError("mse_y / psnr_y expect CUDA tensors on the same device: there is no CPU path.")
-    if sr.dim() != 4 or sr.shape[1] != 3 or sr.shape != hr.shape:
-        raise ValueError(f"expected two (B,3,H,W) batches of the same shape, got {tuple(sr.shape)} and {tuple(hr.shape)}")
+    _check_pair(sr, hr, "mse_y / psnr_y expect")
     sr = sr.contiguous().float()
     hr = hr.contiguous().float()
     B, _, H, W = sr.shape
     lib = _capi.load()
-    with torch.cuda.device(sr.device):
-        stream = torch.cuda.current_stream(sr.device).cuda_stream
-        scratch = torch.empty(int(lib.hitsir_psnr_y_scratch_doubles(B, H, W)), dtype=torch.float64, device=sr.device)
-        out = torch.empty(B, dtype=torch.float64, device=sr.device)
-        _capi.check(lib.hitsir_psnr_y(ctypes.c_void_p(sr.data_ptr()), ctypes.c_void_p(hr.data_ptr()), B, H, W, 1 if clip else 0,
-                                      ctypes.c_void_p(scratch.data_ptr()), ctypes.c_void_p(out.data_ptr()), ctypes.c_void_p(stream)))
+    scratch = torch.empty(int(lib.hitsir_psnr_y_scratch_doubles(B, H, W)), dtype=torch.float64, device=sr.device)
+    out = torch.empty(B, dtype=torch.float64, device=sr.device)
+    _call(lib.hitsir_psnr_y, sr.device, sr, hr, B, H, W, 1 if clip else 0, scratch, out)
     return out
 
 
@@ -47,10 +60,7 @@ def ssim_y(sr: torch.Tensor, hr: torch.Tensor, clip: bool = True, gaussian_weigh
     `structural_similarity(hr_y, sr_y, data_range=1, gaussian_weights=..., use_sample_covariance=...)` with `sr` clipped to [0, 1]
     first when `clip`.  Uniform 7x7 window by default; `gaussian_weights=True` takes the 11x11 Gaussian window (sigma 1.5).
     `gaussian_weights=True, use_sample_covariance=False` is the setting of Wang et al. that most papers report."""
-    if sr.device.type != "cuda" or hr.device != sr.device:
-        raise RuntimeError("ssim_y expects CUDA tensors on the same device: there is no CPU path.")
-    if sr.dim() != 4 or sr.shape[1] != 3 or sr.shape != hr.shape:
-        raise ValueError(f"expected two (B,3,H,W) batches of the same shape, got {tuple(sr.shape)} and {tuple(hr.shape)}")
+    _check_pair(sr, hr, "ssim_y expects")
     win = 11 if gaussian_weights else 7
     B, _, H, W = sr.shape
     if B == 0:
@@ -61,13 +71,9 @@ def ssim_y(sr: torch.Tensor, hr: torch.Tensor, clip: bool = True, gaussian_weigh
     hr = hr.contiguous().float()
     g = 1 if gaussian_weights else 0
     lib = _capi.load()
-    with torch.cuda.device(sr.device):
-        stream = torch.cuda.current_stream(sr.device).cuda_stream
-        scratch = torch.empty(int(lib.hitsir_ssim_y_scratch_doubles(B, H, W, g)), dtype=torch.float64, device=sr.device)
-        out = torch.empty(B, dtype=torch.float64, device=sr.device)
-        _capi.check(lib.hitsir_ssim_y(ctypes.c_void_p(sr.data_ptr()), ctypes.c_void_p(hr.data_ptr()), B, H, W, 1 if clip else 0, g,
-                                      1 if use_sample_covariance else 0, ctypes.c_void_p(scratch.data_ptr()),
-                                      ctypes.c_void_p(out.data_ptr()), ctypes.c_void_p(stream)))
+    scratch = torch.empty(int(lib.hitsir_ssim_y_scratch_doubles(B, H, W, g)), dtype=torch.float64, device=sr.device)
+    out = torch.empty(B, dtype=torch.float64, device=sr.device)
+    _call(lib.hitsir_ssim_y, sr.device, sr, hr, B, H, W, 1 if clip else 0, g, 1 if use_sample_covariance else 0, scratch, out)
     return out
 
 
@@ -79,12 +85,7 @@ def psnr_ssim_basicsr(sr_u8: torch.Tensor, hr_u8: torch.Tensor, crop_border: int
     scale, else the three colour channels.  SSIM is the 11x11 Gaussian (sigma 1.5) window over the valid region, in float64.  Round an
     fp32 SR batch as BasicSR's `tensor2img` does first: ``to_uint8_hwc(sr, rounding="nearest")``.  Returns ``(psnr, ssim)``, float64
     (B,) CUDA tensors; psnr = 10 log10(255^2 / mse), +inf for identical images."""
-    if sr_u8.device.type != "cuda" or hr_u8.device != sr_u8.device:
-        raise RuntimeError("psnr_ssim_basicsr expects CUDA tensors on the same device: there is no CPU path.")
-    if sr_u8.dtype != torch.uint8 or hr_u8.dtype != torch.uint8:
-        raise ValueError(f"psnr_ssim_basicsr takes uint8 images, got {sr_u8.dtype} and {hr_u8.dtype}")
-    if sr_u8.dim() != 4 or sr_u8.shape[3] != 3 or sr_u8.shape != hr_u8.shape:
-        raise ValueError(f"expected two (B,H,W,3) batches of the same shape, got {tuple(sr_u8.shape)} and {tuple(hr_u8.shape)}")
+    _check_pair(sr_u8, hr_u8, "psnr_ssim_basicsr expects", u8_hwc=True)
     c = int(crop_border)
     B, H, W, _ = sr_u8.shape
     if B == 0 or c < 0 or H - 2 * c < 11 or W - 2 * c < 11:
@@ -94,14 +95,10 @@ def psnr_ssim_basicsr(sr_u8: torch.Tensor, hr_u8: torch.Tensor, crop_border: int
     hr_u8 = hr_u8.contiguous()
     y = 1 if test_y_channel else 0
     lib = _capi.load()
-    with torch.cuda.device(sr_u8.device):
-        stream = torch.cuda.current_stream(sr_u8.device).cuda_stream
-        scratch = torch.empty(int(lib.hitsir_basicsr_metrics_scratch_doubles(B, H, W, c, y)), dtype=torch.float64, device=sr_u8.device)
-        mse = torch.empty(B, dtype=torch.float64, device=sr_u8.device)
-        ssim = torch.empty(B, dtype=torch.float64, device=sr_u8.device)
-        _capi.check(lib.hitsir_psnr_ssim_basicsr(ctypes.c_void_p(sr_u8.data_ptr()), ctypes.c_void_p(hr_u8.data_ptr()), B, H, W, c, y,
-                                                 ctypes.c_void_p(scratch.data_ptr()), ctypes.c_void_p(mse.data_ptr()),
-                                                 ctypes.c_void_p(ssim.data_ptr()), ctypes.c_void_p(stream)))
+    scratch = torch.empty(int(lib.hitsir_basicsr_metrics_scratch_doubles(B, H, W, c, y)), dtype=torch.float64, device=sr_u8.device)
+    mse = torch.empty(B, dtype=torch.float64, device=sr_u8.device)
+    ssim = torch.empty(B, dtype=torch.float64, device=sr_u8.device)
+    _call(lib.hitsir_psnr_ssim_basicsr, sr_u8.device, sr_u8, hr_u8, B, H, W, c, y, scratch, mse, ssim)
     return 10.0 * torch.log10(65025.0 / mse), ssim
 
 
@@ -117,8 +114,5 @@ def to_uint8_hwc(y: torch.Tensor, rounding: str = "truncate") -> torch.Tensor:
     B, C, H, W = y.shape
     out = torch.empty((B, H, W, C), dtype=torch.uint8, device=y.device)
     lib = _capi.load()
-    fn = lib.hitsir_f32nchw_to_u8hwc if rounding == "truncate" else lib.hitsir_f32nchw_to_u8hwc_round
-    with torch.cuda.device(y.device):
-        stream = torch.cuda.current_stream(y.device).cuda_stream
-        _capi.check(fn(ctypes.c_void_p(y.data_ptr()), ctypes.c_void_p(out.data_ptr()), B, C, H, W, ctypes.c_void_p(stream)))
+    _call(lib.hitsir_f32nchw_to_u8hwc if rounding == "truncate" else lib.hitsir_f32nchw_to_u8hwc_round, y.device, y, out, B, C, H, W)
     return out

@@ -455,7 +455,7 @@ def reflect_pad(x, win: int):
 
 
 def _split3_conv(a, w, b):
-    """fp32 emulation of the casa gate's three-term split contraction (glue.cu:297-301): a_hi W_hi + a_lo W_hi + a_hi W_lo + b_hi + b_lo
+    """fp32 emulation of the casa gate's three-term split contraction (glue.cu:257-261): a_hi W_hi + a_lo W_hi + a_hi W_lo + b_hi + b_lo
     with x_hi = bf16(x), x_lo = bf16(x - x_hi)."""
     def split(t):
         hi = bf(t).float()
@@ -474,7 +474,7 @@ def casa_qkv(x, P, win: int, ar: Arith, mut=()):
       Linear 180 -> 18 -> 180 twice, fp32 FMA chains:         e_h = |W_f| e_pool + 181 2^-22 M_f ;  e_s = |W_s| e_h + 19 2^-22 M_s
       channel mean / max per padded pixel (180 terms):        e_cavg = 180 2^-22 mean_c|x| + 2^-24 |cavg|
       3x3 Conv2d(1, 180) over the padded statistic maps (zero outside Hp x Wp, reflected values inside) as ONE bf16 MMA of K = 29
-      (glue.cu:297-301): with x_hi = bf16(x), x_lo = bf16(x - x_hi), |x - x_hi| <= 2^-8 |x| and the dropped residual
+      (glue.cu:257-261): with x_hi = bf16(x), x_lo = bf16(x - x_hi), |x - x_hi| <= 2^-8 |x| and the dropped residual
       |x - x_hi - x_lo| <= 2^-16 |x|, the kernel sums a_hi W_hi + a_lo W_hi + a_hi W_lo, which differs from a W by
       a_hi W_r + a_lo (W_lo + W_r) + a_r W (W_r, a_r the residuals), at most (2^-16 + 2^-16 + 2^-16)(1 + 2^-7) |a||W| < 2^-14 |a||W|; the
       bias loses its residual (2^-16 |b|); the 29 products, at most (1 + 2^-6) |a||W| + |b| in magnitude, are summed in fp32:

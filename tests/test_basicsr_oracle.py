@@ -26,8 +26,8 @@ def test_device_order_y_equals_to_y_channel_for_all_triples():
         assert np.array_equal(want.view(np.uint32), got.view(np.uint32)), slab
 
 
-def test_window_constants_of_the_kernel_are_cv2s():
-    src = open(os.path.join(ROOT, "single-image-super-resolution-application_b200", "csrc", "ssim.cu")).read()
+def test_window_constants_of_metrics_cu_are_cv2s():
+    src = open(os.path.join(ROOT, "single-image-super-resolution-application_b200", "csrc", "metrics.cu")).read()
     body = re.search(r"kBsrGauss\[11\]\s*=\s*\{([^}]*)\}", src).group(1)
     taps = np.array([float.fromhex(t.strip()) for t in body.split(",")])
     assert np.array_equal(taps, R.KERNEL)
